@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config C]     # N=1: plain python; N>1: launched under torchrun
     python bench.py --impl reference [...]                                # the reference's CPU path on the host cores
+    python bench.py [...] --dump-outputs DIR                              # also write the last timed step's records as .npy
 
 --config selects one of BASELINE.json's five configurations (default 2, the one the metric is quoted on):
   1  16 x 1280x720, q=90, per GPU (the reference's own CPU-runnable case)                          weak
@@ -12,8 +13,9 @@
   5  512 x 1080p at q in {75, 85, 90, 95} (four passes per step), sharded over the N GPUs           strong
 A step = one pass of the hot path over the configuration's batch, records-only mode, followed for N>1 by the NCCL gather of the
 per-frame (config 4: per-video) records to rank 0.
-  value     : whole-job frames/s with inputs resident in HBM (CUDA events, max over ranks). The timed region runs at least
-              --min-seconds (default 1 s): `steps` is what was timed (>= the --steps asked for), `timed_region_s` its length.
+  value     : whole-job frames/s with inputs resident in HBM (CUDA events, max over ranks). The timed region is --steps steps;
+              with --min-seconds S > 0 steps are added until it lasts at least S: `steps` is what was timed, `timed_region_s`
+              its length.
   e2e       : the same metric through the reference-facing C-ABI call with HOST (pinned) buffers — the H2D copy of every frame and
               the D2H copy of the records are inside the timed region; `ceiling_frames_s` = what a bare pinned cudaMemcpyAsync of
               the same bytes reaches on this rank at the same moment (all ranks copying concurrently), `per_rank_ms` every rank's time.
@@ -24,6 +26,12 @@ per-frame (config 4: per-video) records to rank 0.
   e2e_from_jpeg_files : (config 2) the same work starting from JPEG files in host memory — GPU decode + analyse.
   cpu_baseline : (N=1) the oracle port of the reference's ELA core (Pillow/libjpeg-turbo + NumPy/OpenCV statistics) on all host
               cores, on a bounded sample of the same frames. Reported, not the target.
+--dump-outputs DIR : after the timed steps, rank 0 writes what the last timed step returned to its caller — the records of every
+              quality, after the per-video reduction (config 4) and the gather to rank 0 — one float64 file per record field,
+              DIR/<field>.npy of shape (qualities, records, ...), and DIR/record_index.npy naming the records written: all of them
+              up to 64 MB in all, beyond that a sample drawn with a fixed seed. The frames come from fixed seeds, so two builds run
+              with the same arguments can be compared file for file.
+--impl reference runs min(--steps, 8) steps of CPU work (each takes seconds) and reports that number as `steps`.
 """
 from __future__ import annotations
 
@@ -234,6 +242,31 @@ class ClockSampler:
                 "samples": len(sm), "power_w_max": max(power)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir: str, per_quality: list) -> dict:
+    """--dump-outputs: every field of the records (padding excluded) as float64 — exact for all of them — stacked over the
+    qualities, DIR/<field>.npy of shape (qualities, records, ...), and DIR/record_index.npy, which records they are: all of them,
+    or, where that would pass DUMP_LIMIT_BYTES (~6 kB per record and quality), a sample drawn with a fixed seed."""
+    import numpy as np
+
+    from v5ela.records import RECORD_DTYPE
+
+    fields = [f for f in RECORD_DTYPE.names if f != "pad"]
+    n = len(per_quality[0])
+    per_record = 8 * len(per_quality) * (1 + sum(int(np.prod(RECORD_DTYPE[f].shape)) for f in fields))
+    keep = min(n, DUMP_LIMIT_BYTES // per_record)
+    index = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    arrays = {f: np.stack([r[f][index] for r in per_quality]).astype(np.float64) for f in fields}
+    arrays["record_index"] = index.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {"dir": out_dir, "files": sorted(name + ".npy" for name in arrays), "bytes": sum(a.nbytes for a in arrays.values()),
+            "records": n, "records_written": keep}
+
+
 def load_profile_json(name: str):
     try:
         with open(os.path.join(ROOT, "profiles", name)) as f:
@@ -316,13 +349,14 @@ def run_native_arm(args):
         handle.block_stage = args.block_stage
     small = n_local * 3 * H * W < 2 * 126e6
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev) if small else None
-    gathered = [None]
+    local_out = [None] * len(quals)                             # this rank's records of the latest step, per quality
 
     def step():
         for qi, q in enumerate(quals):
             analyze_batch(frames, quality=q, records_out=records[qi], handle=handle)
-            recs = reduce_records(records[qi], group, handle=handle) if group else records[qi]
-            gathered[0] = gather_records(recs, total_records) if world > 1 else recs
+            local_out[qi] = reduce_records(records[qi], group, handle=handle) if group else records[qi]
+            if world > 1:
+                gather_records(local_out[qi], total_records)
 
     def barrier():
         if world > 1:
@@ -334,18 +368,20 @@ def run_native_arm(args):
         step()
     barrier()
 
-    # ---- step-time estimate -> number of timed steps (at least --steps, at least --min-seconds)
+    # ---- number of timed steps: --steps, or more when --min-seconds asks for a longer timed region
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    step()
-    e1.record()
-    barrier()
-    est = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
-    if world > 1:
-        dist.all_reduce(est, op=dist.ReduceOp.MAX)
-    # (+5 %: a single step timed alone runs a little slower than the steps of the timed region, and the region must not end up short)
-    K = max(args.steps, int(math.ceil(1.05 * args.min_seconds * 1e3 / max(float(est.item()), 1e-3))))
-    K = min(K, 200000 if not small else 4000)                   # L2-sized inputs: one event pair and one flush per step
+    K = args.steps
+    if args.min_seconds > 0:
+        e0.record()
+        step()
+        e1.record()
+        barrier()
+        est = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
+        if world > 1:
+            dist.all_reduce(est, op=dist.ReduceOp.MAX)
+        # (+5 %: a single step timed alone runs a little slower than the steps of the timed region, and the region must not end up short)
+        K_min = int(math.ceil(1.05 * args.min_seconds * 1e3 / max(float(est.item()), 1e-3)))
+        K = max(K, min(K_min, 200000 if not small else 4000))   # L2-sized inputs: one event pair and one flush per step
 
     # ---- device-resident throughput (value) + fused-kernel duration (roofline), clocks sampled during the region
     sampler = ClockSampler(local_rank) if rank == 0 else None
@@ -373,6 +409,14 @@ def run_native_arm(args):
     fused_ms, fused_n = handle.profile_read(reset=True)
     handle.profile_enable(False)
     inst = handle.last_instantiation
+    dumped = []
+    if args.dump_outputs:
+        # the gather returns a view of a receive block that the next gather overwrites, so each quality's result is gathered
+        # again here (untimed, every rank takes part) from the records this rank computed in the last timed step, and copied
+        for r in local_out:
+            r = gather_records(r, total_records) if world > 1 else r
+            if rank == 0:
+                dumped.append(as_records(r))
     # keep the GPU busy a little longer so that slow nvidia-smi polling still sees the load (local work only)
     t_end = time.perf_counter() + 0.4
     while time.perf_counter() < t_end and n_local:
@@ -432,7 +476,7 @@ def run_native_arm(args):
     est_e = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if world > 1:                                               # every rank must run the same number of steps: they end in a collective
         dist.all_reduce(est_e, op=dist.ReduceOp.MAX)
-    Ke = max(2, min(50, int(math.ceil(min(args.min_seconds, 1.0) * 1e3 / max(float(est_e.item()), 1e-3)))))
+    Ke = max(2, min(50, int(math.ceil(1e3 / max(float(est_e.item()), 1e-3)))))            # about 1 s, at most 50 steps
     barrier()
     e0.record()
     for _ in range(Ke):
@@ -574,6 +618,8 @@ def run_native_arm(args):
             line["e2e_from_jpeg_files"] = files_leg
         if cpu_baseline is not None:
             line["cpu_baseline"] = cpu_baseline
+        if args.dump_outputs:
+            line["outputs"] = write_outputs(args.dump_outputs, dumped)
         emit(line)
     if world > 1:
         dist.barrier()
@@ -587,13 +633,20 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS), help="BASELINE.json configuration 1..5 (default 2)")
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="minimum length of the timed region (steps are added to reach it)")
+    ap.add_argument("--min-seconds", type=float, default=0.0,
+                    help="minimum length of the timed region: steps are added to --steps to reach it (default 0: exactly --steps)")
     ap.add_argument("--impl", choices=("native", "reference"), default="native")
     ap.add_argument("--block-stage", choices=("smem", "mma"), default=None, help="build of the fused kernel's block stage (default: library's)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-parity", action="store_true", help="skip the untimed oracle spot-check")
     ap.add_argument("--no-files", action="store_true", help="skip the JPEG-files leg of config 2")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the records of the last timed step to DIR/<field>.npy (float64); native arm only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs is for the native arm")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_native_arm(args)

@@ -1,10 +1,12 @@
-"""CPU: bench.py's command-line contract for the arm that runs without a GPU (--impl reference): exactly one JSON line on
-stdout with the keys the driver reads; and the native arm refuses to run without a CUDA device instead of falling back."""
+"""bench.py's command-line contract. CPU: the arm that runs without a GPU (--impl reference) prints exactly one JSON line on
+stdout with the keys a caller reads; the native arm refuses to run without a CUDA device instead of falling back. GPU: the native
+arm times exactly --steps steps and --dump-outputs writes what they computed."""
 import json
 import os
 import subprocess
 import sys
 
+import pytest
 from helpers import HERE
 
 ROOT = os.path.dirname(HERE)
@@ -40,6 +42,73 @@ def test_native_arm_needs_a_gpu():
                        capture_output=True, text=True, timeout=300)
     assert p.returncode != 0 and p.stdout.strip() == ""
     assert "no CUDA device" in p.stderr
+
+
+def test_bad_step_count_and_reference_dump_are_refused():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120)
+        assert p.returncode == 2 and p.stdout.strip() == "", extra
+
+
+def test_dump_larger_than_the_limit_is_a_seeded_sample(tmp_path):
+    """Past the size limit, --dump-outputs writes the same fixed sample of records every time, and says which ones."""
+    code = f"""
+import sys; sys.argv = ["bench.py"]; sys.path[:0] = [{ROOT!r}, {os.path.join(ROOT, "fake-video-detection-engine_b200")!r}]
+import numpy as np, bench
+from oracle import c_oracle
+from v5ela.synth import gen_batch
+recs, _ = c_oracle.analyze(gen_batch(0, 40, 24, 40, seed=0), 90)
+bench.DUMP_LIMIT_BYTES = 15 * 2 * 8 * 781                       # room for 15 of the 40 records at two qualities
+for d in ("a", "b"):
+    bench.write_outputs({str(tmp_path)!r} + "/" + d, [recs, recs[::-1]])
+"""
+    p = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
+    assert p.returncode == 0, p.stderr[-2000:]
+    import numpy as np
+
+    from oracle import c_oracle
+    from v5ela.synth import gen_batch
+
+    recs, _ = c_oracle.analyze(gen_batch(0, 40, 24, 40, seed=0), 90)
+    idx = np.load(tmp_path / "a" / "record_index.npy")
+    assert len(idx) == 15 and len(set(idx)) == 15 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "record_index.npy"))
+    total = sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a"))
+    assert total <= 15 * 2 * 8 * 781 + 16 * 128                 # + the .npy headers
+    hist = np.load(tmp_path / "a" / "ela_hist.npy")
+    assert hist.shape == (2, 15, 3, 256)
+    assert np.array_equal(hist[0], recs["ela_hist"][idx.astype(int)]) and np.array_equal(hist[1], recs["ela_hist"][::-1][idx.astype(int)])
+
+
+@pytest.mark.gpu
+def test_native_arm_times_the_steps_asked_for_and_dumps_what_they_computed(tmp_path):
+    """`steps` is exactly --steps; --dump-outputs writes the last timed step's records, one float64 file per field, identical from
+    run to run and equal to the oracle's records of the same seeded frames."""
+    import numpy as np
+
+    from oracle import c_oracle
+    from v5ela.records import RECORD_DTYPE
+    from v5ela.synth import gen_frame
+
+    fields = [f for f in RECORD_DTYPE.names if f != "pad"]
+    dumps = []
+    for run in range(2):
+        out = tmp_path / f"run{run}"
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--config", "1", "--steps", "3", "--warmup", "1", "--no-cpu",
+                            "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert p.returncode == 0, p.stderr[-2000:]
+        d = json.loads(p.stdout)
+        assert d["steps"] == 3 and d["parity"]["ok"]
+        assert sorted(os.listdir(out)) == sorted(f + ".npy" for f in fields + ["record_index"]) == d["outputs"]["files"]
+        assert np.array_equal(np.load(out / "record_index.npy"), np.arange(16.0)) and d["outputs"]["records_written"] == 16
+        dumps.append({f: np.load(out / (f + ".npy")) for f in fields})
+    for i in (0, 15):
+        want = c_oracle.analyze_frame(gen_frame(i, 720, 1280, 0), 90)["record"]
+        for f in fields:
+            a = dumps[0][f]
+            assert a.dtype == np.float64 and a.shape == (1, 16) + RECORD_DTYPE[f].shape, f
+            assert np.array_equal(a, dumps[1][f]), f
+            assert np.array_equal(a[0, i], want[f].astype(np.float64)), (i, f)
 
 
 def test_profile_source_hash_ignores_comments_and_matches_the_committed_profile():

@@ -28,8 +28,10 @@ def _build(tag, defs):
     csrc = os.path.join(ROOT, "fake-video-detection-engine_b200", "csrc")
     deps = [src] + [os.path.join(csrc, f) for f in ("v5jpeg_enc.cuh", "v5jpeg_dec.cuh", "v5jpeg_common.h", "v5ela_device.cuh", "v5ela_host.h")]
     if not os.path.exists(so) or any(os.path.getmtime(d) > os.path.getmtime(so) for d in deps):
+        tmp = f"{so}.{os.getpid()}.so"          # written aside, then renamed: parallel test processes never load a half-written file
         subprocess.check_call(["g++", "-O2", "-shared", "-fPIC", "-Wno-unknown-pragmas", *defs, "-I", os.path.join(ROOT, "include"),
-                               "-I", csrc, src, "-o", so])
+                               "-I", csrc, src, "-o", tmp])
+        os.replace(tmp, so)
     lib = ctypes.CDLL(so)
     u8p, i16p = ctypes.POINTER(ctypes.c_uint8), ctypes.POINTER(ctypes.c_int16)
     lib.v5jemu_encode.restype = ctypes.c_int64

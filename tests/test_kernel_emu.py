@@ -39,8 +39,10 @@ def emu(request):
             extra += ["-DV5_EMU_REVERSE=1"]
         if "_mma" in variant:
             extra += ["-DV5_MMA_BLOCKS=1", "-DV5_MMA_NP=2" if "np2" in variant else "-DV5_MMA_NP=1"]
+        tmp = f"{so}.{os.getpid()}.so"          # written aside, then renamed: parallel test processes never load a half-written file
         subprocess.check_call(["g++", "-O2", "-shared", "-fPIC", "-Wno-unknown-pragmas", f"-DV5_MIN_CTAS={variant[0]}", *extra,
-                               "-I", os.path.join(ROOT, "include"), "-I", csrc, src, "-o", so])
+                               "-I", os.path.join(ROOT, "include"), "-I", csrc, src, "-o", tmp])
+        os.replace(tmp, so)
     lib = ctypes.CDLL(so)
     u8p = ctypes.POINTER(ctypes.c_uint8)
     lib.v5emu_analyze.argtypes = [u8p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int64, ctypes.c_int64,

@@ -1,10 +1,12 @@
 """The drop-in claim of INTEGRATION.md, executed: a copy of the reference's ``nodes/`` tree and of its own test file
-(/root/reference/tests/test_v5_texture_ela.py, byte for byte) with ONE file replaced — nodes/V_nodes/v5_texture_ela.py by this repo's
-module — and the reference's tests run against it, unmodified, by tests/dropin_runner.py in a subprocess.
+(tests/test_v5_texture_ela.py of the reference, byte for byte) with ONE file replaced — nodes/V_nodes/v5_texture_ela.py by this
+repo's module — and the reference's tests run against it, unmodified, by tests/dropin_runner.py in a subprocess.
 
-/root/reference only exists in the build container: everywhere else these tests skip. The two tests of the reference's file that
-reach the analysis need the GPU (there is no CPU implementation behind the node); ``test_v5_no_faces`` and the failure-path test run
-anywhere."""
+The reference is not part of this repository: point V5ELA_REFERENCE_ROOT at a checkout of it to run these tests; without one they
+skip. tests/test_node.py restates the same three tests against stored artefacts of the reference (tests/golden/node_golden.json),
+which need no checkout. The two tests of
+the reference's file that reach the analysis need the GPU (there is no CPU implementation behind the node); ``test_v5_no_faces`` and
+the failure-path test run anywhere."""
 import filecmp
 import os
 import shutil
@@ -15,11 +17,11 @@ import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = os.environ.get("V5ELA_REFERENCE_ROOT", "/root/reference")
+REF = os.environ.get("V5ELA_REFERENCE_ROOT", "")
 OURS = os.path.join(ROOT, "fake-video-detection-engine_b200", "nodes", "V_nodes", "v5_texture_ela.py")
 
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "tests", "test_v5_texture_ela.py")),
-                                reason="the reference checkout is only present in the build container")
+pytestmark = pytest.mark.skipif(not (REF and os.path.exists(os.path.join(REF, "tests", "test_v5_texture_ela.py"))),
+                                reason="needs a checkout of the reference project: set V5ELA_REFERENCE_ROOT")
 
 
 @pytest.fixture
@@ -53,7 +55,7 @@ def test_reference_tests_that_need_no_device(dropin_tree):
 
 @pytest.mark.gpu
 def test_reference_test_file_unmodified_against_the_replaced_module(dropin_tree):
-    """/root/reference/tests/test_v5_texture_ela.py:48-89 — all three tests, as the reference wrote them."""
+    """The reference's tests/test_v5_texture_ela.py:48-89 — all three tests, as the reference wrote them."""
     rc, out = run_reference_tests(dropin_tree)
     assert rc == 0, out
     assert "dropin: ran 3 failures 0 errors 0" in out
