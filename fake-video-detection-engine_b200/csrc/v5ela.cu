@@ -20,10 +20,6 @@ static_assert(sizeof(v5ela_record) == 3144, "V5F v1 record layout");
 
 namespace v5 {
 
-cudaError_t fused_prepare_smem() { return fused_prepare(); }
-int fused_launch_smem(v5_fused_args &a) { return fused_launch(a); }
-int fused_launch_ragged_smem(v5_ragged_args &a) { return fused_launch_ragged(a); }
-
 // One warp per (frame, channel): ela_sum = sum b*hist[b], ela_sumsq = sum b^2*hist[b], ela_max = highest non-empty bin.
 __global__ void __launch_bounds__(96) ela_finalize_kernel(v5ela_record *recs, int n)
 {
@@ -139,9 +135,37 @@ __global__ void __launch_bounds__(256) ela_reduce_kernel(const v5ela_record *rec
 
 }  // namespace v5
 
+namespace v5m {                                         // v5ela_mma.cu: the launcher of the tensor-core build
+cudaError_t prepare();
+int launch(const v5plan::KParams &p, int inst, long long total, int max_ctas, cudaStream_t st, cudaEvent_t ev_start, cudaEvent_t ev_stop);
+}
+
 // ======================================================================================================= C ABI
 #include "v5ela_handle.h"
 using namespace v5host;
+
+// The two builds of the fused kernel, indexed by v5ela_handle::block_stage.
+static const struct {
+    cudaError_t (*prepare)();
+    int (*launch)(const v5plan::KParams &, int, long long, int, cudaStream_t, cudaEvent_t, cudaEvent_t);
+} fused_builds[2] = {{v5::prepare, v5::launch}, {v5m::prepare, v5m::launch}};
+static_assert(V5ELA_BLOCKS_SMEM == 0 && V5ELA_BLOCKS_MMA == 1, "fused_builds");
+
+// Launches the planned fused kernel with the handle's block stage, then the finalize kernel: the tail of every analyze call.
+static int launch_fused(v5ela_handle *h, const v5plan::KParams &p, int inst, long long total, cudaStream_t st)
+{
+    const bool prof = h->profiling && h->prof_used + 2 <= h->prof_events.size();
+    const int rc = fused_builds[h->block_stage].launch(p, inst, total, h->sm_count * h->ctas_per_sm, st,
+                                                       prof ? h->prof_events[h->prof_used] : nullptr,
+                                                       prof ? h->prof_events[h->prof_used + 1] : nullptr);
+    if (rc != 0) return fail(h, V5ELA_ERR_CUDA, "fused kernel launch: %s", cudaGetErrorString((cudaError_t)rc));
+    h->last_inst = inst == v5plan::INST_RAGGED ? V5ELA_INST_GENERAL : inst;
+    if (prof) h->prof_used += 2;
+    v5::ela_finalize_kernel<<<p.n, 96, 0, st>>>(p.records, p.n);
+    V5_CUDA(h, cudaGetLastError());
+    h->launches += 2;
+    return V5ELA_OK;
+}
 
 extern "C" {
 
@@ -174,15 +198,15 @@ int v5ela_create(int device, v5ela_handle **out)
     if (!h) return V5ELA_ERR_NOMEM;
     h->device = device;
     h->sm_count = prop.multiProcessorCount;
-    v5::quant_tables(h->quality, h->luma, h->chroma);
+    v5plan::quant_tables(h->quality, h->luma, h->chroma);
     DeviceGuard guard(device);
-    if (v5::fused_prepare_smem() != cudaSuccess || v5m::fused_prepare_mma() != cudaSuccess) {
+    if (fused_builds[0].prepare() != cudaSuccess || fused_builds[1].prepare() != cudaSuccess) {
         delete h;
         return V5ELA_ERR_CUDA;
     }
     {   // per-lane operand fragments of the tensor-core block stage: 32 x 128 bytes, fixed for the life of the handle
-        alignas(16) unsigned char lc[32 * 128];
-        if (!v5m::lane_consts_host(lc) || cudaMalloc(&h->d_lane_consts, sizeof(lc)) != cudaSuccess ||
+        v5plan::LaneConsts lc[32];
+        if (!v5::mma::make_lane_consts(lc) || cudaMalloc(&h->d_lane_consts, sizeof(lc)) != cudaSuccess ||
             cudaMemcpy(h->d_lane_consts, lc, sizeof(lc), cudaMemcpyHostToDevice) != cudaSuccess) {
             cudaFree(h->d_lane_consts);
             delete h;
@@ -195,7 +219,7 @@ int v5ela_create(int device, v5ela_handle **out)
     if (env && sscanf(env, "%d,%d,%d", &h->decomp[0], &h->decomp[1], &h->decomp[2]) == 3 && h->decomp[0] >= 1 && h->decomp[1] >= 4)
         h->decomp_set = true;
     env = getenv("V5ELA_CTAS_PER_SM");                        // tuning knob: launch fewer persistent CTAs than fit
-    if (env && atoi(env) >= 1 && atoi(env) <= v5::MIN_CTAS) h->ctas_per_sm = atoi(env);
+    if (env && atoi(env) >= 1 && atoi(env) <= v5plan::MIN_CTAS) h->ctas_per_sm = atoi(env);
     env = getenv("V5ELA_BLOCK_STAGE");                        // "mma" / "smem": default block stage of new handles (A/B runs)
     if (env) h->block_stage = !strcmp(env, "mma") ? V5ELA_BLOCKS_MMA : (!strcmp(env, "smem") ? V5ELA_BLOCKS_SMEM : h->block_stage);
     env = getenv("V5ELA_HOST_CHUNK");
@@ -244,7 +268,7 @@ int v5ela_set_quality(v5ela_handle *h, int quality)
     if (!h) return V5ELA_ERR_INVALID;
     if (quality < 1 || quality > 100) return fail(h, V5ELA_ERR_INVALID, "quality must be in 1..100%s");
     h->quality = quality;
-    v5::quant_tables(quality, h->luma, h->chroma);
+    v5plan::quant_tables(quality, h->luma, h->chroma);
     return V5ELA_OK;
 }
 
@@ -273,39 +297,19 @@ int v5ela_analyze_ex(v5ela_handle *h, const uint8_t *d_rgb, int n, int height, i
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     ScratchOrder order(h, st);                                  // the ticket counter is handle-owned
     if (!h->d_ticket) V5_CUDA(h, cudaMalloc(&h->d_ticket, sizeof(unsigned int)));
-    const bool prof = h->profiling && h->prof_used + 2 <= h->prof_events.size();
-    v5_fused_args a;
-    memset(&a, 0, sizeof(a));
-    a.rgb = d_rgb; a.n = n; a.h = height; a.w = width;
-    a.frame_stride = frame_stride_bytes; a.row_stride = row_stride_bytes;
-    a.records = static_cast<v5ela_record *>(d_records);
-    a.residual = d_residual; a.tex_hist = d_tex_hist;
-    a.quality = h->quality; a.seg_rows = h->seg_rows;
-    a.target_items = 2 * h->sm_count * h->ctas_per_sm;
-    a.max_ctas = h->sm_count * h->ctas_per_sm;
-    a.tune = h->decomp_set ? h->decomp : nullptr;
-    a.ticket = h->d_ticket; a.lane_consts = h->d_lane_consts;
-    a.stream = st;
-    if (prof) { a.ev_start = h->prof_events[h->prof_used]; a.ev_stop = h->prof_events[h->prof_used + 1]; }
-    const bool use_mma = h->block_stage == V5ELA_BLOCKS_MMA;
-    a.check_only = 1;                                           // validate before anything is written
-    int rc = use_mma ? v5m::fused_launch_mma(a) : v5::fused_launch_smem(a);
-    if (rc == 0) {
-        V5_CUDA(h, cudaMemsetAsync(h->d_ticket, 0, sizeof(unsigned int), st));
-        V5_CUDA(h, cudaMemsetAsync(d_records, 0, sizeof(v5ela_record) * (size_t)n, st));
-        if (d_tex_hist) V5_CUDA(h, cudaMemsetAsync(d_tex_hist, 0, sizeof(uint32_t) * 256 * (size_t)n, st));
-        a.check_only = 0;
-        rc = use_mma ? v5m::fused_launch_mma(a) : v5::fused_launch_smem(a);
-    }
-    if (rc == -1) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze: bad pointer, size or stride%s");
-    if (rc == -2) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze: batch too large%s");
-    if (rc > 0) return fail(h, V5ELA_ERR_CUDA, "fused kernel launch: %s", cudaGetErrorString((cudaError_t)rc));
-    h->last_inst = a.inst;
-    if (prof) h->prof_used += 2;
-    v5::ela_finalize_kernel<<<n, 96, 0, st>>>(static_cast<v5ela_record *>(d_records), n);
-    V5_CUDA(h, cudaGetLastError());
-    h->launches += 2;
-    return V5ELA_OK;
+    v5plan::KParams p;
+    if (v5plan::fill_params(p, d_rgb, n, height, width, frame_stride_bytes, row_stride_bytes, static_cast<v5ela_record *>(d_records),
+                            d_residual, h->quality, h->seg_rows, 2 * h->sm_count * h->ctas_per_sm, h->decomp_set ? h->decomp : nullptr) != 0)
+        return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze: bad pointer, size or stride%s");
+    const long long total = v5plan::total_work_items(p);
+    if (total > 0x7fffffffLL) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze: batch too large%s");
+    p.tex_hist = d_tex_hist;
+    p.ticket = h->d_ticket;
+    p.lane_consts = h->d_lane_consts;
+    V5_CUDA(h, cudaMemsetAsync(h->d_ticket, 0, sizeof(unsigned int), st));
+    V5_CUDA(h, cudaMemsetAsync(d_records, 0, sizeof(v5ela_record) * (size_t)n, st));
+    if (d_tex_hist) V5_CUDA(h, cudaMemsetAsync(d_tex_hist, 0, sizeof(uint32_t) * 256 * (size_t)n, st));
+    return launch_fused(h, p, v5plan::choose_instantiation(p), total, st);
 }
 
 int v5ela_analyze_ragged(v5ela_handle *h, const v5ela_frame_desc *frames_host, int n, void *d_records, void *cuda_stream)
@@ -317,7 +321,7 @@ int v5ela_analyze_ragged(v5ela_handle *h, const v5ela_frame_desc *frames_host, i
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     ScratchOrder order(h, st);                                  // ticket counter and frame table are handle-owned
     if (!h->d_ticket) V5_CUDA(h, cudaMalloc(&h->d_ticket, sizeof(unsigned int)));
-    const size_t desc_bytes = (v5_ragged_args::table_bytes(n) + 15) / 16 * 16, need = desc_bytes + sizeof(v5::EnhDesc) * (size_t)n;
+    const size_t desc_bytes = (sizeof(v5plan::FrameDesc) * (size_t)n + 15) / 16 * 16, need = desc_bytes + sizeof(v5::EnhDesc) * (size_t)n;
     if (h->table_cap < need) {
         if (h->ev_table) cudaEventSynchronize(h->ev_table);
         if (h->h_table) cudaFreeHost(h->h_table);
@@ -331,46 +335,33 @@ int v5ela_analyze_ragged(v5ela_handle *h, const v5ela_frame_desc *frames_host, i
     }
     if (!h->ev_table) V5_CUDA(h, cudaEventCreateWithFlags(&h->ev_table, cudaEventDisableTiming));
     V5_CUDA(h, cudaEventSynchronize(h->ev_table));              // the previous call's upload has left the staging buffer
-    const bool prof = h->profiling && h->prof_used + 2 <= h->prof_events.size();
-    v5_ragged_args a;
-    memset(&a, 0, sizeof(a));
-    a.frames = frames_host; a.n = n;
-    a.records = static_cast<v5ela_record *>(d_records);
-    a.quality = h->quality; a.seg_rows = h->seg_rows;
-    a.target_items = 2 * h->sm_count * h->ctas_per_sm;
-    a.max_ctas = h->sm_count * h->ctas_per_sm;
-    a.ticket = h->d_ticket; a.lane_consts = h->d_lane_consts;
-    a.table = h->h_table; a.d_table = h->d_table;
-    a.stream = st;
-    if (prof) { a.ev_start = h->prof_events[h->prof_used]; a.ev_stop = h->prof_events[h->prof_used + 1]; }
-    const bool use_mma = h->block_stage == V5ELA_BLOCKS_MMA;
-    a.check_only = 1;
-    int rc = use_mma ? v5m::fused_launch_ragged_mma(a) : v5::fused_launch_ragged_smem(a);
-    bool any_enh = false;
-    if (rc == 0) {
-        v5::EnhDesc *et = reinterpret_cast<v5::EnhDesc *>(static_cast<char *>(h->h_table) + desc_bytes);
-        for (int i = 0; i < n; i++) {
-            const v5ela_frame_desc &f = frames_host[i];
-            et[i].src = f.residual ? f.residual : f.enhanced;
-            et[i].dst = f.enhanced;
-            et[i].bytes = f.enhanced ? (long long)f.height * f.width * 3 : 0;
-            any_enh = any_enh || f.enhanced;
-        }
-        V5_CUDA(h, cudaMemcpyAsync(h->d_table, h->h_table, need, cudaMemcpyHostToDevice, st));
-        V5_CUDA(h, cudaEventRecord(h->ev_table, st));
-        V5_CUDA(h, cudaMemsetAsync(h->d_ticket, 0, sizeof(unsigned int), st));
-        V5_CUDA(h, cudaMemsetAsync(d_records, 0, sizeof(v5ela_record) * (size_t)n, st));
-        a.check_only = 0;
-        rc = use_mma ? v5m::fused_launch_ragged_mma(a) : v5::fused_launch_ragged_smem(a);
-    }
+    long long total = 0;
+    int rc = v5plan::plan_ragged(static_cast<v5plan::FrameDesc *>(h->h_table), frames_host, n, h->seg_rows,
+                                       2 * h->sm_count * h->ctas_per_sm, &total);
     if (rc == -1) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_ragged: bad pointer, size or stride in a frame descriptor%s");
     if (rc == -2) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_ragged: batch too large%s");
-    if (rc > 0) return fail(h, V5ELA_ERR_CUDA, "fused kernel launch: %s", cudaGetErrorString((cudaError_t)rc));
-    h->last_inst = V5ELA_INST_GENERAL;
-    if (prof) h->prof_used += 2;
-    v5::ela_finalize_kernel<<<n, 96, 0, st>>>(static_cast<v5ela_record *>(d_records), n);
-    V5_CUDA(h, cudaGetLastError());
-    h->launches += 2;
+    v5::EnhDesc *et = reinterpret_cast<v5::EnhDesc *>(static_cast<char *>(h->h_table) + desc_bytes);
+    bool any_enh = false;
+    for (int i = 0; i < n; i++) {
+        const v5ela_frame_desc &f = frames_host[i];
+        et[i].src = f.residual ? f.residual : f.enhanced;
+        et[i].dst = f.enhanced;
+        et[i].bytes = f.enhanced ? (long long)f.height * f.width * 3 : 0;
+        any_enh = any_enh || f.enhanced;
+    }
+    V5_CUDA(h, cudaMemcpyAsync(h->d_table, h->h_table, need, cudaMemcpyHostToDevice, st));
+    V5_CUDA(h, cudaEventRecord(h->ev_table, st));
+    V5_CUDA(h, cudaMemsetAsync(h->d_ticket, 0, sizeof(unsigned int), st));
+    V5_CUDA(h, cudaMemsetAsync(d_records, 0, sizeof(v5ela_record) * (size_t)n, st));
+    v5plan::KParams p;
+    memset(&p, 0, sizeof(p));
+    p.records = static_cast<v5ela_record *>(d_records);
+    p.n = n;
+    p.ticket = h->d_ticket;
+    p.lane_consts = h->d_lane_consts;
+    p.frames = static_cast<const v5plan::FrameDesc *>(h->d_table);
+    v5plan::fill_quant(p.q, h->quality);
+    if ((rc = launch_fused(h, p, v5plan::choose_instantiation(p), total, st))) return rc;
     if (any_enh) {
         if (n > 65535) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_ragged: more than 65535 frames with enhanced maps%s");
         v5::ela_enhance_ragged_kernel<<<dim3(32, (unsigned)n), 256, 0, st>>>(

@@ -25,21 +25,11 @@
 // reachable on the device. Nothing here is a fallback for anything else.
 #pragma once
 
-namespace V5_NS {
-namespace mma {
-
-constexpr int OFF1 = 8192;      // F1 output + OFF1 in 0..65535 (|F1 output| <= 4096)
-constexpr int OFF2 = 32768;     // dequantised coefficient + OFF2
-constexpr int OFF3 = 32768;     // I1 output + OFF3 (|I1 output| <= 21047, DESIGN.md 4.1)
-// The descale of I1 is 11 bits; with the matrix doubled and the dequantised coefficients handed over x 16 the MMA accumulates
-// 32 x the sum, the descale becomes 16 bits and the two 16-bit results of a lane are bytes 2..3 of its accumulators — one PRMT, no
-// shifts. (|2 M| < 2^15 still fits two signed limbs; |16 c'| <= 16 * 1151 fits the 16-bit limb pair.) The other descales (11 after
-// one-limb pixels, 15 in front of the quantiser, 18 in front of the saturating pack) need their integer anyway.
-constexpr int I1_MSCALE = 2, I1_DSCALE = 16;
+namespace v5plan {
 
 // Per-lane constants, laid out as eight 128-bit words: a lane loads them with eight LDS.128 and every MMA operand that needs
 // consecutive registers — the A pair (a0, a1) of a constants-as-A pass, the C quad of group 0 — is an aligned part of one of those
-// words, so no register moves are needed in front of the IMMAs.
+// words, so no register moves are needed in front of the IMMAs. One layout for both builds: KParams::lane_consts points to them.
 struct alignas(16) LaneConsts {
     uint32_t f1a[2][2];         // F1: A pair (rows G0, rows G1) for the left / right block of a pair
     uint32_t i1a[4];            // I1: A pair of MMA 1 (rows G0, rows G1), A pair of MMA 2 (rows G2, zero)
@@ -51,6 +41,22 @@ struct alignas(16) LaneConsts {
     int32_t ci2[4];             // I2: like F2
 };
 static_assert(sizeof(LaneConsts) == 128, "LaneConsts layout");
+
+}  // namespace v5plan
+
+namespace V5_NS {
+namespace mma {
+
+using v5plan::LaneConsts;
+
+constexpr int OFF1 = 8192;      // F1 output + OFF1 in 0..65535 (|F1 output| <= 4096)
+constexpr int OFF2 = 32768;     // dequantised coefficient + OFF2
+constexpr int OFF3 = 32768;     // I1 output + OFF3 (|I1 output| <= 21047, DESIGN.md 4.1)
+// The descale of I1 is 11 bits; with the matrix doubled and the dequantised coefficients handed over x 16 the MMA accumulates
+// 32 x the sum, the descale becomes 16 bits and the two 16-bit results of a lane are bytes 2..3 of its accumulators — one PRMT, no
+// shifts. (|2 M| < 2^15 still fits two signed limbs; |16 c'| <= 16 * 1151 fits the 16-bit limb pair.) The other descales (11 after
+// one-limb pixels, 15 in front of the quantiser, 18 in front of the saturating pack) need their integer anyway.
+constexpr int I1_MSCALE = 2, I1_DSCALE = 16;
 
 // ---- host side: the pass matrices and the per-lane constants ---------------------------------------------------------------------
 #define V5M_C0_298 2446

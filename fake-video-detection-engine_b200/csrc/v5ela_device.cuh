@@ -37,7 +37,9 @@
 #define V5_NS v5
 #endif
 
-namespace V5_NS {
+// The kernel's parameter block and the work decomposition it carries are the same in both builds: namespace v5plan holds them
+// once, for the two builds, the C ABI and the emulator (v5ela_host.h fills them).
+namespace v5plan {
 
 // ----------------------------------------------------------------------------------------------- geometry constants
 #ifndef V5_NT
@@ -49,25 +51,9 @@ namespace V5_NS {
 #ifndef V5_MIN_CTAS
 #define V5_MIN_CTAS 2
 #endif
-// Block stage (8x8 round trip): 1 = int8 limb-split tensor-core form (v5ela_dctmma.cuh, kernel v11), 0 = the v2..v10 form
-// (4 threads per block, two shared-memory transposes) kept as a compile-time variant for A/B runs.
-#ifndef V5_MMA_BLOCKS
-#define V5_MMA_BLOCKS 0
-#endif
-#ifndef V5_MMA_NP
-#define V5_MMA_NP 1                         // pairs of blocks in flight per warp (1, 2, 4 measured: profiles/r02/variants.txt)
-#endif
 constexpr int NT = V5_NT;                   // threads per CTA
 constexpr int TW_MAX = V5_TW_MAX;           // strip width, MCUs (16 px)
 constexpr int MIN_CTAS = V5_MIN_CTAS;       // resident CTAs per SM the kernel is built for
-constexpr int BAND_MCUS = TW_MAX + 2;       // + halo MCU column each side
-constexpr int BAND_PX = BAND_MCUS * 16;     // 512
-constexpr int RGB_PITCH = BAND_PX * 3;      // 1536 bytes per band line
-// Plane pitches. The tensor-core block stage reads 4 pixels of 8 consecutive lines per quarter warp: 16 bytes of padding per line
-// put those lines into different banks (pitch / 4 = 4 mod 32) — conflict-free 32-bit loads and 16-bit stores.
-constexpr int PLANE_PAD = V5_MMA_BLOCKS ? 16 : 0;
-constexpr int Y_PITCH = BAND_PX + PLANE_PAD;        // 512 (+16)
-constexpr int C_PITCH = BAND_PX / 2 + PLANE_PAD;    // 256 (+16)
 
 // Exact division constants for one quantisation table entry T (divisor d = 8T), see make_quant():
 //   q_biased = umulhi(c + (c >> 31) + bias, recip);  dequantised = q_biased * t - unbias
@@ -78,7 +64,7 @@ struct QuantTab {
     int32_t unbias[64];
 };
 
-namespace mma { struct LaneConsts; }
+struct LaneConsts;              // v5ela_dctmma.cuh
 
 // One frame of a ragged batch (v5ela_analyze_ragged): its own geometry, pointers and work decomposition. Built on the host,
 // read by the RAGGED instantiation's make_geo; uniform batches keep everything in KParams (the kernel-parameter constant bank).
@@ -105,25 +91,35 @@ struct KParams {
     int split_frame, n_segs_b;  // frames >= split_frame are cut into n_segs_b (shorter) segments: the tail of the launch (fill_params)
     int work_split;             // first work item of the frames >= split_frame
     unsigned int *ticket;       // work-item counter (zeroed before every launch): CTAs draw items dynamically
-    const mma::LaneConsts *lane_consts;   // 32 entries (v5ela_dctmma.cuh), device memory owned by the handle
+    const LaneConsts *lane_consts;        // 32 entries (v5ela_dctmma.cuh), device memory owned by the handle
     const FrameDesc *frames;    // ragged batches only: n descriptors in device memory (then h, w, ... above are unused)
     int vec_ok;                 // 1: every band line start is 16-byte aligned in global memory (128-bit loads)
     int resid_vec_ok;           // 1: residual rows are 16-byte aligned (3*W % 16 == 0 and base aligned): 128-bit stores
     QuantTab q[2];              // [0] luma, [1] chroma — lives in the kernel parameter constant bank
 };
 
-// Host side: fills the reciprocal constants (called by v5ela_set_quality).
-inline void make_quant(const uint16_t tab[64], QuantTab &q)
-{
-    for (int i = 0; i < 64; i++) {
-        const uint32_t t = tab[i], d = t << 3;
-        const uint32_t b = (8192u + d - 1) / d;                     // b*d >= 8192 >= max |coef|
-        q.recip[i] = (uint32_t)(0x100000000ull / d) + 1u;           // exact for x*d < 2^32, x < 2^15
-        q.bias[i] = (int32_t)(d / 2 + b * d);
-        q.t[i] = (int32_t)t;
-        q.unbias[i] = (int32_t)(b * t);
-    }
-}
+}  // namespace v5plan
+
+namespace V5_NS {
+
+using namespace v5plan;                     // the device code, and callers that name the plan through a build (v5::fill_params, ...)
+
+// Block stage (8x8 round trip): 1 = int8 limb-split tensor-core form (v5ela_dctmma.cuh, kernel v11), 0 = the v2..v10 form
+// (4 threads per block, two shared-memory transposes) kept as a compile-time variant for A/B runs.
+#ifndef V5_MMA_BLOCKS
+#define V5_MMA_BLOCKS 0
+#endif
+#ifndef V5_MMA_NP
+#define V5_MMA_NP 1                         // pairs of blocks in flight per warp (1, 2, 4 measured: profiles/r02/variants.txt)
+#endif
+constexpr int BAND_MCUS = TW_MAX + 2;       // + halo MCU column each side
+constexpr int BAND_PX = BAND_MCUS * 16;     // 512
+constexpr int RGB_PITCH = BAND_PX * 3;      // 1536 bytes per band line
+// Plane pitches. The tensor-core block stage reads 4 pixels of 8 consecutive lines per quarter warp: 16 bytes of padding per line
+// put those lines into different banks (pitch / 4 = 4 mod 32) — conflict-free 32-bit loads and 16-bit stores.
+constexpr int PLANE_PAD = V5_MMA_BLOCKS ? 16 : 0;
+constexpr int Y_PITCH = BAND_PX + PLANE_PAD;        // 512 (+16)
+constexpr int C_PITCH = BAND_PX / 2 + PLANE_PAD;    // 256 (+16)
 
 // ------------------------------------------------------------------------------------------------------- shims
 struct alignas(16) U4 { uint32_t x, y, z, w; };

@@ -9,7 +9,6 @@
 
 #include "v5ela.h"
 #include "v5ela_device.cuh"
-#include "v5ela_fused_args.h"
 
 struct v5ela_handle {
     int device = 0;
@@ -18,7 +17,7 @@ struct v5ela_handle {
     int seg_rows = 0;                      // 0 = default
     int decomp[3] = {0, 0, 0};             // V5ELA_DECOMP=a,b,c development knob (fill_params' tune); decomp_set = it was given
     bool decomp_set = false;
-    int ctas_per_sm = v5::MIN_CTAS;
+    int ctas_per_sm = v5plan::MIN_CTAS;
     int64_t launches = 0;
     int last_inst = -1;                    // V5ELA_INST_* of the most recent fused-kernel launch
     cudaStream_t own_stream = nullptr;     // v5ela_analyze_host with a NULL stream
@@ -36,7 +35,7 @@ struct v5ela_handle {
     void *h_table = nullptr, *d_table = nullptr;
     size_t table_cap = 0;
     cudaEvent_t ev_table = nullptr;        // the last upload out of h_table has completed
-    void *d_lane_consts = nullptr;         // 32 x mma::LaneConsts: operand fragments of the tensor-core block stage (v5ela_dctmma.cuh)
+    v5plan::LaneConsts *d_lane_consts = nullptr;   // 32 entries: operand fragments of the tensor-core block stage (v5ela_dctmma.cuh)
     int block_stage = V5ELA_BLOCKS_DEFAULT; // which build of the fused kernel analyze launches (v5ela_set_block_stage)
     size_t d_in_cap = 0, d_res_cap = 0, d_enh_cap = 0, d_rec_cap = 0;
     // spectrum path (v5ela_fft.cuh): twiddle tables for the last (width, height), DFT workspace

@@ -1,11 +1,11 @@
-// v5ela_launch.cuh — the fused kernel's __global__ entry and its host-side launcher, written once and compiled twice: by v5ela.cu
+// v5ela_launch.cuh — the fused kernel's __global__ entry and its launcher, written once and compiled twice: by v5ela.cu
 // (namespace v5: the 4-threads-per-block shared-memory-transpose block stage) and by v5ela_mma.cu (namespace v5m, V5_MMA_BLOCKS=1: the
-// tensor-core block stage). The C ABI (v5ela.cu) picks one per call through FusedArgs::..., see v5ela_set_block_stage in v5ela.h.
+// tensor-core block stage). The C ABI (v5ela.cu) plans the launch (v5ela_host.h) and picks the build per handle, see
+// v5ela_set_block_stage in v5ela.h.
 #pragma once
 #include <cuda_runtime.h>
 
 #include "v5ela.h"
-#include "v5ela_fused_args.h"
 #include "v5ela_host.h"
 #include "v5ela_workitem.cuh"
 
@@ -39,7 +39,7 @@ __global__ void __launch_bounds__(NT, MIN_CTAS) ela_fused_kernel(const __grid_co
 }
 
 // once per device: opt in to the dynamic shared memory the kernel needs
-inline cudaError_t fused_prepare()
+cudaError_t prepare()
 {
     cudaError_t e = cudaFuncSetAttribute(ela_fused_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ela_fused_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
@@ -48,105 +48,19 @@ inline cudaError_t fused_prepare()
     return e;
 }
 
-// Fills the kernel parameters, picks the instantiation and launches. Returns 0, -1 (bad arguments), -2 (batch too large) or a
-// positive cudaError_t. a.inst / a.total report what was (or, with a.check_only, would be) launched.
-inline int fused_launch(v5_fused_args &a)
+// Launches instantiation `inst` (v5plan::choose_instantiation) over the `total` work items of the plan p, on at most max_ctas
+// persistent CTAs; p.ticket must be zeroed before on the same stream, and a ragged plan's frame table uploaded. ev_start / ev_stop
+// (optional) are recorded right around the kernel. Returns 0 or a positive cudaError_t.
+int launch(const KParams &p, int inst, long long total, int max_ctas, cudaStream_t st, cudaEvent_t ev_start, cudaEvent_t ev_stop)
 {
-    KParams p;
-    if (fill_params(p, a.rgb, a.n, a.h, a.w, a.frame_stride, a.row_stride, a.records, a.residual, a.quality, a.seg_rows, a.target_items, a.tune) != 0)
-        return -1;
-    p.tex_hist = a.tex_hist;
-    p.ticket = a.ticket;
-    p.lane_consts = static_cast<const mma::LaneConsts *>(a.lane_consts);
-    const long long total = total_work_items(p);
-    if (total > 0x7fffffffLL) return -2;
-    a.total = total;
-    const int grid = total < a.max_ctas ? (int)total : a.max_ctas;
-    a.inst = p.tex_hist ? V5ELA_INST_TEXHIST : (fast_path_ok(p) ? V5ELA_INST_FAST : V5ELA_INST_GENERAL);
-    if (a.check_only) return 0;
-    if (a.ev_start) cudaEventRecord(a.ev_start, a.stream);
-    if (a.inst == V5ELA_INST_TEXHIST) ela_fused_kernel<false, true><<<grid, NT, sizeof(Smem), a.stream>>>(p, (int)total);
-    else if (a.inst == V5ELA_INST_FAST) ela_fused_kernel<true, false><<<grid, NT, sizeof(Smem), a.stream>>>(p, (int)total);
-    else ela_fused_kernel<false, false><<<grid, NT, sizeof(Smem), a.stream>>>(p, (int)total);
+    const int grid = total < max_ctas ? (int)total : max_ctas;
+    if (ev_start) cudaEventRecord(ev_start, st);
+    if (inst == v5plan::INST_RAGGED) ela_fused_kernel<false, false, true><<<grid, NT, sizeof(Smem), st>>>(p, (int)total);
+    else if (inst == V5ELA_INST_TEXHIST) ela_fused_kernel<false, true><<<grid, NT, sizeof(Smem), st>>>(p, (int)total);
+    else if (inst == V5ELA_INST_FAST) ela_fused_kernel<true, false><<<grid, NT, sizeof(Smem), st>>>(p, (int)total);
+    else ela_fused_kernel<false, false><<<grid, NT, sizeof(Smem), st>>>(p, (int)total);
     const cudaError_t e = cudaGetLastError();
-    if (a.ev_stop) cudaEventRecord(a.ev_stop, a.stream);
-    return e == cudaSuccess ? 0 : (int)e;
-}
-
-
-// Ragged batch: n frames of different sizes in one launch (v5ela_analyze_ragged). Fills `table` (host memory, n FrameDesc =
-// v5_ragged_args::table_bytes(n) bytes) for the caller to upload to a.d_table BEFORE the launch on the same stream: call with
-// check_only = 1 first (validates, fills the table and a.total), upload, then again with check_only = 0.
-inline int fused_launch_ragged(v5_ragged_args &a)
-{
-    static_assert(sizeof(FrameDesc) == V5_RAGGED_DESC_BYTES, "v5_ragged_args::table_bytes");
-    if (!a.frames || !a.records || a.n <= 0 || !a.table || a.quality < 1 || a.quality > 100) return -1;
-    FrameDesc *tab = static_cast<FrameDesc *>(a.table);
-    if (a.check_only) {
-        long long columns = 0;
-        for (int i = 0; i < a.n; i++) {
-            const v5ela_frame_desc &f = a.frames[i];
-            if (!f.rgb || f.height <= 0 || f.width <= 0 || f.height > 65536 || f.width > 65536 || (int64_t)f.height * f.width > 0x7fffffffLL ||
-                f.row_stride_bytes < (int64_t)3 * f.width)
-                return -1;
-            columns += ((f.width + 15) / 16 + TW_MAX - 1) / TW_MAX;
-        }
-        // as few segments per frame as still give >= 2 work items per resident CTA (fill_params' rule), down to 4 MCU rows each
-        const long long ctas = (a.target_items + 1) / 2;
-        long long want_segs = a.target_items > 0 ? (2 * ctas + columns - 1) / columns : 4;
-        if (want_segs < 1) want_segs = 1;
-        long long items4 = 0;                                   // work items with the default strips and these segments
-        for (int i = 0; i < a.n; i++) {
-            const int mw = (a.frames[i].width + 15) / 16, mh = (a.frames[i].height + 15) / 16;
-            long long sr = (mh + want_segs - 1) / want_segs;
-            sr = sr < 4 ? 4 : sr;
-            items4 += (long long)((mw + TW_MAX - 1) / TW_MAX) * ((mh + sr - 1) / sr);
-        }
-        long long total = 0;
-        for (int i = 0; i < a.n; i++) {
-            const v5ela_frame_desc &f = a.frames[i];
-            FrameDesc &d = tab[i];
-            uint8_t *resid = f.residual ? f.residual : f.enhanced;                // an enhanced map alone: the residual is formed in place
-            d.rgb = f.rgb;
-            d.resid = resid;
-            d.row_stride = f.row_stride_bytes;
-            d.h = f.height; d.w = f.width;
-            d.mw = (f.width + 15) / 16; d.mh = (f.height + 15) / 16;
-            d.n_strips = (d.mw + TW_MAX - 1) / TW_MAX;
-            int seg_rows = a.seg_rows;
-            if (seg_rows <= 0) {
-                seg_rows = (int)((d.mh + want_segs - 1) / want_segs);
-                if (seg_rows < 4) seg_rows = 4;
-            }
-            d.n_segs = (d.mh + seg_rows - 1) / seg_rows;
-            if (a.seg_rows <= 0 && a.target_items > 0 && items4 < a.target_items) d.n_strips = widen_strips(d.n_strips, d.mw, items4, a.target_items);
-            if (total > 0x7fffffffLL) return -2;
-            d.work_base = (uint32_t)total;
-            total += (long long)d.n_strips * d.n_segs;
-            const bool vec = ((reinterpret_cast<uintptr_t>(f.rgb) | (uintptr_t)f.row_stride_bytes) & 15) == 0;
-            const bool rvec = resid && ((reinterpret_cast<uintptr_t>(resid) | (uintptr_t)(3 * f.width)) & 15) == 0;
-            d.flags = (vec ? 1u : 0u) | (rvec ? 2u : 0u);
-        }
-        if (total > 0x7fffffffLL) return -2;
-        a.total = total;
-        return 0;
-    }
-    KParams p;
-    memset(&p, 0, sizeof(p));
-    p.records = a.records;
-    p.n = a.n;
-    p.ticket = a.ticket;
-    p.lane_consts = static_cast<const mma::LaneConsts *>(a.lane_consts);
-    p.frames = static_cast<const FrameDesc *>(a.d_table);
-    uint16_t ql[64], qc[64];
-    quant_tables(a.quality, ql, qc);
-    make_quant(ql, p.q[0]);
-    make_quant(qc, p.q[1]);
-    const int grid = a.total < a.max_ctas ? (int)a.total : a.max_ctas;
-    if (a.ev_start) cudaEventRecord(a.ev_start, a.stream);
-    ela_fused_kernel<false, false, true><<<grid, NT, sizeof(Smem), a.stream>>>(p, (int)a.total);
-    const cudaError_t e = cudaGetLastError();
-    if (a.ev_stop) cudaEventRecord(a.ev_stop, a.stream);
+    if (ev_stop) cudaEventRecord(ev_stop, st);
     return e == cudaSuccess ? 0 : (int)e;
 }
 

@@ -4,12 +4,3 @@
 #define V5_NS v5m
 #define V5_MMA_BLOCKS 1
 #include "v5ela_launch.cuh"
-
-namespace v5m {
-
-cudaError_t fused_prepare_mma() { return fused_prepare(); }
-int fused_launch_mma(v5_fused_args &a) { return fused_launch(a); }
-int fused_launch_ragged_mma(v5_ragged_args &a) { return fused_launch_ragged(a); }
-bool lane_consts_host(void *dst128x32) { return mma::make_lane_consts(static_cast<mma::LaneConsts *>(dst128x32)); }
-
-}  // namespace v5m

@@ -126,7 +126,7 @@ static int v5ela_jpeg_encode_impl(v5ela_handle *h, const uint8_t *d_img, int n, 
 
     const v5j::EncGeo g = v5j::enc_geo(height, width, channels);
     uint16_t ql[64], qc[64];
-    v5::quant_tables(quality, ql, qc);
+    v5plan::quant_tables(quality, ql, qc);
     const std::vector<uint8_t> header = v5j::file_header(height, width, channels, ql, qc);
     if (!s->d_enc_tabs) {
         v5j::EncTables tabs;

@@ -26,7 +26,7 @@ constexpr int ENC_NT = 384;            // coef_kernel: 96 blocks x 4 threads
 constexpr int ENC_TM = 16;             // MCUs (colour) per CTA strip; 96 blocks per strip in either mode
 constexpr int ENC_BLOCKS = 96;
 
-struct EncQuant {                      // exact division by 8T, see v5::make_quant: q = umulhi(c + (c>>31) + bias, recip) - b
+struct EncQuant {                      // exact division by 8T, see v5plan::make_quant: q = umulhi(c + (c>>31) + bias, recip) - b
     uint32_t recip[64];
     int32_t bias[64];
     int32_t b[64];

@@ -3,6 +3,7 @@ from __future__ import annotations
 
 import ctypes
 import os
+import threading
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # V5ELA_LIB: development knob — load another build of the SAME library (kernel-tuning variants under profiles/variants/).
@@ -224,3 +225,18 @@ class Handle:
             self.close()
         except Exception:
             pass
+
+
+_tls = threading.local()
+
+
+def get_handle(device_index: int) -> Handle:
+    """One library handle per (thread, device), shared by every entry point of the package; handles are not thread-safe
+    (include/v5ela.h)."""
+    cache = getattr(_tls, "handles", None)
+    if cache is None:
+        cache = _tls.handles = {}
+    h = cache.get(device_index)
+    if h is None:
+        h = cache[device_index] = Handle(device_index)
+    return h

@@ -5,23 +5,9 @@ There is no CPU path: tensors must live on a CUDA device and the library must lo
 """
 from __future__ import annotations
 
-import threading
-
 from . import _abi
+from ._abi import get_handle
 from .records import RECORD_BYTES
-
-_tls = threading.local()
-
-
-def get_handle(device_index: int) -> "_abi.Handle":
-    """One library handle per (thread, device); handles are not thread-safe (include/v5ela.h)."""
-    cache = getattr(_tls, "handles", None)
-    if cache is None:
-        cache = _tls.handles = {}
-    h = cache.get(device_index)
-    if h is None:
-        h = cache[device_index] = _abi.Handle(device_index)
-    return h
 
 
 def analyze_batch(frames, quality: int = 90, want_residual: bool = False, want_enhanced: bool = False,

@@ -5,24 +5,10 @@ the records / residual / enhanced maps copied back. No CPU implementation exists
 """
 from __future__ import annotations
 
-import threading
-
 import numpy as np
 
-from . import _abi
+from ._abi import get_handle
 from .records import RECORD_DTYPE
-
-_tls = threading.local()
-
-
-def _handle(device: int) -> "_abi.Handle":
-    cache = getattr(_tls, "handles", None)
-    if cache is None:
-        cache = _tls.handles = {}
-    h = cache.get(device)
-    if h is None:
-        h = cache[device] = _abi.Handle(device)
-    return h
 
 
 def analyze_frames_host(frames: np.ndarray, quality: int = 90, want_residual: bool = False, want_enhanced: bool = False,
@@ -37,7 +23,7 @@ def analyze_frames_host(frames: np.ndarray, quality: int = 90, want_residual: bo
     enhanced = np.empty_like(frames) if want_enhanced else None
     if n == 0 or h == 0 or w == 0:
         return recs, residual, enhanced
-    hd = _handle(device)
+    hd = get_handle(device)
     if hd.quality != quality:
         hd.set_quality(quality)
     hd.analyze_host(frames.ctypes.data, n, h, w, recs.ctypes.data,
@@ -69,7 +55,7 @@ def analyze_ragged_host(frames, quality: int = 90, want_residual: bool = False, 
         descs[i].row_stride_bytes = a.strides[0]
         descs[i].residual = residual[i].ctypes.data if residual is not None else None
         descs[i].enhanced = enhanced[i].ctypes.data if enhanced is not None else None
-    hd = _handle(device)
+    hd = get_handle(device)
     if hd.quality != quality:
         hd.set_quality(quality)
     hd.analyze_ragged_host(descs, n, recs.ctypes.data)
@@ -87,5 +73,5 @@ def spectrum_host(gray: np.ndarray, device: int = 0) -> np.ndarray:
     out = np.empty_like(g)
     n, h, w = g.shape
     if n and h and w:
-        _handle(device).spectrum_host(g.ctypes.data, n, h, w, out.ctypes.data)
+        get_handle(device).spectrum_host(g.ctypes.data, n, h, w, out.ctypes.data)
     return out[0] if single else out

@@ -64,8 +64,6 @@ def bound(h: int, w: int, channels: int) -> int:
 
 def encode_host(images: np.ndarray, quality: int, device: int = 0, capacity: int | None = None):
     """images: (N, H, W) gray or (N, H, W, 3) RGB uint8 host array -> list of N bytes objects (complete JPEG files)."""
-    from .host import _handle
-
     img = np.ascontiguousarray(images, dtype=np.uint8)
     if img.ndim not in (3, 4) or (img.ndim == 4 and img.shape[-1] != 3):
         raise ValueError("images must have shape (N, H, W) or (N, H, W, 3)")
@@ -76,7 +74,7 @@ def encode_host(images: np.ndarray, quality: int, device: int = 0, capacity: int
     cap = int(capacity or default_capacity(h, w, ch))
     out = np.empty((n, cap), np.uint8)
     sizes = np.zeros(n, np.int32)
-    _handle(device).jpeg_encode_host(img.ctypes.data, n, h, w, ch, int(quality), out.ctypes.data, cap, sizes.ctypes.data)
+    _abi.get_handle(device).jpeg_encode_host(img.ctypes.data, n, h, w, ch, int(quality), out.ctypes.data, cap, sizes.ctypes.data)
     if (sizes > cap).any():
         if capacity is None:
             return encode_host(images, quality, device, bound(h, w, ch))
@@ -89,8 +87,6 @@ def encode_batch(images, quality: int, capacity: int | None = None):
     on the same device, asynchronous on the current stream. sizes[i] > capacity marks a file that did not fit."""
     import torch
 
-    from .batch import get_handle
-
     if not images.is_cuda or images.dtype != torch.uint8:
         raise ValueError("encode_batch needs a uint8 CUDA tensor")
     ch = 3 if images.dim() == 4 else 1
@@ -102,7 +98,7 @@ def encode_batch(images, quality: int, capacity: int | None = None):
     out = torch.empty((n, cap), dtype=torch.uint8, device=images.device)
     sizes = torch.zeros(n, dtype=torch.int32, device=images.device)
     if n:
-        hd = get_handle(images.device.index or 0)
+        hd = _abi.get_handle(images.device.index or 0)
         hd.jpeg_encode(images.data_ptr(), n, h, w, ch, images.stride(0), images.stride(1), int(quality), out.data_ptr(), cap,
                        sizes.data_ptr(), torch.cuda.current_stream(images.device).cuda_stream)
     return out, sizes
@@ -110,8 +106,6 @@ def encode_batch(images, quality: int, capacity: int | None = None):
 
 def decode_host(files, want_rgb: bool = True, want_gray: bool = False, device: int = 0):
     """files: list of bytes -> list of dicts {'rgb': (H,W,3), 'gray': (H,W)} (keys as requested), host arrays."""
-    from .host import _handle
-
     n = len(files)
     if n == 0:
         return []
@@ -122,7 +116,7 @@ def decode_host(files, want_rgb: bool = True, want_gray: bool = False, device: i
     rgb = np.empty(3 * int(offs[-1]), np.uint8) if want_rgb else None
     gray = np.empty(int(offs[-1]), np.uint8) if want_gray else None
     keep, ptrs, lens = table
-    _handle(device).jpeg_decode_host(ptrs, lens, n, rgb.ctypes.data if want_rgb else None, None,
+    _abi.get_handle(device).jpeg_decode_host(ptrs, lens, n, rgb.ctypes.data if want_rgb else None, None,
                                      gray.ctypes.data if want_gray else None, None)
     del keep
     out = []
@@ -142,8 +136,6 @@ def decode_batch(files, device=0, want_rgb: bool = True, want_gray: bool = False
     staged before the call returns, files that are views into pinned memory are read asynchronously (keep the arena alive)."""
     import torch
 
-    from .batch import get_handle
-
     n = len(files)
     dev = torch.device("cuda", device) if not isinstance(device, torch.device) else device
     table = _file_table(files)
@@ -157,7 +149,7 @@ def decode_batch(files, device=0, want_rgb: bool = True, want_gray: bool = False
     if want_gray:
         out["gray"] = torch.empty((n, h, w), dtype=torch.uint8, device=dev)
     keep, ptrs, lens = table
-    (handle or get_handle(dev.index or 0)).jpeg_decode(ptrs, lens, n, out["rgb"].data_ptr() if want_rgb else None, None,
+    (handle or _abi.get_handle(dev.index or 0)).jpeg_decode(ptrs, lens, n, out["rgb"].data_ptr() if want_rgb else None, None,
                                            out["gray"].data_ptr() if want_gray else None, None, out["status"].data_ptr(),
                                            torch.cuda.current_stream(dev).cuda_stream)
     del keep

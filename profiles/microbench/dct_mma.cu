@@ -233,8 +233,8 @@ static void make_lane_consts(LaneConsts lc[32])
 // position (8 u + v) ^ (u & 1) — two LDS.128 per thread, bank-conflict free; unbias absorbs -OFF2
 static void make_qswz(const uint16_t tab[64], v5::QEntry out[64])
 {
-    v5::QuantTab qt;
-    v5::make_quant(tab, qt);
+    v5plan::QuantTab qt;
+    v5plan::make_quant(tab, qt);
     for (int u = 0; u < 8; u++)
         for (int v = 0; v < 8; v++) {
             const int nat = 8 * v + u;
@@ -683,7 +683,7 @@ int main(int argc, char **argv)
         long long bad = 0, total = 0;
         for (int quality : {1, 10, 50, 75, 90, 95, 100}) {
             uint16_t luma[64], chroma[64];
-            v5::quant_tables(quality, luma, chroma);
+            v5plan::quant_tables(quality, luma, chroma);
             for (int comp = 0; comp < 2; comp++) {
                 const uint16_t *tab = comp ? chroma : luma;
                 v5::QEntry qs[64];
@@ -747,12 +747,12 @@ int main(int argc, char **argv)
     for (int quality : {90, 1, 100, 50}) {
         for (int comp = 0; comp < 2; comp++) {
             uint16_t luma[64], chroma[64];
-            v5::quant_tables(quality, luma, chroma);
+            v5plan::quant_tables(quality, luma, chroma);
             const uint16_t *tab = comp ? chroma : luma;
             v5::QEntry qs[64], qn[64];
             make_qswz(tab, qs);
-            v5::QuantTab qt;
-            v5::make_quant(tab, qt);
+            v5plan::QuantTab qt;
+            v5plan::make_quant(tab, qt);
             for (int i = 0; i < 64; i++) qn[i] = v5::QEntry{qt.recip[i], qt.bias[i], qt.t[i], qt.unbias[i]};
             CK(cudaMemcpy(d_qs, qs, sizeof(qs), cudaMemcpyHostToDevice));
             CK(cudaMemcpy(d_qn, qn, sizeof(qn), cudaMemcpyHostToDevice));

@@ -40,7 +40,7 @@ def main():
     counts = {"records_only_fast": 0, "ragged_frames": 0}
     t0 = time.time()
     pending, crops = [], []
-    hd = v5host._handle(0)
+    hd = v5host.get_handle(0)
     for it in range(cases):
         hd.block_stage = "mma" if it % 2 else "smem"                      # both builds of the block stage, alternating
         big = it % 20 == 0

@@ -20,7 +20,7 @@ extern "C" int64_t v5jemu_encode(const uint8_t *img, int h, int w, int channels,
 {
     const EncGeo g = enc_geo(h, w, channels);
     uint16_t ql[64], qc[64];
-    v5::quant_tables(quality, ql, qc);
+    v5plan::quant_tables(quality, ql, qc);
     std::vector<int16_t> coef((size_t)g.blocks * 64);
     CoefParams p;
     memset(&p, 0, sizeof(p));

@@ -136,10 +136,11 @@ def test_emulated_kernel_vs_reference_goldens(emu):
         assert record_matches_golden(recs[0], case) == []
 
 
-@pytest.mark.parametrize("seg", [0, 2])
-def test_emulated_ragged_instantiation_vs_oracle(emu, seg):
-    """v5ela_analyze_ragged's kernel instantiation: frames of different sizes share one work-item space (binary search over the
-    frame table per work item); every frame against the oracle."""
+@pytest.mark.parametrize("seg,target", [(0, 0), (2, 0), (0, 592), (2, 592)], ids=["0", "2", "0-592", "2-592"])
+def test_emulated_ragged_instantiation_vs_oracle(emu, seg, target):
+    """v5ela_analyze_ragged's kernel instantiation over the library's ragged plan (csrc/v5ela_host.h plan_ragged): frames of different
+    sizes share one work-item space (binary search over the frame table per work item); every frame against the oracle. target=592
+    (2 x 148 SMs x 2 CTAs) is the plan the library launches on a B200: short segments and, for this small batch, narrowed strips."""
     import ctypes
 
     sizes = [(1, 1), (17, 33), (16, 16), (40, 48), (33, 497), (9, 976), (100, 1000), (2, 3)]
@@ -150,8 +151,12 @@ def test_emulated_ragged_instantiation_vs_oracle(emu, seg):
     recs = np.zeros(len(sizes), RECORD_DTYPE)
     res = np.zeros_like(blob)
     u8p = ctypes.POINTER(ctypes.c_uint8)
-    rc = emu.lib.v5emu_analyze_ragged(blob.ctypes.data_as(u8p), hw.ctypes.data_as(ctypes.POINTER(ctypes.c_int)), len(sizes), 90,
-                                      recs.ctypes.data_as(ctypes.c_void_p), res.ctypes.data_as(u8p), seg)
+    try:
+        emu.lib.v5emu_set_target_items(target)
+        rc = emu.lib.v5emu_analyze_ragged(blob.ctypes.data_as(u8p), hw.ctypes.data_as(ctypes.POINTER(ctypes.c_int)), len(sizes), 90,
+                                          recs.ctypes.data_as(ctypes.c_void_p), res.ctypes.data_as(u8p), seg)
+    finally:
+        emu.lib.v5emu_set_target_items(0)
     assert rc == 0
     off = 0
     for i, f in enumerate(frames):
@@ -159,6 +164,70 @@ def test_emulated_ragged_instantiation_vs_oracle(emu, seg):
         assert recs[i].tobytes() == o["record"].tobytes(), sizes[i]
         assert np.array_equal(res[off:off + f.size].reshape(f.shape), o["residual"]), sizes[i]
         off += f.size
+
+
+def ragged_plan(lib, sizes, seg, target):
+    """csrc/v5ela_host.h plan_ragged of frames `sizes` -> (total work items, [(n_strips, n_segs)] per frame); checks work_base."""
+    import ctypes
+
+    hw = np.array(sizes, np.int32).reshape(-1)
+    plan = np.zeros(3 * len(sizes), np.int32)
+    total = ctypes.c_longlong(-1)
+    rc = lib.v5emu_plan_ragged(hw.ctypes.data_as(ctypes.c_void_p), len(sizes), seg, target, plan.ctypes.data_as(ctypes.c_void_p),
+                               ctypes.byref(total))
+    assert rc == 0
+    plan = plan.reshape(-1, 3)
+    items = [int(s) * int(g) for s, g, _ in plan]
+    assert list(plan[:, 2]) == [sum(items[:i]) for i in range(len(items))] and total.value == sum(items)
+    return total.value, [(int(s), int(g)) for s, g, _ in plan]
+
+
+def test_ragged_plan_of_three_face_crops(emu):
+    """DESIGN.md 4.1: three 257x301 crops on a B200 (target 592) are 4 strips x 5 segments each, 60 work items."""
+    assert ragged_plan(emu.lib, [(257, 301)] * 3, 0, 592) == (60, [(4, 5)] * 3)
+
+
+def test_ragged_plan_of_equal_frames_is_the_uniform_plan(emu):
+    """n frames of one size: plan_ragged cuts them as fill_params does wherever fill_params has no tail split (the ragged plan has
+    none); an explicit segment height is taken as given by both."""
+    import ctypes
+
+    compared = 0
+    for h, w in [(257, 301), (1080, 1920), (64, 1000), (300, 32), (17, 33), (2160, 3840)]:
+        for n in (1, 3, 5, 40):
+            for target in (16, 592, 888):
+                for seg in (0, 3):
+                    uni = np.zeros(4, np.int32)
+                    assert emu.lib.v5emu_plan_uniform(n, h, w, seg, target, uni.ctypes.data_as(ctypes.c_void_p)) == 0
+                    if uni[2] != n:                           # split_frame < n: a tail split
+                        continue
+                    _, plan = ragged_plan(emu.lib, [(h, w)] * n, seg, target)
+                    assert plan == [(int(uni[0]), int(uni[1]))] * n, (h, w, n, target, seg)
+                    compared += 1
+    assert compared >= 100
+
+
+# Ragged plans of a few mixed batches, pinned: a change to the rule changes how v5ela_analyze_ragged cuts its work and with it its
+# speed, which wants a measurement of its own. (batch, seg_rows, target_items) -> (total work items, [(n_strips, n_segs)] per frame)
+RAGGED_BATCHES = {"faces": [(257, 301), (180, 160), (320, 240)],
+                  "emu": [(1, 1), (17, 33), (16, 16), (40, 48), (33, 497), (9, 976), (100, 1000), (2, 3)],
+                  "big": [(1080, 1920), (720, 1280), (64, 64), (2160, 3840)]}
+RAGGED_PLANS = {
+    ("faces", 0, 0): (11, [(1, 4), (1, 3), (1, 4)]),
+    ("emu", 0, 0): (16, [(1, 1), (1, 1), (1, 1), (1, 1), (2, 1), (3, 1), (3, 2), (1, 1)]),
+    ("faces", 0, 16): (26, [(2, 5), (2, 3), (2, 5)]),
+    ("big", 0, 16): (16, [(4, 1), (3, 1), (1, 1), (8, 1)]),
+    ("faces", 0, 592): (41, [(4, 5), (2, 3), (3, 5)]),
+    ("emu", 0, 592): (58, [(1, 1), (1, 1), (1, 1), (1, 1), (8, 1), (15, 1), (15, 2), (1, 1)]),
+    ("big", 0, 592): (753, [(8, 17), (6, 12), (1, 1), (16, 34)]),
+    ("faces", 2, 592): (25, [(1, 9), (1, 6), (1, 10)]),
+    ("big", 0, 888): (1129, [(12, 17), (9, 12), (1, 1), (24, 34)]),
+}
+
+
+def test_ragged_plans_of_mixed_batches(emu):
+    for (batch, seg, target), want in RAGGED_PLANS.items():
+        assert ragged_plan(emu.lib, RAGGED_BATCHES[batch], seg, target) == want, (batch, seg, target)
 
 
 @pytest.mark.parametrize("hw", [(257, 301), (40, 1000), (64, 96), (300, 48)])
