@@ -10,6 +10,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
+#include <utility>
 #include <vector>
 
 #include "v5ela.h"
@@ -156,8 +157,8 @@ static int launch_fused(v5ela_handle *h, const v5plan::KParams &p, int inst, lon
 {
     const bool prof = h->profiling && h->prof_used + 2 <= h->prof_events.size();
     const int rc = fused_builds[h->block_stage].launch(p, inst, total, h->sm_count * h->ctas_per_sm, st,
-                                                       prof ? h->prof_events[h->prof_used] : nullptr,
-                                                       prof ? h->prof_events[h->prof_used + 1] : nullptr);
+                                                       prof ? static_cast<cudaEvent_t>(h->prof_events[h->prof_used]) : nullptr,
+                                                       prof ? static_cast<cudaEvent_t>(h->prof_events[h->prof_used + 1]) : nullptr);
     if (rc != 0) return fail(h, V5ELA_ERR_CUDA, "fused kernel launch: %s", cudaGetErrorString((cudaError_t)rc));
     h->last_inst = inst == v5plan::INST_RAGGED ? V5ELA_INST_GENERAL : inst;
     if (prof) h->prof_used += 2;
@@ -206,9 +207,8 @@ int v5ela_create(int device, v5ela_handle **out)
     }
     {   // per-lane operand fragments of the tensor-core block stage: 32 x 128 bytes, fixed for the life of the handle
         v5plan::LaneConsts lc[32];
-        if (!v5::mma::make_lane_consts(lc) || cudaMalloc(&h->d_lane_consts, sizeof(lc)) != cudaSuccess ||
+        if (!v5::mma::make_lane_consts(lc) || h->d_lane_consts.ensure(h, sizeof(lc)) != 0 ||
             cudaMemcpy(h->d_lane_consts, lc, sizeof(lc), cudaMemcpyHostToDevice) != cudaSuccess) {
-            cudaFree(h->d_lane_consts);
             delete h;
             return V5ELA_ERR_CUDA;
         }
@@ -231,32 +231,7 @@ int v5ela_create(int device, v5ela_handle **out)
 int v5ela_destroy(v5ela_handle *h)
 {
     if (!h) return V5ELA_ERR_INVALID;
-    DeviceGuard guard(h->device);
-    if (h->own_stream) cudaStreamDestroy(h->own_stream);
-    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    if (h->work_stream) cudaStreamDestroy(h->work_stream);
-    for (cudaEvent_t e : {h->ev_fork, h->ev_join_copy, h->ev_join_work})
-        if (e) cudaEventDestroy(e);
-    for (cudaEvent_t e : h->ev_chunk) cudaEventDestroy(e);
-    for (cudaEvent_t e : h->prof_events) cudaEventDestroy(e);
-    cudaFree(h->d_in);
-    cudaFree(h->d_res);
-    cudaFree(h->d_enh);
-    cudaFree(h->d_rec);
-    if (h->ev_scratch) cudaEventDestroy(h->ev_scratch);
-    if (h->ev_table) cudaEventDestroy(h->ev_table);
-    if (h->h_table) cudaFreeHost(h->h_table);
-    cudaFree(h->d_table);
-    cudaFree(h->d_ticket);
-    cudaFree(h->d_lane_consts);
-    cudaFree(h->tw_w);
-    cudaFree(h->tw_h);
-    cudaFree(h->d_g);
-    cudaFree(h->d_ms);
-    cudaFree(h->d_minmax);
-    cudaFree(h->d_gray);
-    cudaFree(h->d_spec);
-    v5jpeg_release(h);
+    DeviceGuard guard(h->device);                                // the members release what they own on the handle's device
     delete h;
     return V5ELA_OK;
 }
@@ -296,7 +271,7 @@ int v5ela_analyze_ex(v5ela_handle *h, const uint8_t *d_rgb, int n, int height, i
     DeviceGuard guard(h->device);
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     ScratchOrder order(h, st);                                  // the ticket counter is handle-owned
-    if (!h->d_ticket) V5_CUDA(h, cudaMalloc(&h->d_ticket, sizeof(unsigned int)));
+    if (const int rc = h->d_ticket.ensure(h, sizeof(unsigned int))) return rc;
     v5plan::KParams p;
     if (v5plan::fill_params(p, d_rgb, n, height, width, frame_stride_bytes, row_stride_bytes, static_cast<v5ela_record *>(d_records),
                             d_residual, h->quality, h->seg_rows, 2 * h->sm_count * h->ctas_per_sm, h->decomp_set ? h->decomp : nullptr) != 0)
@@ -320,27 +295,24 @@ int v5ela_analyze_ragged(v5ela_handle *h, const v5ela_frame_desc *frames_host, i
     DeviceGuard guard(h->device);
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     ScratchOrder order(h, st);                                  // ticket counter and frame table are handle-owned
-    if (!h->d_ticket) V5_CUDA(h, cudaMalloc(&h->d_ticket, sizeof(unsigned int)));
+    int rc;
+    if ((rc = h->d_ticket.ensure(h, sizeof(unsigned int)))) return rc;
     const size_t desc_bytes = (sizeof(v5plan::FrameDesc) * (size_t)n + 15) / 16 * 16, need = desc_bytes + sizeof(v5::EnhDesc) * (size_t)n;
-    if (h->table_cap < need) {
+    if (h->h_table.capacity() < need || h->d_table.capacity() < need) {   // the staging buffer and its device copy grow together
         if (h->ev_table) cudaEventSynchronize(h->ev_table);
-        if (h->h_table) cudaFreeHost(h->h_table);
-        cudaFree(h->d_table);
-        h->h_table = h->d_table = nullptr;
-        h->table_cap = 0;
+        h->h_table.reset();
+        h->d_table.reset();
         const size_t cap = need < 4096 ? 4096 : need * 2;
-        V5_CUDA(h, cudaMallocHost(&h->h_table, cap));
-        V5_CUDA(h, cudaMalloc(&h->d_table, cap));
-        h->table_cap = cap;
+        if ((rc = h->h_table.ensure(h, need, cap)) || (rc = h->d_table.ensure(h, cap))) return rc;
     }
-    if (!h->ev_table) V5_CUDA(h, cudaEventCreateWithFlags(&h->ev_table, cudaEventDisableTiming));
+    V5_CUDA(h, h->ev_table.create());
     V5_CUDA(h, cudaEventSynchronize(h->ev_table));              // the previous call's upload has left the staging buffer
     long long total = 0;
-    int rc = v5plan::plan_ragged(static_cast<v5plan::FrameDesc *>(h->h_table), frames_host, n, h->seg_rows,
-                                       2 * h->sm_count * h->ctas_per_sm, &total);
+    rc = v5plan::plan_ragged(reinterpret_cast<v5plan::FrameDesc *>(static_cast<uint8_t *>(h->h_table)), frames_host, n, h->seg_rows,
+                             2 * h->sm_count * h->ctas_per_sm, &total);
     if (rc == -1) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_ragged: bad pointer, size or stride in a frame descriptor%s");
     if (rc == -2) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_ragged: batch too large%s");
-    v5::EnhDesc *et = reinterpret_cast<v5::EnhDesc *>(static_cast<char *>(h->h_table) + desc_bytes);
+    v5::EnhDesc *et = reinterpret_cast<v5::EnhDesc *>(h->h_table + desc_bytes);
     bool any_enh = false;
     for (int i = 0; i < n; i++) {
         const v5ela_frame_desc &f = frames_host[i];
@@ -359,40 +331,28 @@ int v5ela_analyze_ragged(v5ela_handle *h, const v5ela_frame_desc *frames_host, i
     p.n = n;
     p.ticket = h->d_ticket;
     p.lane_consts = h->d_lane_consts;
-    p.frames = static_cast<const v5plan::FrameDesc *>(h->d_table);
+    p.frames = reinterpret_cast<const v5plan::FrameDesc *>(static_cast<uint8_t *>(h->d_table));
     v5plan::fill_quant(p.q, h->quality);
     if ((rc = launch_fused(h, p, v5plan::choose_instantiation(p), total, st))) return rc;
     if (any_enh) {
         if (n > 65535) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_ragged: more than 65535 frames with enhanced maps%s");
         v5::ela_enhance_ragged_kernel<<<dim3(32, (unsigned)n), 256, 0, st>>>(
-            reinterpret_cast<const v5::EnhDesc *>(static_cast<const char *>(h->d_table) + desc_bytes), static_cast<const v5ela_record *>(d_records));
+            reinterpret_cast<const v5::EnhDesc *>(h->d_table + desc_bytes), static_cast<const v5ela_record *>(d_records));
         V5_CUDA(h, cudaGetLastError());
         h->launches += 1;
     }
     return V5ELA_OK;
 }
 
-static int analyze_ragged_host_impl(v5ela_handle *h, const v5ela_frame_desc *frames_host, int n, void *records_host);
-
 int v5ela_analyze_ragged_host(v5ela_handle *h, const v5ela_frame_desc *frames_host, int n, void *records_host)
-{
-    try {                                                       // std::vector below: nothing may unwind through the C ABI
-        return analyze_ragged_host_impl(h, frames_host, n, records_host);
-    } catch (const std::bad_alloc &) {
-        return fail(h, V5ELA_ERR_NOMEM, "out of host memory%s");
-    } catch (...) {
-        return fail(h, V5ELA_ERR_INVALID, "host-side failure%s");
-    }
-}
-
-static int analyze_ragged_host_impl(v5ela_handle *h, const v5ela_frame_desc *frames_host, int n, void *records_host)
-{
+try {
     if (!h) return V5ELA_ERR_INVALID;
     if (n == 0) return V5ELA_OK;
     if (!frames_host || !records_host || n < 0) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_ragged_host: bad pointer or count%s");
     DeviceGuard guard(h->device);
-    if (!h->own_stream) V5_CUDA(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
-    cudaStream_t st = h->own_stream;
+    int rc;
+    cudaStream_t st;
+    if ((rc = internal_stream(h, &st))) return rc;
     ScratchOrder order(h, st);
     // device arena: per frame the pixels (rows packed), then the maps it asked for; every part 256-byte aligned
     std::vector<v5ela_frame_desc> dev((size_t)n);
@@ -407,9 +367,8 @@ static int analyze_ragged_host_impl(v5ela_handle *h, const v5ela_frame_desc *fra
         off_res[i] = total; total += (f.residual || f.enhanced) ? bytes : 0;
         off_enh[i] = total; total += f.enhanced ? bytes : 0;
     }
-    int rc;
-    if ((rc = ensure(h, (void **)&h->d_in, &h->d_in_cap, total))) return rc;
-    if ((rc = ensure(h, &h->d_rec, &h->d_rec_cap, sizeof(v5ela_record) * (size_t)n))) return rc;
+    if ((rc = h->d_in.ensure(h, total))) return rc;
+    if ((rc = h->d_rec.ensure(h, sizeof(v5ela_record) * (size_t)n))) return rc;
     for (int i = 0; i < n; i++) {
         const v5ela_frame_desc &f = frames_host[i];
         V5_CUDA(h, cudaMemcpy2DAsync(h->d_in + off_in[i], (size_t)3 * f.width, f.rgb, (size_t)f.row_stride_bytes, (size_t)3 * f.width,
@@ -431,7 +390,7 @@ static int analyze_ragged_host_impl(v5ela_handle *h, const v5ela_frame_desc *fra
     }
     V5_CUDA(h, cudaStreamSynchronize(st));
     return V5ELA_OK;
-}
+} V5_CATCH(h)
 
 int v5ela_enhance(v5ela_handle *h, const uint8_t *d_residual, const void *d_records, int n, int height, int width,
                   uint8_t *d_enhanced, void *cuda_stream)
@@ -469,27 +428,26 @@ int v5ela_reduce_records(v5ela_handle *h, const void *d_records, int n, int grou
 
 int v5ela_analyze_host(v5ela_handle *h, const uint8_t *rgb_host, int n, int height, int width, void *records_host,
                        uint8_t *residual_host_or_null, uint8_t *enhanced_host_or_null, void *cuda_stream)
-{
+try {
     if (!h) return V5ELA_ERR_INVALID;
     if (n == 0) return V5ELA_OK;
     if (!rgb_host || !records_host || n < 0 || height <= 0 || width <= 0)
         return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_host: bad pointer or size%s");
     DeviceGuard guard(h->device);
-    if (!h->copy_stream) {
-        if (!h->own_stream) V5_CUDA(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
-        V5_CUDA(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-        V5_CUDA(h, cudaStreamCreateWithFlags(&h->work_stream, cudaStreamNonBlocking));
-        V5_CUDA(h, cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-        V5_CUDA(h, cudaEventCreateWithFlags(&h->ev_join_copy, cudaEventDisableTiming));
-        V5_CUDA(h, cudaEventCreateWithFlags(&h->ev_join_work, cudaEventDisableTiming));
-    }
+    int rc;
+    cudaStream_t own;
+    if ((rc = internal_stream(h, &own))) return rc;
+    V5_CUDA(h, h->copy_stream.create());
+    V5_CUDA(h, h->work_stream.create());
+    V5_CUDA(h, h->ev_fork.create());
+    V5_CUDA(h, h->ev_join_copy.create());
+    V5_CUDA(h, h->ev_join_work.create());
     const size_t fbytes = (size_t)height * width * 3, in_bytes = fbytes * n, rec_bytes = sizeof(v5ela_record) * (size_t)n;
     const bool want_map = residual_host_or_null || enhanced_host_or_null;
-    int rc;
-    if ((rc = ensure(h, (void **)&h->d_in, &h->d_in_cap, in_bytes))) return rc;
-    if ((rc = ensure(h, &h->d_rec, &h->d_rec_cap, rec_bytes))) return rc;
-    if (want_map && (rc = ensure(h, (void **)&h->d_res, &h->d_res_cap, in_bytes))) return rc;
-    if (enhanced_host_or_null && (rc = ensure(h, (void **)&h->d_enh, &h->d_enh_cap, in_bytes))) return rc;
+    if ((rc = h->d_in.ensure(h, in_bytes))) return rc;
+    if ((rc = h->d_rec.ensure(h, rec_bytes))) return rc;
+    if (want_map && (rc = h->d_res.ensure(h, in_bytes))) return rc;
+    if (enhanced_host_or_null && (rc = h->d_enh.ensure(h, in_bytes))) return rc;
 
     // chunking: ~64 MB of frames per chunk keeps the copy engine and the SMs both busy
     int chunk = h->host_chunk_frames > 0 ? h->host_chunk_frames : (int)((64u << 20) / fbytes);
@@ -497,30 +455,29 @@ int v5ela_analyze_host(v5ela_handle *h, const uint8_t *rgb_host, int n, int heig
     if (chunk > n) chunk = n;
     const int n_chunks = (n + chunk - 1) / chunk;
     while ((int)h->ev_chunk.size() < n_chunks) {
-        cudaEvent_t e;
-        V5_CUDA(h, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        h->ev_chunk.push_back(e);
+        Event e;
+        V5_CUDA(h, e.create());
+        h->ev_chunk.push_back(std::move(e));
     }
-    cudaStream_t user = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : h->own_stream;
+    cudaStream_t user = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : own;
     cudaStream_t cs = h->copy_stream, ws = h->work_stream;
     ScratchOrder order(h, user);                                // d_in / d_rec / d_res / d_enh and the two internal streams
     V5_CUDA(h, cudaEventRecord(h->ev_fork, user));
     V5_CUDA(h, cudaStreamWaitEvent(cs, h->ev_fork, 0));
     V5_CUDA(h, cudaStreamWaitEvent(ws, h->ev_fork, 0));
-    uint8_t *d_rec = static_cast<uint8_t *>(h->d_rec);
     for (int c = 0; c < n_chunks; c++) {
         const int f0 = c * chunk, fn = (f0 + chunk <= n ? chunk : n - f0);
         const size_t off = fbytes * f0, bytes = fbytes * fn, roff = sizeof(v5ela_record) * (size_t)f0;
         V5_CUDA(h, cudaMemcpyAsync(h->d_in + off, rgb_host + off, bytes, cudaMemcpyHostToDevice, cs));
         V5_CUDA(h, cudaEventRecord(h->ev_chunk[c], cs));
         V5_CUDA(h, cudaStreamWaitEvent(ws, h->ev_chunk[c], 0));
-        rc = v5ela_analyze(h, h->d_in + off, fn, height, width, (int64_t)fbytes, (int64_t)width * 3, d_rec + roff,
+        rc = v5ela_analyze(h, h->d_in + off, fn, height, width, (int64_t)fbytes, (int64_t)width * 3, h->d_rec + roff,
                            want_map ? h->d_res + off : nullptr, ws);
         if (rc) return rc;
         if (residual_host_or_null)
             V5_CUDA(h, cudaMemcpyAsync(residual_host_or_null + off, h->d_res + off, bytes, cudaMemcpyDeviceToHost, ws));
         if (enhanced_host_or_null) {
-            rc = v5ela_enhance(h, h->d_res + off, d_rec + roff, fn, height, width, h->d_enh + off, ws);
+            rc = v5ela_enhance(h, h->d_res + off, h->d_rec + roff, fn, height, width, h->d_enh + off, ws);
             if (rc) return rc;
             V5_CUDA(h, cudaMemcpyAsync(enhanced_host_or_null + off, h->d_enh + off, bytes, cudaMemcpyDeviceToHost, ws));
         }
@@ -532,7 +489,7 @@ int v5ela_analyze_host(v5ela_handle *h, const uint8_t *rgb_host, int n, int heig
     V5_CUDA(h, cudaStreamWaitEvent(user, h->ev_join_work, 0));
     if (!cuda_stream) V5_CUDA(h, cudaStreamSynchronize(user));
     return V5ELA_OK;
-}
+} V5_CATCH(h)
 
 // threads per CTA of the FFT kernels: 256; 512 measured no faster (profiles/r02/spectrum.txt). V5ELA_FFT_THREADS overrides
 // (tuning knob: 128 / 256 / 512)
@@ -560,13 +517,13 @@ int v5ela_spectrum(v5ela_handle *h, const uint8_t *d_gray, int n, int height, in
     const int wh = width / 2 + 1;
     int rc;
     if (h->tw_w_n != width) {
-        if ((rc = ensure(h, (void **)&h->tw_w, &h->tw_w_cap, sizeof(double2) * (size_t)width))) return rc;
+        if ((rc = h->tw_w.ensure(h, sizeof(double2) * (size_t)width))) return rc;
         v5fft::twiddle_kernel<<<(width + 255) / 256, 256, 0, st>>>(h->tw_w, width);
         h->tw_w_n = width;
         h->launches++;
     }
     if (h->tw_h_n != height) {
-        if ((rc = ensure(h, (void **)&h->tw_h, &h->tw_h_cap, sizeof(double2) * (size_t)height))) return rc;
+        if ((rc = h->tw_h.ensure(h, sizeof(double2) * (size_t)height))) return rc;
         v5fft::twiddle_kernel<<<(height + 255) / 256, 256, 0, st>>>(h->tw_h, height);
         h->tw_h_n = height;
         h->launches++;
@@ -584,9 +541,9 @@ int v5ela_spectrum(v5ela_handle *h, const uint8_t *d_gray, int n, int height, in
     if (chunk < 1) chunk = 1;
     if (chunk > n) chunk = n;
     if (chunk > 65535) chunk = 65535;
-    if ((rc = ensure(h, &h->d_g, &h->d_g_cap, per_frame * 16 * chunk))) return rc;
-    if ((rc = ensure(h, &h->d_ms, &h->d_ms_cap, per_frame * 8 * chunk))) return rc;
-    if ((rc = ensure(h, &h->d_minmax, &h->d_minmax_cap, sizeof(unsigned long long) * 2 * (size_t)chunk))) return rc;
+    if ((rc = h->d_g.ensure(h, per_frame * 16 * chunk))) return rc;
+    if ((rc = h->d_ms.ensure(h, per_frame * 8 * chunk))) return rc;
+    if ((rc = h->d_minmax.ensure(h, sizeof(unsigned long long) * 2 * (size_t)chunk))) return rc;
     const dim3 grid((wh + v5fft::TILE - 1) / v5fft::TILE, (height + v5fft::TILE - 1) / v5fft::TILE, 1);
     // Sizes with only 2/3/5 as prime factors take the shared-memory FFT; anything else (crops are arbitrary) the exact-size
     // DFT products. V5ELA_FFT=0 forces the latter (tests compare the two).
@@ -610,30 +567,26 @@ int v5ela_spectrum(v5ela_handle *h, const uint8_t *d_gray, int n, int height, in
         V5_CUDA(h, cudaMemset2DAsync(h->d_minmax, 16, 0xff, 8, (size_t)fn, st));
         if (fast) {
             v5fft::fft_rows_kernel<<<dim3((unsigned)((height + 1) / 2), (unsigned)fn), fft_threads(width), rows_smem, st>>>(
-                d_gray + (int64_t)f0 * frame_stride_bytes, frame_stride_bytes, row_stride_bytes, height, width, wh, plan_w, h->tw_w,
-                static_cast<double2 *>(h->d_g));
+                d_gray + (int64_t)f0 * frame_stride_bytes, frame_stride_bytes, row_stride_bytes, height, width, wh, plan_w, h->tw_w, h->d_g);
             V5_CUDA(h, cudaGetLastError());
             v5fft::fft_cols_kernel<<<dim3((unsigned)((wh + cc - 1) / cc), (unsigned)fn), fft_threads(cc * height), cols_smem, st>>>(
-                static_cast<const double2 *>(h->d_g), height, wh, cc, plan_h, h->tw_h, static_cast<double *>(h->d_ms),
-                static_cast<unsigned long long *>(h->d_minmax));
+                h->d_g, height, wh, cc, plan_h, h->tw_h, h->d_ms, h->d_minmax);
             V5_CUDA(h, cudaGetLastError());
         } else {
             dim3 gr = grid;
             gr.z = (unsigned)fn;
             v5fft::dft_rows_kernel<<<gr, 256, 0, st>>>(d_gray + (int64_t)f0 * frame_stride_bytes, frame_stride_bytes, row_stride_bytes,
-                                                       height, width, wh, h->tw_w, static_cast<double2 *>(h->d_g));
+                                                       height, width, wh, h->tw_w, h->d_g);
             V5_CUDA(h, cudaGetLastError());
-            v5fft::dft_cols_kernel<<<gr, 256, 0, st>>>(static_cast<const double2 *>(h->d_g), height, wh, h->tw_h,
-                                                       static_cast<double *>(h->d_ms), static_cast<unsigned long long *>(h->d_minmax));
+            v5fft::dft_cols_kernel<<<gr, 256, 0, st>>>(h->d_g, height, wh, h->tw_h, h->d_ms, h->d_minmax);
             V5_CUDA(h, cudaGetLastError());
         }
         // every CTA walks ~16 rows: the per-thread set-up (the double-precision 255 / (max - min)) is paid once per 16 pixels
         const unsigned bx = (unsigned)((width + 255) / 256);
         unsigned by = (unsigned)((height + 15) / 16);
         by = by < 1 ? 1 : (by > 65535 ? 65535 : by);
-        v5fft::spectrum_image_kernel<<<dim3(bx, by, (unsigned)fn), 256, 0, st>>>(
-            static_cast<const double *>(h->d_ms), static_cast<const unsigned long long *>(h->d_minmax), height, width, wh,
-            d_out + (int64_t)f0 * height * width);
+        v5fft::spectrum_image_kernel<<<dim3(bx, by, (unsigned)fn), 256, 0, st>>>(h->d_ms, h->d_minmax, height, width, wh,
+                                                                                  d_out + (int64_t)f0 * height * width);
         V5_CUDA(h, cudaGetLastError());
         h->launches += 3;
     }
@@ -647,33 +600,31 @@ int v5ela_spectrum_host(v5ela_handle *h, const uint8_t *gray_host, int n, int he
     if (!gray_host || !out_host || n < 0 || height <= 0 || width <= 0)
         return fail(h, V5ELA_ERR_INVALID, "v5ela_spectrum_host: bad pointer or size%s");
     DeviceGuard guard(h->device);
-    if (!h->own_stream) V5_CUDA(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
-    const size_t bytes = (size_t)n * height * width;
     int rc;
-    if ((rc = ensure(h, (void **)&h->d_gray, &h->d_gray_cap, bytes))) return rc;
-    if ((rc = ensure(h, (void **)&h->d_spec, &h->d_spec_cap, bytes))) return rc;
-    V5_CUDA(h, cudaMemcpyAsync(h->d_gray, gray_host, bytes, cudaMemcpyHostToDevice, h->own_stream));
-    rc = v5ela_spectrum(h, h->d_gray, n, height, width, (int64_t)height * width, width, h->d_spec, h->own_stream);
+    cudaStream_t st;
+    if ((rc = internal_stream(h, &st))) return rc;
+    const size_t bytes = (size_t)n * height * width;
+    if ((rc = h->d_gray.ensure(h, bytes))) return rc;
+    if ((rc = h->d_spec.ensure(h, bytes))) return rc;
+    V5_CUDA(h, cudaMemcpyAsync(h->d_gray, gray_host, bytes, cudaMemcpyHostToDevice, st));
+    rc = v5ela_spectrum(h, h->d_gray, n, height, width, (int64_t)height * width, width, h->d_spec, st);
     if (rc) return rc;
-    V5_CUDA(h, cudaMemcpyAsync(out_host, h->d_spec, bytes, cudaMemcpyDeviceToHost, h->own_stream));
-    V5_CUDA(h, cudaStreamSynchronize(h->own_stream));
+    V5_CUDA(h, cudaMemcpyAsync(out_host, h->d_spec, bytes, cudaMemcpyDeviceToHost, st));
+    V5_CUDA(h, cudaStreamSynchronize(st));
     return V5ELA_OK;
 }
 
 int v5ela_profile_enable(v5ela_handle *h, int enable)
-{
+try {
     if (!h) return V5ELA_ERR_INVALID;
     DeviceGuard guard(h->device);
     if (enable && h->prof_events.empty()) {
         h->prof_events.resize(8192);
-        for (auto &e : h->prof_events) {
-            e = nullptr;
-            V5_CUDA(h, cudaEventCreate(&e));
-        }
+        for (Event &e : h->prof_events) V5_CUDA(h, e.create(cudaEventDefault));
     }
     h->profiling = enable != 0;
     return V5ELA_OK;
-}
+} V5_CATCH(h)
 
 int v5ela_profile_read(v5ela_handle *h, double *fused_ms_sum, int64_t *fused_launches, int reset)
 {

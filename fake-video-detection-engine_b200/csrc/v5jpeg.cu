@@ -19,77 +19,42 @@ using namespace v5host;
 
 struct v5jpeg_state {
     // encoder
-    v5j::EncTables *d_enc_tabs = nullptr;
-    uint8_t *d_header = nullptr;
-    void *d_coef = nullptr, *d_bitoff = nullptr, *d_total = nullptr, *d_raw = nullptr;
-    size_t coef_cap = 0, bitoff_cap = 0, total_cap = 0, raw_cap = 0;
+    DeviceBuf<v5j::EncTables> d_enc_tabs;
+    DeviceBuf<uint8_t> d_header;
+    DeviceBuf<int16_t> d_coef;
+    DeviceBuf<uint32_t> d_bitoff, d_total, d_raw;
     // host-buffer entry points
-    uint8_t *d_img = nullptr, *d_out = nullptr;
-    int32_t *d_sizes = nullptr;
-    size_t img_cap = 0, out_cap = 0, sizes_cap = 0;
+    DeviceBuf<uint8_t> d_img, d_out;
+    DeviceBuf<int32_t> d_sizes;
     // decoder: one pinned staging buffer (descriptors | table sets | quantisation tables | scan segments) mirrored on the
     // device, plus the per-batch workspace (unstuffed streams, coefficients, sample planes)
     // Two of each, used alternately: the upload of one batch (on upload_stream) overlaps the kernels of the previous one.
-    uint8_t *stage_host[2] = {nullptr, nullptr}, *d_stage[2] = {nullptr, nullptr};
-    size_t stage_host_cap[2] = {0, 0}, stage_cap[2] = {0, 0};
-    cudaEvent_t uploaded[2] = {nullptr, nullptr};   // the upload into d_stage[b] (and out of stage_host[b]) has completed
-    cudaEvent_t consumed[2] = {nullptr, nullptr};   // the kernels that read d_stage[b] have completed
-    cudaStream_t upload_stream = nullptr;
+    PinnedBuf stage_host[2];
+    DeviceBuf<uint8_t> d_stage[2];
+    Event uploaded[2];                     // the upload into d_stage[b] (and out of stage_host[b]) has completed
+    Event consumed[2];                     // the kernels that read d_stage[b] have completed
+    Stream upload_stream;
     int toggle = 0;
-    void *d_streams = nullptr, *d_dcoef = nullptr, *d_planes = nullptr, *d_bits = nullptr, *d_status = nullptr, *d_dc = nullptr;
-    void *d_sub_info = nullptr, *d_sub_block0 = nullptr, *d_rst = nullptr;
-    size_t rst_cap = 0;
-    size_t streams_cap = 0, dcoef_cap = 0, planes_cap = 0, bits_cap = 0, status_cap = 0, dc_cap = 0, sub_info_cap = 0, sub_block0_cap = 0;
-    uint8_t *d_dec_rgb = nullptr, *d_dec_gray = nullptr;
-    int32_t *d_dec_status = nullptr;
-    size_t dec_rgb_cap = 0, dec_gray_cap = 0, dec_status_cap = 0;
+    DeviceBuf<uint8_t> d_streams, d_planes;
+    DeviceBuf<int16_t> d_dcoef, d_dc;
+    DeviceBuf<uint32_t> d_bits, d_sub_block0, d_rst;
+    DeviceBuf<int32_t> d_status;
+    DeviceBuf<v5j::SubInfo> d_sub_info;
+    DeviceBuf<uint8_t> d_dec_rgb, d_dec_gray;
+    DeviceBuf<int32_t> d_dec_status;
 };
 
-void v5jpeg_release(v5ela_handle *h)
-{
-    v5jpeg_state *s = h->jpeg;
-    if (!s) return;
-    cudaFree(s->d_enc_tabs);
-    cudaFree(s->d_header);
-    cudaFree(s->d_coef);
-    cudaFree(s->d_bitoff);
-    cudaFree(s->d_total);
-    cudaFree(s->d_raw);
-    cudaFree(s->d_img);
-    cudaFree(s->d_out);
-    cudaFree(s->d_sizes);
-    for (int b = 0; b < 2; b++) {
-        if (s->stage_host[b]) cudaFreeHost(s->stage_host[b]);
-        if (s->uploaded[b]) cudaEventDestroy(s->uploaded[b]);
-        if (s->consumed[b]) cudaEventDestroy(s->consumed[b]);
-        cudaFree(s->d_stage[b]);
-    }
-    if (s->upload_stream) cudaStreamDestroy(s->upload_stream);
-    cudaFree(s->d_streams);
-    cudaFree(s->d_dcoef);
-    cudaFree(s->d_planes);
-    cudaFree(s->d_bits);
-    cudaFree(s->d_status);
-    cudaFree(s->d_dc);
-    cudaFree(s->d_sub_info);
-    cudaFree(s->d_sub_block0);
-    cudaFree(s->d_rst);
-    cudaFree(s->d_dec_rgb);
-    cudaFree(s->d_dec_gray);
-    cudaFree(s->d_dec_status);
-    delete s;
-    h->jpeg = nullptr;
-}
+void v5host::JpegStateDelete::operator()(v5jpeg_state *s) const { delete s; }
 
 namespace {
 
 int jpeg_state(v5ela_handle *h, v5jpeg_state **out)
 {
     if (!h->jpeg) {
-        h->jpeg = new (std::nothrow) v5jpeg_state();
+        h->jpeg.reset(new (std::nothrow) v5jpeg_state());
         if (!h->jpeg) return fail(h, V5ELA_ERR_NOMEM, "v5ela_jpeg: out of host memory%s");
     }
-    *out = h->jpeg;
+    *out = h->jpeg.get();
     return 0;
 }
 
@@ -106,10 +71,9 @@ int64_t v5ela_jpeg_bound(int height, int width, int channels)
     return (int64_t)v5j::enc_geo(height, width, channels).blocks * 416 + kHeaderMax;
 }
 
-static int v5ela_jpeg_encode_impl(v5ela_handle *h, const uint8_t *d_img, int n, int height, int width, int channels,
-                      int64_t frame_stride_bytes, int64_t row_stride_bytes, int quality, uint8_t *d_out,
-                      int64_t out_stride_bytes, int32_t *d_sizes, void *cuda_stream)
-{
+int v5ela_jpeg_encode(v5ela_handle *h, const uint8_t *d_img, int n, int height, int width, int channels, int64_t frame_stride_bytes,
+                      int64_t row_stride_bytes, int quality, uint8_t *d_out, int64_t out_stride_bytes, int32_t *d_sizes, void *cuda_stream)
+try {
     if (!h) return V5ELA_ERR_INVALID;
     if (n == 0) return V5ELA_OK;
     if (!d_img || !d_out || !d_sizes || n < 0 || height <= 0 || width <= 0 || height > 65535 || width > 65535 ||
@@ -131,9 +95,9 @@ static int v5ela_jpeg_encode_impl(v5ela_handle *h, const uint8_t *d_img, int n, 
     if (!s->d_enc_tabs) {
         v5j::EncTables tabs;
         v5j::standard_enc_tables(tabs);
-        V5_CUDA(h, cudaMalloc(&s->d_enc_tabs, sizeof(tabs)));
+        if ((rc = s->d_enc_tabs.ensure(h, sizeof(tabs)))) return rc;
         V5_CUDA(h, cudaMemcpyAsync(s->d_enc_tabs, &tabs, sizeof(tabs), cudaMemcpyHostToDevice, st));
-        V5_CUDA(h, cudaMalloc(&s->d_header, kHeaderMax));
+        if ((rc = s->d_header.ensure(h, kHeaderMax))) return rc;
     }
     V5_CUDA(h, cudaMemcpyAsync(s->d_header, header.data(), header.size(), cudaMemcpyHostToDevice, st));
 
@@ -145,16 +109,16 @@ static int v5ela_jpeg_encode_impl(v5ela_handle *h, const uint8_t *d_img, int n, 
     if (chunk < 1) chunk = 1;
     if (chunk > n) chunk = n;
     if (chunk > 65535) chunk = 65535;
-    if ((rc = ensure(h, &s->d_coef, &s->coef_cap, (size_t)chunk * g.blocks * 128))) return rc;
-    if ((rc = ensure(h, &s->d_bitoff, &s->bitoff_cap, (size_t)chunk * g.blocks * 4))) return rc;
-    if ((rc = ensure(h, &s->d_total, &s->total_cap, (size_t)chunk * 4))) return rc;
-    if ((rc = ensure(h, &s->d_raw, &s->raw_cap, (size_t)chunk * raw_words * 4))) return rc;
+    if ((rc = s->d_coef.ensure(h, (size_t)chunk * g.blocks * 128))) return rc;
+    if ((rc = s->d_bitoff.ensure(h, (size_t)chunk * g.blocks * 4))) return rc;
+    if ((rc = s->d_total.ensure(h, (size_t)chunk * 4))) return rc;
+    if ((rc = s->d_raw.ensure(h, (size_t)chunk * raw_words * 4))) return rc;
 
     v5j::CoefParams cp;
     memset(&cp, 0, sizeof(cp));
     cp.frame_stride = frame_stride_bytes;
     cp.row_stride = row_stride_bytes;
-    cp.coef = static_cast<int16_t *>(s->d_coef);
+    cp.coef = s->d_coef;
     cp.g = g;
     v5j::make_enc_quant(ql, cp.q[0]);
     v5j::make_enc_quant(qc, cp.q[1]);
@@ -168,9 +132,9 @@ static int v5ela_jpeg_encode_impl(v5ela_handle *h, const uint8_t *d_img, int n, 
         V5_CUDA(h, cudaGetLastError());
         v5j::EntropyParams ep;
         ep.coef = cp.coef;
-        ep.bitoff = static_cast<uint32_t *>(s->d_bitoff);
-        ep.total_bits = static_cast<uint32_t *>(s->d_total);
-        ep.raw = static_cast<uint32_t *>(s->d_raw);
+        ep.bitoff = s->d_bitoff;
+        ep.total_bits = s->d_total;
+        ep.raw = s->d_raw;
         ep.raw_words = raw_words;
         ep.blocks = g.blocks;
         ep.bpm = g.bpm;
@@ -197,11 +161,11 @@ static int v5ela_jpeg_encode_impl(v5ela_handle *h, const uint8_t *d_img, int n, 
         h->launches += 5;
     }
     return V5ELA_OK;
-}
+} V5_CATCH(h)
 
-static int v5ela_jpeg_encode_host_impl(v5ela_handle *h, const uint8_t *img_host, int n, int height, int width, int channels, int quality,
+int v5ela_jpeg_encode_host(v5ela_handle *h, const uint8_t *img_host, int n, int height, int width, int channels, int quality,
                            uint8_t *out_host, int64_t out_stride_bytes, int32_t *sizes_host)
-{
+try {
     if (!h) return V5ELA_ERR_INVALID;
     if (n == 0) return V5ELA_OK;
     if (!img_host || !out_host || !sizes_host || n < 0 || height <= 0 || width <= 0 || (channels != 1 && channels != 3) ||
@@ -211,12 +175,12 @@ static int v5ela_jpeg_encode_host_impl(v5ela_handle *h, const uint8_t *img_host,
     v5jpeg_state *s;
     int rc;
     if ((rc = jpeg_state(h, &s))) return rc;
-    if (!h->own_stream) V5_CUDA(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
-    cudaStream_t st = h->own_stream;
+    cudaStream_t st;
+    if ((rc = internal_stream(h, &st))) return rc;
     const size_t fbytes = (size_t)height * width * channels;
-    if ((rc = ensure(h, (void **)&s->d_img, &s->img_cap, fbytes * n))) return rc;
-    if ((rc = ensure(h, (void **)&s->d_out, &s->out_cap, (size_t)out_stride_bytes * n))) return rc;
-    if ((rc = ensure(h, (void **)&s->d_sizes, &s->sizes_cap, sizeof(int32_t) * (size_t)n))) return rc;
+    if ((rc = s->d_img.ensure(h, fbytes * n))) return rc;
+    if ((rc = s->d_out.ensure(h, (size_t)out_stride_bytes * n))) return rc;
+    if ((rc = s->d_sizes.ensure(h, sizeof(int32_t) * (size_t)n))) return rc;
     V5_CUDA(h, cudaMemcpyAsync(s->d_img, img_host, fbytes * n, cudaMemcpyHostToDevice, st));
     rc = v5ela_jpeg_encode(h, s->d_img, n, height, width, channels, (int64_t)fbytes, (int64_t)width * channels, quality,
                            s->d_out, out_stride_bytes, s->d_sizes, st);
@@ -230,7 +194,7 @@ static int v5ela_jpeg_encode_host_impl(v5ela_handle *h, const uint8_t *img_host,
     }
     V5_CUDA(h, cudaStreamSynchronize(st));
     return V5ELA_OK;
-}
+} V5_CATCH(h)
 
 
 // ---------------------------------------------------------------------------------------------------------- decode
@@ -251,8 +215,8 @@ int v5ela_jpeg_info(const uint8_t *file_host, int64_t len, int *height, int *wid
 
 /* n files at once: dims_out[3 i .. 3 i + 2] = height, width, channels of file i. Stops at the first unreadable file and returns
  * its status; *bad_index (optional) names it. */
-static int v5ela_jpeg_info_batch_impl(const uint8_t *const *files_host, const int64_t *lens, int n, int32_t *dims_out, int *bad_index)
-{
+int v5ela_jpeg_info_batch(const uint8_t *const *files_host, const int64_t *lens, int n, int32_t *dims_out, int *bad_index)
+try {
     if (!files_host || !lens || n < 0 || !dims_out) return V5ELA_ERR_INVALID;
     for (int i = 0; i < n; i++) {
         int hh = 0, ww = 0, cc = 0;
@@ -266,7 +230,7 @@ static int v5ela_jpeg_info_batch_impl(const uint8_t *const *files_host, const in
         dims_out[3 * i + 2] = cc;
     }
     return V5ELA_OK;
-}
+} V5_CATCH(nullptr)
 
 }  // extern "C"
 
@@ -323,10 +287,9 @@ struct DecPlan {                               // host-side description of one c
 
 extern "C" {
 
-static int v5ela_jpeg_decode_impl(v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n, uint8_t *d_rgb,
-                      const int64_t *rgb_offsets, uint8_t *d_gray, const int64_t *gray_offsets, int32_t *d_status,
-                      void *cuda_stream)
-{
+int v5ela_jpeg_decode(v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n, uint8_t *d_rgb,
+                      const int64_t *rgb_offsets, uint8_t *d_gray, const int64_t *gray_offsets, int32_t *d_status, void *cuda_stream)
+try {
     if (!h) return V5ELA_ERR_INVALID;
     if (n == 0) return V5ELA_OK;
     if (!files_host || !lens || n < 0 || (!d_rgb && !d_gray))
@@ -338,10 +301,10 @@ static int v5ela_jpeg_decode_impl(v5ela_handle *h, const uint8_t *const *files_h
     int rc;
     if ((rc = jpeg_state(h, &s))) return rc;
     if (!s->upload_stream) {
-        V5_CUDA(h, cudaStreamCreateWithFlags(&s->upload_stream, cudaStreamNonBlocking));
+        V5_CUDA(h, s->upload_stream.create());
         for (int b = 0; b < 2; b++) {
-            V5_CUDA(h, cudaEventCreateWithFlags(&s->uploaded[b], cudaEventDisableTiming));
-            V5_CUDA(h, cudaEventCreateWithFlags(&s->consumed[b], cudaEventDisableTiming));
+            V5_CUDA(h, s->uploaded[b].create());
+            V5_CUDA(h, s->consumed[b].create());
         }
         V5_CUDA(h, cudaFuncSetAttribute(v5j::huffman_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(v5j::HuffSmem)));
         V5_CUDA(h, cudaFuncSetAttribute(v5j::huffman_sync_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(v5j::HuffSmem)));
@@ -471,23 +434,17 @@ static int v5ela_jpeg_decode_impl(v5ela_handle *h, const uint8_t *const *files_h
         cudaStream_t up = s->upload_stream;
         // host: the previous upload out of stage_host[b] is over; device: the kernels that read d_stage[b] are over
         V5_CUDA(h, cudaEventSynchronize(s->uploaded[b]));
-        if (s->stage_host_cap[b] < host_stage_bytes) {
-            if (s->stage_host[b]) cudaFreeHost(s->stage_host[b]);
-            s->stage_host[b] = nullptr;
-            s->stage_host_cap[b] = 0;
-            V5_CUDA(h, cudaHostAlloc((void **)&s->stage_host[b], host_stage_bytes + host_stage_bytes / 4, cudaHostAllocDefault));
-            s->stage_host_cap[b] = host_stage_bytes + host_stage_bytes / 4;
-        }
-        if ((rc = ensure(h, (void **)&s->d_stage[b], &s->stage_cap[b], stage_bytes))) return rc;
-        if ((rc = ensure(h, &s->d_streams, &s->streams_cap, P.stream_bytes))) return rc;
-        if ((rc = ensure(h, &s->d_dcoef, &s->dcoef_cap, P.coef_blocks * 128))) return rc;
-        if ((rc = ensure(h, &s->d_planes, &s->planes_cap, P.plane_bytes))) return rc;
-        if ((rc = ensure(h, &s->d_bits, &s->bits_cap, sizeof(uint32_t) * (size_t)cn))) return rc;
-        if ((rc = ensure(h, &s->d_status, &s->status_cap, sizeof(int32_t) * (size_t)cn))) return rc;
-        if ((rc = ensure(h, &s->d_dc, &s->dc_cap, sizeof(int16_t) * P.coef_blocks))) return rc;
-        if ((rc = ensure(h, &s->d_sub_info, &s->sub_info_cap, sizeof(v5j::SubInfo) * P.subs))) return rc;
-        if ((rc = ensure(h, &s->d_sub_block0, &s->sub_block0_cap, sizeof(uint32_t) * P.subs))) return rc;
-        if ((rc = ensure(h, &s->d_rst, &s->rst_cap, sizeof(uint32_t) * (P.rst_entries + 1)))) return rc;
+        if ((rc = s->stage_host[b].ensure(h, host_stage_bytes, host_stage_bytes + host_stage_bytes / 4))) return rc;
+        if ((rc = s->d_stage[b].ensure(h, stage_bytes))) return rc;
+        if ((rc = s->d_streams.ensure(h, P.stream_bytes))) return rc;
+        if ((rc = s->d_dcoef.ensure(h, P.coef_blocks * 128))) return rc;
+        if ((rc = s->d_planes.ensure(h, P.plane_bytes))) return rc;
+        if ((rc = s->d_bits.ensure(h, sizeof(uint32_t) * (size_t)cn))) return rc;
+        if ((rc = s->d_status.ensure(h, sizeof(int32_t) * (size_t)cn))) return rc;
+        if ((rc = s->d_dc.ensure(h, sizeof(int16_t) * P.coef_blocks))) return rc;
+        if ((rc = s->d_sub_info.ensure(h, sizeof(v5j::SubInfo) * P.subs))) return rc;
+        if ((rc = s->d_sub_block0.ensure(h, sizeof(uint32_t) * P.subs))) return rc;
+        if ((rc = s->d_rst.ensure(h, sizeof(uint32_t) * (P.rst_entries + 1)))) return rc;
         uint8_t *stage_host = s->stage_host[b], *d_stage = s->d_stage[b];
         for (int k = 0; k < cn; k++) P.images[(size_t)k].scan_off += (int64_t)off_scan;
         if (!all_pinned)
@@ -526,9 +483,9 @@ static int v5ela_jpeg_decode_impl(v5ela_handle *h, const uint8_t *const *files_h
         const v5j::DecImage *d_images = reinterpret_cast<const v5j::DecImage *>(d_stage + off_img);
         const v5j::DecTabSet *d_tabs = reinterpret_cast<const v5j::DecTabSet *>(d_stage + off_tab);
         const uint16_t *d_q = reinterpret_cast<const uint16_t *>(d_stage + off_q);
-        uint32_t *d_bits = static_cast<uint32_t *>(s->d_bits);
-        int32_t *d_st = static_cast<int32_t *>(s->d_status);
-        v5j::unstuff_kernel<<<cn, 1024, 0, st>>>(d_images, d_stage, static_cast<uint8_t *>(s->d_streams), d_bits, static_cast<uint32_t *>(s->d_rst));
+        uint32_t *d_bits = s->d_bits;
+        int32_t *d_st = s->d_status;
+        v5j::unstuff_kernel<<<cn, 1024, 0, st>>>(d_images, d_stage, s->d_streams, d_bits, s->d_rst);
         V5_CUDA(h, cudaGetLastError());
         // Huffman decoding in three launches: synchronisation (the windows of a file shared out among `parts` CTAs so that a
         // small batch still fills the GPU), boundary fix-up + block offsets, then one CTA per window writes coefficients.
@@ -536,9 +493,9 @@ static int v5ela_jpeg_decode_impl(v5ela_handle *h, const uint8_t *const *files_h
         unsigned parts = (unsigned)(h->sm_count / cn);
         parts = parts < 1 ? 1 : (parts > 16 ? 16 : parts);
         parts = parts > P.max_windows ? P.max_windows : parts;
-        const uint8_t *d_str = static_cast<const uint8_t *>(s->d_streams);
-        v5j::SubInfo *d_sub_info = static_cast<v5j::SubInfo *>(s->d_sub_info);
-        uint32_t *d_sub_block0 = static_cast<uint32_t *>(s->d_sub_block0);
+        const uint8_t *d_str = s->d_streams;
+        v5j::SubInfo *d_sub_info = s->d_sub_info;
+        uint32_t *d_sub_block0 = s->d_sub_block0;
         const char *force = getenv("V5ELA_HUFF_PATH");                    // tests: "one" / "three" force a path
         if (const char *fp = getenv("V5ELA_HUFF_PARTS")) {                 // experiments: parts per file of the three-launch path
             const int v = atoi(fp);
@@ -547,8 +504,7 @@ static int v5ela_jpeg_decode_impl(v5ela_handle *h, const uint8_t *const *files_h
         // nothing to gain from splitting when there is no room for two parts per file, or no file has more than one window
         const bool one_launch = force ? force[0] == 'o' : (h->sm_count / cn < 2 || P.max_windows < 2);
         if (one_launch) {
-            v5j::huffman_kernel<<<cn, v5j::HUFF_NT, sizeof(v5j::HuffSmem), st>>>(d_images, d_tabs, d_str, d_bits, static_cast<int16_t *>(s->d_dcoef),
-                                                                            static_cast<int16_t *>(s->d_dc), d_st);
+            v5j::huffman_kernel<<<cn, v5j::HUFF_NT, sizeof(v5j::HuffSmem), st>>>(d_images, d_tabs, d_str, d_bits, s->d_dcoef, s->d_dc, d_st);
             V5_CUDA(h, cudaGetLastError());
         } else {
             v5j::huffman_sync_kernel<<<dim3(parts, (unsigned)cn), v5j::HUFF_NT, sizeof(v5j::HuffSmem), st>>>(d_images, d_tabs, d_str, d_bits, d_sub_info);
@@ -556,23 +512,22 @@ static int v5ela_jpeg_decode_impl(v5ela_handle *h, const uint8_t *const *files_h
             v5j::huffman_fixup_kernel<<<cn, 1024, 0, st>>>(d_images, d_tabs, d_str, d_bits, parts, d_sub_info, d_sub_block0, d_st);
             V5_CUDA(h, cudaGetLastError());
             v5j::huffman_write_kernel<<<dim3(P.max_windows, (unsigned)cn), v5j::HUFF_NT, sizeof(v5j::HuffSmem), st>>>(
-                d_images, d_tabs, d_str, d_bits, d_sub_info, d_sub_block0, static_cast<int16_t *>(s->d_dcoef), static_cast<int16_t *>(s->d_dc));
+                d_images, d_tabs, d_str, d_bits, d_sub_info, d_sub_block0, s->d_dcoef, s->d_dc);
             V5_CUDA(h, cudaGetLastError());
         }
         if (P.max_intervals > 0) {                                         // files with restart intervals: one thread per interval
             v5j::huffman_rst_kernel<<<dim3((unsigned)((P.max_intervals + 127) / 128), (unsigned)cn), 128, 0, st>>>(
-                d_images, d_tabs, d_str, d_bits, static_cast<const uint32_t *>(s->d_rst), static_cast<int16_t *>(s->d_dcoef),
-                static_cast<int16_t *>(s->d_dc), d_st);
+                d_images, d_tabs, d_str, d_bits, s->d_rst, s->d_dcoef, s->d_dc, d_st);
             V5_CUDA(h, cudaGetLastError());
             h->launches += 1;
         }
-        v5j::dc_kernel<<<cn, 1024, 0, st>>>(d_images, static_cast<int16_t *>(s->d_dc));
+        v5j::dc_kernel<<<cn, 1024, 0, st>>>(d_images, s->d_dc);
         V5_CUDA(h, cudaGetLastError());
         v5j::idct_kernel<<<dim3((unsigned)((P.max_blocks + 63) / 64), (unsigned)cn), 256, 0, st>>>(
-            d_images, d_q, static_cast<const int16_t *>(s->d_dcoef), static_cast<const int16_t *>(s->d_dc), static_cast<uint8_t *>(s->d_planes));
+            d_images, d_q, s->d_dcoef, s->d_dc, s->d_planes);
         V5_CUDA(h, cudaGetLastError());
         v5j::colour_kernel<<<dim3((unsigned)((P.max_groups + 255) / 256), (unsigned)cn), 256, 0, st>>>(
-            d_images, static_cast<const uint8_t *>(s->d_planes), d_rgb, d_gray);
+            d_images, s->d_planes, d_rgb, d_gray);
         V5_CUDA(h, cudaGetLastError());
         if (d_status)                                                      // chunks keep file order: one contiguous range
             V5_CUDA(h, cudaMemcpyAsync(d_status + P.file_index[0], d_st, sizeof(int32_t) * (size_t)cn, cudaMemcpyDeviceToDevice, st));
@@ -580,11 +535,11 @@ static int v5ela_jpeg_decode_impl(v5ela_handle *h, const uint8_t *const *files_h
         h->launches += one_launch ? 5 : 7;
     }
     return V5ELA_OK;
-}
+} V5_CATCH(h)
 
-static int v5ela_jpeg_decode_host_impl(v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n, uint8_t *rgb_host,
+int v5ela_jpeg_decode_host(v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n, uint8_t *rgb_host,
                            const int64_t *rgb_offsets, uint8_t *gray_host, const int64_t *gray_offsets)
-{
+try {
     if (!h) return V5ELA_ERR_INVALID;
     if (n == 0) return V5ELA_OK;
     if (!files_host || !lens || n < 0 || (!rgb_host && !gray_host))
@@ -593,8 +548,8 @@ static int v5ela_jpeg_decode_host_impl(v5ela_handle *h, const uint8_t *const *fi
     v5jpeg_state *s;
     int rc;
     if ((rc = jpeg_state(h, &s))) return rc;
-    if (!h->own_stream) V5_CUDA(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
-    cudaStream_t st = h->own_stream;
+    cudaStream_t st;
+    if ((rc = internal_stream(h, &st))) return rc;
     // output extents: the caller's offsets, or tight packing in file order
     std::vector<int64_t> px((size_t)n);
     int64_t rgb_end = 0, gray_end = 0, run = 0;
@@ -609,13 +564,13 @@ static int v5ela_jpeg_decode_host_impl(v5ela_handle *h, const uint8_t *const *fi
         if (go + px[(size_t)i] > gray_end) gray_end = go + px[(size_t)i];
         run += px[(size_t)i];
     }
-    if (rgb_host && (rc = ensure(h, (void **)&s->d_dec_rgb, &s->dec_rgb_cap, (size_t)rgb_end))) return rc;
-    if (gray_host && (rc = ensure(h, (void **)&s->d_dec_gray, &s->dec_gray_cap, (size_t)gray_end))) return rc;
+    if (rgb_host && (rc = s->d_dec_rgb.ensure(h, (size_t)rgb_end))) return rc;
+    if (gray_host && (rc = s->d_dec_gray.ensure(h, (size_t)gray_end))) return rc;
     std::vector<int32_t> status((size_t)n, 0);
-    if ((rc = ensure(h, (void **)&s->d_dec_status, &s->dec_status_cap, sizeof(int32_t) * (size_t)n))) return rc;
+    if ((rc = s->d_dec_status.ensure(h, sizeof(int32_t) * (size_t)n))) return rc;
     int32_t *d_status = s->d_dec_status;
-    rc = v5ela_jpeg_decode(h, files_host, lens, n, rgb_host ? s->d_dec_rgb : nullptr, rgb_offsets, gray_host ? s->d_dec_gray : nullptr,
-                           gray_offsets, d_status, st);
+    rc = v5ela_jpeg_decode(h, files_host, lens, n, rgb_host ? static_cast<uint8_t *>(s->d_dec_rgb) : nullptr, rgb_offsets,
+                           gray_host ? static_cast<uint8_t *>(s->d_dec_gray) : nullptr, gray_offsets, d_status, st);
     if (rc == V5ELA_OK) {
         cudaMemcpyAsync(status.data(), d_status, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st);
         run = 0;
@@ -636,49 +591,6 @@ static int v5ela_jpeg_decode_host_impl(v5ela_handle *h, const uint8_t *const *fi
             return fail(h, V5ELA_ERR_INVALID, "v5ela_jpeg_decode_host: entropy-coded data ends early or is corrupt%s", which);
         }
     return V5ELA_OK;
-}
-
-
-// ---- the exported entry points: nothing may unwind through the C ABI (std::vector / std::thread inside the implementations can throw)
-#define V5J_GUARD(h, call)                                                                       \
-    try {                                                                                        \
-        return call;                                                                             \
-    } catch (const std::bad_alloc &) {                                                           \
-        return fail((h), V5ELA_ERR_NOMEM, "out of host memory%s");                               \
-    } catch (const std::exception &e) {                                                          \
-        return fail((h), V5ELA_ERR_INVALID, "host-side failure: %s", e.what());                  \
-    } catch (...) {                                                                              \
-        return fail((h), V5ELA_ERR_INVALID, "host-side failure%s");                              \
-    }
-
-int v5ela_jpeg_encode(v5ela_handle *h, const uint8_t *d_img, int n, int height, int width, int channels, int64_t frame_stride_bytes,
-                      int64_t row_stride_bytes, int quality, uint8_t *d_out, int64_t out_stride_bytes, int32_t *d_sizes, void *cuda_stream)
-{
-    V5J_GUARD(h, v5ela_jpeg_encode_impl(h, d_img, n, height, width, channels, frame_stride_bytes, row_stride_bytes, quality, d_out,
-                                        out_stride_bytes, d_sizes, cuda_stream))
-}
-
-int v5ela_jpeg_encode_host(v5ela_handle *h, const uint8_t *img_host, int n, int height, int width, int channels, int quality,
-                           uint8_t *out_host, int64_t out_stride_bytes, int32_t *sizes_host)
-{
-    V5J_GUARD(h, v5ela_jpeg_encode_host_impl(h, img_host, n, height, width, channels, quality, out_host, out_stride_bytes, sizes_host))
-}
-
-int v5ela_jpeg_info_batch(const uint8_t *const *files_host, const int64_t *lens, int n, int32_t *dims_out, int *bad_index)
-{
-    V5J_GUARD(static_cast<v5ela_handle *>(nullptr), v5ela_jpeg_info_batch_impl(files_host, lens, n, dims_out, bad_index))
-}
-
-int v5ela_jpeg_decode(v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n, uint8_t *d_rgb,
-                      const int64_t *rgb_offsets, uint8_t *d_gray, const int64_t *gray_offsets, int32_t *d_status, void *cuda_stream)
-{
-    V5J_GUARD(h, v5ela_jpeg_decode_impl(h, files_host, lens, n, d_rgb, rgb_offsets, d_gray, gray_offsets, d_status, cuda_stream))
-}
-
-int v5ela_jpeg_decode_host(v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n, uint8_t *rgb_host,
-                           const int64_t *rgb_offsets, uint8_t *gray_host, const int64_t *gray_offsets)
-{
-    V5J_GUARD(h, v5ela_jpeg_decode_host_impl(h, files_host, lens, n, rgb_host, rgb_offsets, gray_host, gray_offsets))
-}
+} V5_CATCH(h)
 
 }  // extern "C"
