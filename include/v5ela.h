@@ -214,7 +214,8 @@ V5ELA_API int v5ela_jpeg_encode_host(v5ela_handle *h, const uint8_t *img_host, i
  *             to the device asynchronously from where they are — keep them alive until the stream has been synchronised;
  *             pageable files are staged through a pinned buffer inside the handle before the call returns.
  *   d_rgb   : optional DEVICE buffer; file i is decoded to RGB (HWC; a one-component file is replicated) at byte offset
- *             rgb_offsets[i], or tightly packed in file order when rgb_offsets is NULL.
+ *             rgb_offsets[i], or tightly packed in file order when rgb_offsets is NULL. A negative offset is refused with
+ *             V5ELA_ERR_INVALID (v5ela_last_error names the file) before anything is launched.
  *   d_gray  : optional DEVICE buffer; the luma plane alone (what IMREAD_GRAYSCALE returns), offsets likewise.
  *   d_status: optional DEVICE array of n ints: 0, or -1 when the entropy-coded data of that file ended early (or a restart
  *             marker is missing).

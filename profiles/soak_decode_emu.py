@@ -4,7 +4,7 @@ import io, sys, ctypes, numpy as np, cv2
 import os; ROOT=os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path.insert(0,ROOT); sys.path.insert(0,os.path.join(ROOT,'tests'))
 from PIL import Image
 import test_jpeg_emu as T
-libs=[T._build("full",[]), T._build("tiny",["-DV5J_HUFF_NT=8","-DV5J_SUB_BITS=64"])]
+libs=[T.Emu(T._build("full",[]),0), T.Emu(T._build("tiny",T.TINY),0)]
 rng=np.random.default_rng(123)
 bad=0; n=0
 for it in range(700):

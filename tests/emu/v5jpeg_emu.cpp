@@ -12,6 +12,7 @@
 #include "v5ela_host.h"
 #include "v5jpeg_enc.cuh"
 #include "v5jpeg_dec.cuh"
+#include "v5jpeg_plan.h"
 
 using namespace v5j;
 
@@ -124,7 +125,10 @@ static int emu_finish(const DecImage &im, const FileInfo &F, std::vector<int16_t
     return 0;
 }
 
-extern "C" int v5jemu_decode(const uint8_t *data, int64_t len, uint8_t *rgb_out, uint8_t *gray_out, int16_t *coef_out, int *rounds_out)
+// parts: 0 = huffman_kernel (one CTA per file), otherwise the three-launch flow with the file's windows shared out among up to
+// `parts` CTAs (the plan's DecChunk::one_launch / parts)
+extern "C" int v5jemu_decode(const uint8_t *data, int64_t len, uint8_t *rgb_out, uint8_t *gray_out, int16_t *coef_out, int *rounds_out,
+                             int parts_wanted)
 {
     FileInfo *F = new FileInfo();
     const int rc = parse_file(data, (size_t)len, *F);
@@ -166,9 +170,6 @@ extern "C" int v5jemu_decode(const uint8_t *data, int64_t len, uint8_t *rgb_out,
     BlockHead *heads = new BlockHead();                                     // (all zero: what the kernels establish before the write pass)
     memset(heads, 0, sizeof(*heads));
     J.heads = heads;
-#ifndef V5J_EMU_PARTS
-#define V5J_EMU_PARTS 0
-#endif
     if (F->restart > 0) {
         // ---- huffman_rst_kernel: one thread per restart interval, DC values written directly
         const int mcus = im.mcux * im.mcuy, n_int = (mcus + F->restart - 1) / F->restart;
@@ -188,50 +189,15 @@ extern "C" int v5jemu_decode(const uint8_t *data, int64_t len, uint8_t *rgb_out,
         delete T; delete F; delete heads;
         return rc2 ? rc2 : (ok ? 0 : -3);
     }
-#if V5J_EMU_PARTS == 0
-    // ---- huffman_kernel: one CTA per file, windows in order, coefficients written window by window
-    HuffWindow *W = new HuffWindow();
-    memset(W, 0xA5, sizeof(*W));
-    W->carry.p = 0; W->carry.c = 0; W->carry.z = 0;
-    W->base_blocks = 0;
-    int max_rounds = 0;
-    for (uint32_t w0 = 0; w0 < J.nsub; w0 += HUFF_NT) {
-        J.staged.base_word = w0 * (uint32_t)SUB_WORDS;
-        for (int t = 0; t < HUFF_NT; t++) stage_window(t, HUFF_NT, staged.data(), J.stream, J.staged.base_word, J.stream_words);
-        for (int t = 0; t < HUFF_NT; t++) huff_phase_first(t, *W, J, *T, w0);
-        for (int r = 1; r < HUFF_NT; r++) {
-            for (int t = 0; t < HUFF_NT; t++) huff_phase_round(t, r, *W, J, *T, w0);
-            bool all = true;
-            for (int t = 0; t < HUFF_NT; t++) all = all && W->done[t];
-            if (r > max_rounds) max_rounds = r;
-            if (all) break;
-        }
-        uint32_t run = W->base_blocks;
-        std::vector<uint32_t> b0(HUFF_NT);
-        for (int t = 0; t < HUFF_NT; t++) {
-            b0[t] = run;
-            if (w0 + (uint32_t)t < J.nsub) run += W->info[t].n;
-        }
-        for (int t = HUFF_NT - 1; t >= 0; t--) huff_phase_write(t, *W, J, *T, w0, b0[t]);
-        const uint32_t last = J.nsub - w0 < (uint32_t)HUFF_NT ? J.nsub - w0 - 1 : HUFF_NT - 1;
-        W->carry = W->info[last].s;
-        W->base_blocks = run;
-    }
-    const bool ok = W->base_blocks >= (uint32_t)im.blocks;
-#else
-    // ---- huffman_sync_kernel / huffman_fixup_kernel / huffman_write_kernel
     HuffWindow *W = new HuffWindow();
     int max_rounds = 0;
-    // pass 1 (huffman_sync_kernel): the file's windows shared out among `parts` CTAs; part 0 starts true, the others blind
-    std::vector<SubInfo> sub_info(J.nsub + 1);
-    std::vector<uint32_t> sub_block0(J.nsub + 1, 0xA5A5A5A5u);
-    const uint32_t windows = window_count(J.nsub), parts = part_count(J.nsub, V5J_EMU_PARTS);
-    for (uint32_t q = parts; q-- > 0;) {                                    // any order: the parts are independent CTAs
+    bool ok;
+    if (parts_wanted == 0) {
+        // ---- huffman_kernel: one CTA per file, windows in order, coefficients written window by window
         memset(W, 0xA5, sizeof(*W));
-        const uint32_t w_first = part_first(q, parts, windows), w_end = part_first(q + 1, parts, windows);
-        W->carry.p = w_first * (uint32_t)HUFF_NT * SUB_BITS; W->carry.c = 0; W->carry.z = 0;
-        for (uint32_t w = w_first; w < w_end; w++) {
-            const uint32_t w0 = w * (uint32_t)HUFF_NT;
+        W->carry.p = 0; W->carry.c = 0; W->carry.z = 0;
+        W->base_blocks = 0;
+        for (uint32_t w0 = 0; w0 < J.nsub; w0 += HUFF_NT) {
             J.staged.base_word = w0 * (uint32_t)SUB_WORDS;
             for (int t = 0; t < HUFF_NT; t++) stage_window(t, HUFF_NT, staged.data(), J.stream, J.staged.base_word, J.stream_words);
             for (int t = 0; t < HUFF_NT; t++) huff_phase_first(t, *W, J, *T, w0);
@@ -242,47 +208,81 @@ extern "C" int v5jemu_decode(const uint8_t *data, int64_t len, uint8_t *rgb_out,
                 if (r > max_rounds) max_rounds = r;
                 if (all) break;
             }
-            for (int t = 0; t < HUFF_NT; t++)
-                if (w0 + (uint32_t)t < J.nsub) sub_info[w0 + t] = W->info[t];
+            uint32_t run = W->base_blocks;
+            std::vector<uint32_t> b0(HUFF_NT);
+            for (int t = 0; t < HUFF_NT; t++) {
+                b0[t] = run;
+                if (w0 + (uint32_t)t < J.nsub) run += W->info[t].n;
+            }
+            for (int t = HUFF_NT - 1; t >= 0; t--) huff_phase_write(t, *W, J, *T, w0, b0[t]);
             const uint32_t last = J.nsub - w0 < (uint32_t)HUFF_NT ? J.nsub - w0 - 1 : HUFF_NT - 1;
             W->carry = W->info[last].s;
+            W->base_blocks = run;
         }
+        ok = W->base_blocks >= (uint32_t)im.blocks;
+    } else {
+        // ---- huffman_sync_kernel / huffman_fixup_kernel / huffman_write_kernel
+        // pass 1 (huffman_sync_kernel): the file's windows shared out among `parts` CTAs; part 0 starts true, the others blind
+        std::vector<SubInfo> sub_info(J.nsub + 1);
+        std::vector<uint32_t> sub_block0(J.nsub + 1, 0xA5A5A5A5u);
+        const uint32_t windows = window_count(J.nsub), parts = part_count(J.nsub, (uint32_t)parts_wanted);
+        for (uint32_t q = parts; q-- > 0;) {                                    // any order: the parts are independent CTAs
+            memset(W, 0xA5, sizeof(*W));
+            const uint32_t w_first = part_first(q, parts, windows), w_end = part_first(q + 1, parts, windows);
+            W->carry.p = w_first * (uint32_t)HUFF_NT * SUB_BITS; W->carry.c = 0; W->carry.z = 0;
+            for (uint32_t w = w_first; w < w_end; w++) {
+                const uint32_t w0 = w * (uint32_t)HUFF_NT;
+                J.staged.base_word = w0 * (uint32_t)SUB_WORDS;
+                for (int t = 0; t < HUFF_NT; t++) stage_window(t, HUFF_NT, staged.data(), J.stream, J.staged.base_word, J.stream_words);
+                for (int t = 0; t < HUFF_NT; t++) huff_phase_first(t, *W, J, *T, w0);
+                for (int r = 1; r < HUFF_NT; r++) {
+                    for (int t = 0; t < HUFF_NT; t++) huff_phase_round(t, r, *W, J, *T, w0);
+                    bool all = true;
+                    for (int t = 0; t < HUFF_NT; t++) all = all && W->done[t];
+                    if (r > max_rounds) max_rounds = r;
+                    if (all) break;
+                }
+                for (int t = 0; t < HUFF_NT; t++)
+                    if (w0 + (uint32_t)t < J.nsub) sub_info[w0 + t] = W->info[t];
+                const uint32_t last = J.nsub - w0 < (uint32_t)HUFF_NT ? J.nsub - w0 - 1 : HUFF_NT - 1;
+                W->carry = W->info[last].s;
+            }
+        }
+        // pass 2 (huffman_fixup_kernel): all boundary walks from the recorded states, then the in-order check, then the scan
+        std::vector<SubState> started_from(parts + 1);
+        auto bounds = [&](uint32_t q, uint32_t &j0, uint32_t &j_end) {
+            j0 = part_first(q, parts, windows) * (uint32_t)HUFF_NT;
+            j_end = part_first(q + 1, parts, windows) * (uint32_t)HUFF_NT;
+            j_end = j_end < J.nsub ? j_end : J.nsub;
+        };
+        for (uint32_t q = 1; q < parts; q++) started_from[q] = sub_info[part_first(q, parts, windows) * (uint32_t)HUFF_NT - 1].s;
+        for (uint32_t q = parts; q-- > 1;) {                                    // "concurrent": each from the state it saw at the start
+            uint32_t j0, j_end;
+            bounds(q, j0, j_end);
+            SubInfo saved = sub_info[j0 - 1];
+            sub_info[j0 - 1].s = started_from[q];
+            fixup_walk(J.stream, J.total_bits, *T, J.bpm, sub_info.data(), j0, j_end);
+            sub_info[j0 - 1] = saved;
+        }
+        for (uint32_t q = 1; q < parts; q++) {
+            uint32_t j0, j_end;
+            bounds(q, j0, j_end);
+            if (!same_state(started_from[q], sub_info[j0 - 1].s)) fixup_walk(J.stream, J.total_bits, *T, J.bpm, sub_info.data(), j0, j_end);
+        }
+        uint32_t total_blocks = 0;
+        for (uint32_t j = 0; j < J.nsub; j++) {
+            sub_block0[j] = total_blocks;
+            total_blocks += sub_info[j].n;
+        }
+        // pass 3 (huffman_write_kernel): one CTA per window
+        for (uint32_t w = windows; w-- > 0;) {
+            const uint32_t w0 = w * (uint32_t)HUFF_NT;
+            J.staged.base_word = w0 * (uint32_t)SUB_WORDS;
+            for (int t = 0; t < HUFF_NT; t++) stage_window(t, HUFF_NT, staged.data(), J.stream, J.staged.base_word, J.stream_words);
+            for (int t = HUFF_NT - 1; t >= 0; t--) huff_write_sub(t, J, *T, w0, sub_info.data(), sub_block0.data());
+        }
+        ok = total_blocks >= (uint32_t)im.blocks;
     }
-    // pass 2 (huffman_fixup_kernel): all boundary walks from the recorded states, then the in-order check, then the scan
-    std::vector<SubState> started_from(parts + 1);
-    auto bounds = [&](uint32_t q, uint32_t &j0, uint32_t &j_end) {
-        j0 = part_first(q, parts, windows) * (uint32_t)HUFF_NT;
-        j_end = part_first(q + 1, parts, windows) * (uint32_t)HUFF_NT;
-        j_end = j_end < J.nsub ? j_end : J.nsub;
-    };
-    for (uint32_t q = 1; q < parts; q++) started_from[q] = sub_info[part_first(q, parts, windows) * (uint32_t)HUFF_NT - 1].s;
-    for (uint32_t q = parts; q-- > 1;) {                                    // "concurrent": each from the state it saw at the start
-        uint32_t j0, j_end;
-        bounds(q, j0, j_end);
-        SubInfo saved = sub_info[j0 - 1];
-        sub_info[j0 - 1].s = started_from[q];
-        fixup_walk(J.stream, J.total_bits, *T, J.bpm, sub_info.data(), j0, j_end);
-        sub_info[j0 - 1] = saved;
-    }
-    for (uint32_t q = 1; q < parts; q++) {
-        uint32_t j0, j_end;
-        bounds(q, j0, j_end);
-        if (!same_state(started_from[q], sub_info[j0 - 1].s)) fixup_walk(J.stream, J.total_bits, *T, J.bpm, sub_info.data(), j0, j_end);
-    }
-    uint32_t total_blocks = 0;
-    for (uint32_t j = 0; j < J.nsub; j++) {
-        sub_block0[j] = total_blocks;
-        total_blocks += sub_info[j].n;
-    }
-    // pass 3 (huffman_write_kernel): one CTA per window
-    for (uint32_t w = windows; w-- > 0;) {
-        const uint32_t w0 = w * (uint32_t)HUFF_NT;
-        J.staged.base_word = w0 * (uint32_t)SUB_WORDS;
-        for (int t = 0; t < HUFF_NT; t++) stage_window(t, HUFF_NT, staged.data(), J.stream, J.staged.base_word, J.stream_words);
-        for (int t = HUFF_NT - 1; t >= 0; t--) huff_write_sub(t, J, *T, w0, sub_info.data(), sub_block0.data());
-    }
-    const bool ok = total_blocks >= (uint32_t)im.blocks;
-#endif
     if (rounds_out) *rounds_out = max_rounds;
     const int rc2 = emu_finish(im, *F, coef, dcv, true, rgb_out, gray_out, coef_out);
     bool heads_clean = true;                                                // every write pass must leave the block heads zeroed
@@ -310,4 +310,80 @@ extern "C" int v5jemu_huff_actions(const uint8_t *bits, const uint8_t *vals, int
     const int lb = (int)t->long_base;
     delete t;
     return lb;
+}
+
+// The decoder's plan of a call (v5j::plan_decode) as the library makes it, summarised for the tests. Returns the plan's status;
+// *n_chunks, *bad_file. Per chunk k (up to max_chunks), chunk_rows[PLAN_ROW * k ..]:
+//   files, first file, off_tab, off_q, off_scan, stage_bytes, host_stage_bytes, upload runs, scan_bytes, stream_bytes, coef_blocks,
+//   plane_bytes, subs, rst_entries, max_windows, max_intervals, max_blocks, max_groups, one_launch, parts, launches,
+//   hash of the DecImage table, hash of the upload runs (host addresses relative to files[0])
+// Per file i, file_rows[FILE_ROW * i ..]: chunk, position in the chunk, tabset, qt, rgb_off, gray_off, scan_off, rst_off.
+// Per upload run (up to max_runs; *n_runs counts them all), run_rows[4 * r ..]: chunk, device offset, host address - files[0], bytes.
+constexpr int PLAN_ROW = 23, FILE_ROW = 8;
+
+static uint64_t fnv(uint64_t hsh, int64_t v)
+{
+    for (int b = 0; b < 8; b++) hsh = (hsh ^ (uint8_t)((uint64_t)v >> (8 * b))) * 0x100000001b3ull;
+    return hsh;
+}
+
+extern "C" int v5jemu_plan_decode(const uint8_t *const *files, const int64_t *lens, int n, const int64_t *rgb_offsets,
+                                  const int64_t *gray_offsets, int want_rgb, int want_gray, int all_pinned, int sm_count, int huff_path,
+                                  int huff_parts, int64_t chunk_bytes, int64_t *chunk_rows, int max_chunks, int64_t *file_rows,
+                                  int64_t *run_rows, int max_runs, int *n_chunks, int *n_runs, int *bad_file)
+{
+    v5j::DecodeCall c;
+    c.files = files;
+    c.lens = lens;
+    c.n = n;
+    c.rgb_offsets = rgb_offsets;
+    c.gray_offsets = gray_offsets;
+    c.want_rgb = want_rgb != 0;
+    c.want_gray = want_gray != 0;
+    c.all_pinned = all_pinned != 0;
+    c.sm_count = sm_count;
+    c.huff_path = huff_path;
+    c.huff_parts = huff_parts;
+    c.threads = 4;
+    c.chunk_bytes = (size_t)chunk_bytes;
+    v5j::DecodePlan *P = new v5j::DecodePlan();
+    v5j::plan_decode(c, *P);
+    *bad_file = P->bad_file;
+    *n_chunks = (int)P->chunks.size();
+    *n_runs = 0;
+    const intptr_t base = n > 0 ? reinterpret_cast<intptr_t>(files[0]) : 0;
+    for (size_t k = 0; P->status == V5ELA_OK && k < P->chunks.size(); k++) {
+        const v5j::DecChunk &C = P->chunks[k];
+        uint64_t h_img = 0xcbf29ce484222325ull, h_run = 0xcbf29ce484222325ull;
+        for (size_t j = 0; j < C.images.size(); j++) {
+            const DecImage &im = C.images[j];
+            for (int64_t v : {(int64_t)im.h, (int64_t)im.w, (int64_t)im.ncomp, (int64_t)im.hs, (int64_t)im.vs, (int64_t)im.mcux, (int64_t)im.mcuy,
+                              (int64_t)im.bpm, (int64_t)im.blocks, (int64_t)im.restart, (int64_t)im.rst_off, (int64_t)im.tabset, (int64_t)im.qt,
+                              (int64_t)im.yw, (int64_t)im.yh, (int64_t)im.cw, (int64_t)im.ch, im.scan_off, im.scan_len, im.stream_off, im.coef_off,
+                              im.sub_off, im.plane_off, im.rgb_off, im.gray_off})
+                h_img = fnv(h_img, v);
+            int64_t *f = file_rows + (size_t)FILE_ROW * C.file_index[j];
+            const int64_t row[FILE_ROW] = {(int64_t)k, (int64_t)j, im.tabset, im.qt, im.rgb_off, im.gray_off, im.scan_off, im.rst_off};
+            memcpy(f, row, sizeof(row));
+        }
+        for (const v5j::UploadRun &r : C.runs) {
+            const int64_t rel = (int64_t)(reinterpret_cast<intptr_t>(r.src) - base);
+            h_run = fnv(fnv(fnv(h_run, (int64_t)r.dev_off), rel), (int64_t)r.bytes);
+            if (*n_runs < max_runs) {
+                const int64_t row[4] = {(int64_t)k, (int64_t)r.dev_off, rel, (int64_t)r.bytes};
+                memcpy(run_rows + 4 * (size_t)*n_runs, row, sizeof(row));
+            }
+            ++*n_runs;
+        }
+        if ((int)k >= max_chunks) continue;
+        const int64_t row[PLAN_ROW] = {(int64_t)C.images.size(), C.file_index[0], (int64_t)C.off_tab, (int64_t)C.off_q, (int64_t)C.off_scan,
+                                       (int64_t)C.stage_bytes, (int64_t)C.host_stage_bytes, (int64_t)C.runs.size(), (int64_t)C.scan_bytes,
+                                       (int64_t)C.stream_bytes, (int64_t)C.coef_blocks, (int64_t)C.plane_bytes, (int64_t)C.subs,
+                                       (int64_t)C.rst_entries, C.max_windows, C.max_intervals, C.max_blocks, C.max_groups, C.one_launch,
+                                       C.parts, C.launches, (int64_t)(h_img >> 1), (int64_t)(h_run >> 1)};
+        memcpy(chunk_rows + (size_t)PLAN_ROW * k, row, sizeof(row));
+    }
+    const int rc = P->status;
+    delete P;
+    return rc;
 }
