@@ -503,6 +503,23 @@ static unsigned fft_threads(int points)
     return 256u;
 }
 
+// V5ELA_FFT=0 sends every frame down the exact-size DFT (tests compare the two paths); read on every call.
+static bool fft_enabled()
+{
+    const char *env = getenv("V5ELA_FFT");
+    return !(env && atoi(env) == 0);
+}
+
+// Workspace cap of one pass of a spectrum call: ~1 GiB of float64 intermediates, or V5ELA_SPEC_CHUNK_MB (tuning knob).
+static size_t spec_chunk_bytes()
+{
+    if (const char *env = getenv("V5ELA_SPEC_CHUNK_MB")) {
+        const long v = atol(env);
+        if (v >= 1 && v <= 4096) return (size_t)v << 20;
+    }
+    return (size_t)1 << 30;
+}
+
 int v5ela_spectrum(v5ela_handle *h, const uint8_t *d_gray, int n, int height, int width, int64_t frame_stride_bytes,
                    int64_t row_stride_bytes, uint8_t *d_out, void *cuda_stream)
 {
@@ -530,14 +547,9 @@ int v5ela_spectrum(v5ela_handle *h, const uint8_t *d_gray, int n, int height, in
     }
     // frames per pass: keep the float64 workspace (24 bytes per half-spectrum sample) under ~1 GiB. Smaller, L2-sized passes were
     // measured and are SLOWER (profiles/r02/spectrum.txt: 64 MB -10 %, 32 MB -25 %): the passes are bound by their own latency chains,
-    // not by where the intermediate lives. V5ELA_SPEC_CHUNK_MB overrides (tuning knob).
+    // not by where the intermediate lives.
     const size_t per_frame = (size_t)height * wh;
-    size_t chunk_bytes = (size_t)1 << 30;
-    if (const char *env = getenv("V5ELA_SPEC_CHUNK_MB")) {
-        const long v = atol(env);
-        if (v >= 1 && v <= 4096) chunk_bytes = (size_t)v << 20;
-    }
-    int chunk = (int)(chunk_bytes / (per_frame * 24));
+    int chunk = (int)(spec_chunk_bytes() / (per_frame * 24));
     if (chunk < 1) chunk = 1;
     if (chunk > n) chunk = n;
     if (chunk > 65535) chunk = 65535;
@@ -546,15 +558,12 @@ int v5ela_spectrum(v5ela_handle *h, const uint8_t *d_gray, int n, int height, in
     if ((rc = h->d_minmax.ensure(h, sizeof(unsigned long long) * 2 * (size_t)chunk))) return rc;
     const dim3 grid((wh + v5fft::TILE - 1) / v5fft::TILE, (height + v5fft::TILE - 1) / v5fft::TILE, 1);
     // Sizes with only 2/3/5 as prime factors take the shared-memory FFT; anything else (crops are arbitrary) the exact-size
-    // DFT products. V5ELA_FFT=0 forces the latter (tests compare the two).
+    // DFT products (v5fft::fft_path).
     v5fft::FftPlan plan_w, plan_h;
-    const char *fft_env = getenv("V5ELA_FFT");
-    const size_t rows_smem = sizeof(double2) * 2 * (size_t)width;
-    int cc = (int)((size_t)(96u << 10) / (sizeof(double2) * 2 * (size_t)height));
-    cc = cc >= 4 ? 4 : (cc >= 2 ? 2 : cc);                      // 1, 2 or 4 adjacent columns per CTA (the kernel shifts and masks)
-    const size_t cols_smem = sizeof(double2) * 2 * (size_t)(cc > 0 ? cc : 1) * (size_t)height;
-    const bool fast = !(fft_env && atoi(fft_env) == 0) && v5fft::make_plan(width, plan_w) && v5fft::make_plan(height, plan_h) &&
-                      cc >= 1 && rows_smem <= (200u << 10) && cols_smem <= (200u << 10) && n <= 65535;
+    v5fft::FftShape shape;
+    const bool fast = v5fft::fft_path(fft_enabled(), height, width, plan_w, plan_h, shape) && n <= 65535;
+    const int cc = shape.cc;
+    const size_t rows_smem = shape.rows_smem, cols_smem = shape.cols_smem;
     if (fast && !h->fft_attr_set) {
         V5_CUDA(h, cudaFuncSetAttribute(v5fft::fft_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 << 10));
         V5_CUDA(h, cudaFuncSetAttribute(v5fft::fft_cols_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 << 10));
@@ -613,6 +622,126 @@ int v5ela_spectrum_host(v5ela_handle *h, const uint8_t *gray_host, int n, int he
     V5_CUDA(h, cudaStreamSynchronize(st));
     return V5ELA_OK;
 }
+
+int v5ela_spectrum_ragged(v5ela_handle *h, const v5ela_gray_desc *frames_host, int n, void *cuda_stream)
+try {
+    if (!h) return V5ELA_ERR_INVALID;
+    if (n == 0) return V5ELA_OK;
+    v5fft::SpecPlan P;
+    v5fft::plan_spectrum_ragged(frames_host, n, fft_enabled(), spec_chunk_bytes(), P);
+    if (P.status) {
+        if (P.bad_frame >= 0) snprintf(h->err, sizeof(h->err), "v5ela_spectrum_ragged: frame %d: %s", P.bad_frame, P.error);
+        else snprintf(h->err, sizeof(h->err), "v5ela_spectrum_ragged: %s", P.error);
+        return P.status;
+    }
+    DeviceGuard guard(h->device);
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    ScratchOrder order(h, st);                                  // twiddle arena, d_g / d_ms / d_minmax, plan table
+    int rc;
+    if ((rc = h->tw_rag.ensure(h, sizeof(double2) * P.tw_elems)) || (rc = h->d_g.ensure(h, sizeof(double2) * P.g_max)) ||
+        (rc = h->d_ms.ensure(h, sizeof(double) * P.ms_max)) || (rc = h->d_minmax.ensure(h, sizeof(unsigned long long) * 2 * (size_t)P.mm_max)))
+        return rc;
+    const size_t need = P.table_bytes;
+    if (h->h_table.capacity() < need || h->d_table.capacity() < need) {   // the staging buffer and its device copy grow together
+        if (h->ev_table) cudaEventSynchronize(h->ev_table);
+        h->h_table.reset();
+        h->d_table.reset();
+        const size_t cap = need < 4096 ? 4096 : need * 2;
+        if ((rc = h->h_table.ensure(h, need, cap)) || (rc = h->d_table.ensure(h, cap))) return rc;
+    }
+    V5_CUDA(h, h->ev_table.create());
+    V5_CUDA(h, cudaEventSynchronize(h->ev_table));              // the previous call's upload has left the staging buffer
+    uint8_t *tab = h->h_table;
+    memcpy(tab + P.off_sizes, P.sizes.data(), sizeof(v5fft::SpecSize) * P.sizes.size());
+    memcpy(tab + P.off_frames, P.frames.data(), sizeof(v5fft::SpecFrame) * P.frames.size());
+    memcpy(tab + P.off_tw_base, P.tw_base.data(), sizeof(uint32_t) * P.tw_base.size());
+    memcpy(tab + P.off_bases, P.bases.data(), sizeof(uint32_t) * P.bases.size());
+    V5_CUDA(h, cudaMemcpyAsync(h->d_table, h->h_table, need, cudaMemcpyHostToDevice, st));
+    V5_CUDA(h, cudaEventRecord(h->ev_table, st));
+    if (!h->fft_rag_attr_set) {
+        V5_CUDA(h, cudaFuncSetAttribute(v5fft::fft_rows_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)v5fft::FFT_SMEM_MAX));
+        V5_CUDA(h, cudaFuncSetAttribute(v5fft::fft_cols_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)v5fft::FFT_SMEM_MAX));
+        h->fft_rag_attr_set = true;
+    }
+    const uint8_t *dt = h->d_table;
+    const auto *sizes = reinterpret_cast<const v5fft::SpecSize *>(dt + P.off_sizes);
+    const auto *frames = reinterpret_cast<const v5fft::SpecFrame *>(dt + P.off_frames);
+    const auto *bases = reinterpret_cast<const uint32_t *>(dt + P.off_bases);
+    v5fft::twiddle_ragged_kernel<<<P.tw_base.back(), 256, 0, st>>>(sizes, (int)P.sizes.size(), reinterpret_cast<const uint32_t *>(dt + P.off_tw_base),
+                                                                   h->tw_rag);
+    V5_CUDA(h, cudaGetLastError());
+    h->launches++;
+    for (const v5fft::SpecChunk &C : P.chunks) {
+        const v5fft::SpecFrame *cf = frames + C.f0;
+        const uint32_t *base = bases + C.off_base;
+        auto kind = [&](int k) { return base + (size_t)k * (C.n + 1); };
+        // min/max slots: {~0, 0} per frame
+        V5_CUDA(h, cudaMemsetAsync(h->d_minmax, 0, sizeof(unsigned long long) * 2 * (size_t)C.n, st));
+        V5_CUDA(h, cudaMemset2DAsync(h->d_minmax, 16, 0xff, 8, (size_t)C.n, st));
+        if (C.ctas[v5fft::L_FFT_ROWS]) {
+            v5fft::fft_rows_ragged_kernel<<<C.ctas[v5fft::L_FFT_ROWS], 256, C.rows_smem, st>>>(cf, C.n, kind(v5fft::L_FFT_ROWS), sizes, h->tw_rag, h->d_g);
+            V5_CUDA(h, cudaGetLastError());
+            v5fft::fft_cols_ragged_kernel<<<C.ctas[v5fft::L_FFT_COLS], 256, C.cols_smem, st>>>(cf, C.n, kind(v5fft::L_FFT_COLS), sizes, h->tw_rag, h->d_g,
+                                                                                              h->d_ms, h->d_minmax);
+            V5_CUDA(h, cudaGetLastError());
+            h->launches += 2;
+        }
+        if (C.ctas[v5fft::L_DFT_ROWS]) {
+            v5fft::dft_rows_ragged_kernel<<<C.ctas[v5fft::L_DFT_ROWS], 256, 0, st>>>(cf, C.n, kind(v5fft::L_DFT_ROWS), sizes, h->tw_rag, h->d_g);
+            V5_CUDA(h, cudaGetLastError());
+            v5fft::dft_cols_ragged_kernel<<<C.ctas[v5fft::L_DFT_COLS], 256, 0, st>>>(cf, C.n, kind(v5fft::L_DFT_COLS), sizes, h->tw_rag, h->d_g, h->d_ms,
+                                                                                    h->d_minmax);
+            V5_CUDA(h, cudaGetLastError());
+            h->launches += 2;
+        }
+        v5fft::spectrum_image_ragged_kernel<<<C.ctas[v5fft::L_IMAGE], 256, 0, st>>>(cf, C.n, kind(v5fft::L_IMAGE), h->d_ms, h->d_minmax);
+        V5_CUDA(h, cudaGetLastError());
+        h->launches++;
+    }
+    return V5ELA_OK;
+} V5_CATCH(h)
+
+int v5ela_spectrum_ragged_host(v5ela_handle *h, const v5ela_gray_desc *frames_host, int n)
+try {
+    if (!h) return V5ELA_ERR_INVALID;
+    if (n == 0) return V5ELA_OK;
+    if (!frames_host || n < 0) return fail(h, V5ELA_ERR_INVALID, "v5ela_spectrum_ragged_host: null descriptor array or negative count%s");
+    // device arena: per image its pixels (rows packed), 256-byte aligned; the images' spectra at the same offsets of d_spec
+    std::vector<v5ela_gray_desc> dev((size_t)n);
+    std::vector<size_t> off((size_t)n);
+    size_t total = 0;
+    for (int i = 0; i < n; i++) {
+        if (const char *why = v5fft::gray_desc_error(frames_host[i])) {
+            snprintf(h->err, sizeof(h->err), "v5ela_spectrum_ragged_host: frame %d: %s", i, why);
+            return V5ELA_ERR_INVALID;
+        }
+        off[(size_t)i] = total;
+        total += ((size_t)frames_host[i].height * frames_host[i].width + 255) / 256 * 256;
+    }
+    DeviceGuard guard(h->device);
+    int rc;
+    cudaStream_t st;
+    if ((rc = internal_stream(h, &st))) return rc;
+    ScratchOrder order(h, st);                                  // d_gray / d_spec
+    if ((rc = h->d_gray.ensure(h, total)) || (rc = h->d_spec.ensure(h, total))) return rc;
+    for (int i = 0; i < n; i++) {
+        const v5ela_gray_desc &f = frames_host[i];
+        V5_CUDA(h, cudaMemcpy2DAsync(h->d_gray + off[(size_t)i], (size_t)f.width, f.gray, (size_t)f.row_stride_bytes, (size_t)f.width,
+                                     (size_t)f.height, cudaMemcpyHostToDevice, st));
+        dev[(size_t)i].gray = h->d_gray + off[(size_t)i];
+        dev[(size_t)i].height = f.height;
+        dev[(size_t)i].width = f.width;
+        dev[(size_t)i].row_stride_bytes = f.width;
+        dev[(size_t)i].out = h->d_spec + off[(size_t)i];
+    }
+    if ((rc = v5ela_spectrum_ragged(h, dev.data(), n, st))) return rc;
+    for (int i = 0; i < n; i++) {
+        const v5ela_gray_desc &f = frames_host[i];
+        V5_CUDA(h, cudaMemcpyAsync(f.out, h->d_spec + off[(size_t)i], (size_t)f.height * f.width, cudaMemcpyDeviceToHost, st));
+    }
+    V5_CUDA(h, cudaStreamSynchronize(st));
+    return V5ELA_OK;
+} V5_CATCH(h)
 
 int v5ela_profile_enable(v5ela_handle *h, int enable)
 try {

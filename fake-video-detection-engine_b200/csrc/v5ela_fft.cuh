@@ -11,6 +11,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "v5ela_spec_plan.h"                                    // FftPlan, make_plan, TILE, the ragged plan
+
 namespace v5fft {
 
 // tw[m] = exp(-2*pi*i*m/n)
@@ -23,7 +25,6 @@ __global__ void twiddle_kernel(double2 *tw, int n)
     tw[m] = make_double2(c, -s);
 }
 
-constexpr int TILE = 32;     // output tile edge per CTA (16x16 threads, 2x2 outputs each)
 constexpr int KC = 32;       // reduction chunk staged in shared memory
 
 // G[y][v] = sum_x gray[y][x] * twW[(x*v) mod W],  v in [0, W/2]
@@ -133,37 +134,8 @@ __global__ void __launch_bounds__(256) dft_cols_kernel(const double2 *__restrict
 // (n * s == N): for p in [0, n/r), q in [0, s):
 //     a_t = x[q + s*(p + t*n/r)],  b_u = (sum_t a_t w_r^{t u}) * exp(-2 pi i p u s / N),  y[q + s*(r*p + u)] = b_u
 // then n /= r, s *= r and the buffers swap. p*u*s < N, so the twiddle is a direct index into the N-entry table.
-struct FftPlan {
-    int n;
-    int nst;
-    int radix[24];
-    uint32_t inv_s[24];         // floor(2^32 / s) + 1 for the stride s of every stage: idx / s == umulhi(idx, inv_s) for idx < 2^16
-    uint32_t inv_per_seq[24];   // the same for N / radix (butterflies per sequence)
-};
-
-// exact unsigned division of a < 2^16 by d in 2..2^16 through its reciprocal (error term a / 2^32 < 1 / d)
-__host__ __device__ __forceinline__ uint32_t recip_u16(uint32_t d) { return (uint32_t)(0x100000000ull / d) + 1u; }
+// (FftPlan, recip_u16 and make_plan live in v5ela_spec_plan.h)
 __device__ __forceinline__ int div_u16(int a, uint32_t inv) { return (int)__umulhi((uint32_t)a, inv); }
-
-// Host: factor n into 5s, 3s and 2s; returns false when another prime factor remains.
-inline bool make_plan(int n, FftPlan &plan)
-{
-    plan.n = n;
-    plan.nst = 0;
-    const int rs[4] = {5, 3, 4, 2};                             // radix 4 before 2: half the stages (barriers, shared-memory passes)
-    for (int r : rs)
-        while (n % r == 0 && plan.nst < 24) {
-            plan.radix[plan.nst++] = r;
-            n /= r;
-        }
-    int s = 1;
-    for (int st = 0; st < plan.nst; st++) {
-        plan.inv_s[st] = recip_u16((uint32_t)s);
-        plan.inv_per_seq[st] = recip_u16((uint32_t)(plan.n / plan.radix[st]));
-        s *= plan.radix[st];
-    }
-    return n == 1 && plan.n <= 65536;
-}
 
 __device__ __forceinline__ double2 cadd(double2 a, double2 b) { return make_double2(a.x + b.x, a.y + b.y); }
 __device__ __forceinline__ double2 csub(double2 a, double2 b) { return make_double2(a.x - b.x, a.y - b.y); }
@@ -377,6 +349,263 @@ __global__ void __launch_bounds__(256) spectrum_image_kernel(const double *__res
             const int u = v >= wh ? um : u0;
             v = v >= wh ? w - v : v;
             double r = rint(__dadd_rn(__dmul_rn(src[(int64_t)u * wh + v], scale), shift));   // cvRound: ties to even
+            r = r < 0.0 ? 0.0 : (r > 255.0 ? 255.0 : r);
+            dst[(int64_t)i * w + j] = (uint8_t)r;
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// Ragged calls (v5ela_spectrum_ragged): frames of different sizes in one launch sequence, planned on the host
+// (v5ela_spec_plan.h). Each kernel flattens its grid in x; a CTA finds its frame through the chunk's CTA prefix table
+// (cta_frame) and then runs the body of the uniform kernel above for that frame, with the frame's FftPlan read from the size
+// table instead of a __grid_constant__. The bodies are copies, not shared functions, so that the uniform kernels' code stays
+// exactly as it is; every arithmetic step is the same, so every frame's image is byte-identical to v5ela_spectrum's.
+
+// The twiddle tables of every distinct side of the call, back to back in one arena: blockDim.x entries per CTA.
+__global__ void __launch_bounds__(256) twiddle_ragged_kernel(const SpecSize *__restrict__ sizes, int ns, const uint32_t *__restrict__ base,
+                                                             double2 *__restrict__ tw)
+{
+    const int k = cta_frame(base, ns, blockIdx.x);
+    const int n = sizes[k].n;
+    const int m = (int)(blockIdx.x - base[k]) * blockDim.x + threadIdx.x;
+    if (m >= n) return;
+    double s, c;
+    sincospi(2.0 * (double)m / (double)n, &s, &c);
+    tw[sizes[k].tw + m] = make_double2(c, -s);
+}
+
+// dft_rows_kernel for one TILE x TILE output tile of one frame
+__global__ void __launch_bounds__(256) dft_rows_ragged_kernel(const SpecFrame *__restrict__ frames, int nf, const uint32_t *__restrict__ base,
+                                                              const SpecSize *__restrict__ sizes, const double2 *__restrict__ tw_arena,
+                                                              double2 *__restrict__ g)
+{
+    __shared__ double xs[TILE][KC + 1];
+    const int fi = cta_frame(base, nf, blockIdx.x);
+    const SpecFrame f = frames[fi];
+    const int local = (int)(blockIdx.x - base[fi]), ty_ = local / f.gx;
+    const int h = f.h, w = f.w, wh = f.wh;
+    const int64_t row_stride = f.row_stride;
+    const double2 *__restrict__ tw = tw_arena + sizes[f.sw].tw;
+    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+    const int y0 = ty_ * TILE, v0 = (local - ty_ * f.gx) * TILE;
+    const uint8_t *src = f.gray;
+    const int va = v0 + tx, vb = v0 + tx + 16;
+    int ia = 0, ib = 0;
+    const int sa = va % w, sb = vb % w;
+    double2 acc[2][2] = {{{0, 0}, {0, 0}}, {{0, 0}, {0, 0}}};
+    for (int x0 = 0; x0 < w; x0 += KC) {
+        for (int i = threadIdx.x; i < TILE * KC; i += 256) {
+            const int r = i / KC, c = i - r * KC;
+            const int y = y0 + r, x = x0 + c;
+            xs[r][c] = (y < h && x < w) ? (double)src[(int64_t)y * row_stride + x] : 0.0;
+        }
+        __syncthreads();
+        const int kn = min(KC, w - x0);
+        for (int k = 0; k < kn; k++) {
+            const double2 ta = tw[ia], tb = tw[ib];
+            const double xa = xs[ty][k], xb = xs[ty + 16][k];
+            acc[0][0].x = fma(xa, ta.x, acc[0][0].x); acc[0][0].y = fma(xa, ta.y, acc[0][0].y);
+            acc[0][1].x = fma(xa, tb.x, acc[0][1].x); acc[0][1].y = fma(xa, tb.y, acc[0][1].y);
+            acc[1][0].x = fma(xb, ta.x, acc[1][0].x); acc[1][0].y = fma(xb, ta.y, acc[1][0].y);
+            acc[1][1].x = fma(xb, tb.x, acc[1][1].x); acc[1][1].y = fma(xb, tb.y, acc[1][1].y);
+            ia += sa; ia = ia >= w ? ia - w : ia;
+            ib += sb; ib = ib >= w ? ib - w : ib;
+        }
+        __syncthreads();
+    }
+    double2 *dst = g + f.g_off;
+#pragma unroll
+    for (int i = 0; i < 2; i++) {
+        const int y = y0 + ty + 16 * i;
+        if (y >= h) continue;
+        if (va < wh) dst[(int64_t)y * wh + va] = acc[i][0];
+        if (vb < wh) dst[(int64_t)y * wh + vb] = acc[i][1];
+    }
+}
+
+// dft_cols_kernel for one TILE x TILE output tile of one frame
+__global__ void __launch_bounds__(256) dft_cols_ragged_kernel(const SpecFrame *__restrict__ frames, int nf, const uint32_t *__restrict__ base,
+                                                              const SpecSize *__restrict__ sizes, const double2 *__restrict__ tw_arena,
+                                                              const double2 *__restrict__ g, double *__restrict__ ms,
+                                                              unsigned long long *__restrict__ minmax)
+{
+    __shared__ double2 gs[KC][TILE + 1];
+    __shared__ unsigned long long smin, smax;
+    const int fi = cta_frame(base, nf, blockIdx.x);
+    const SpecFrame f = frames[fi];
+    const int local = (int)(blockIdx.x - base[fi]), ty_ = local / f.gx;
+    const int h = f.h, wh = f.wh;
+    const double2 *__restrict__ tw = tw_arena + sizes[f.sh].tw;
+    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+    const int u0 = ty_ * TILE, v0 = (local - ty_ * f.gx) * TILE;
+    const double2 *src = g + f.g_off;
+    if (threadIdx.x == 0) { smin = ~0ull; smax = 0ull; }
+    const int ua = u0 + ty, ub = u0 + ty + 16;
+    int ia = 0, ib = 0;
+    const int sa = ua % h, sb = ub % h;
+    double2 acc[2][2] = {{{0, 0}, {0, 0}}, {{0, 0}, {0, 0}}};
+    for (int y0 = 0; y0 < h; y0 += KC) {
+        for (int i = threadIdx.x; i < KC * TILE; i += 256) {
+            const int r = i / TILE, c = i - r * TILE;
+            const int y = y0 + r, v = v0 + c;
+            gs[r][c] = (y < h && v < wh) ? src[(int64_t)y * wh + v] : make_double2(0.0, 0.0);
+        }
+        __syncthreads();
+        const int kn = min(KC, h - y0);
+        for (int k = 0; k < kn; k++) {
+            const double2 ta = tw[ia], tb = tw[ib];
+            const double2 ga = gs[k][tx], gb = gs[k][tx + 16];
+            acc[0][0].x = fma(ga.x, ta.x, fma(-ga.y, ta.y, acc[0][0].x)); acc[0][0].y = fma(ga.x, ta.y, fma(ga.y, ta.x, acc[0][0].y));
+            acc[0][1].x = fma(gb.x, ta.x, fma(-gb.y, ta.y, acc[0][1].x)); acc[0][1].y = fma(gb.x, ta.y, fma(gb.y, ta.x, acc[0][1].y));
+            acc[1][0].x = fma(ga.x, tb.x, fma(-ga.y, tb.y, acc[1][0].x)); acc[1][0].y = fma(ga.x, tb.y, fma(ga.y, tb.x, acc[1][0].y));
+            acc[1][1].x = fma(gb.x, tb.x, fma(-gb.y, tb.y, acc[1][1].x)); acc[1][1].y = fma(gb.x, tb.y, fma(gb.y, tb.x, acc[1][1].y));
+            ia += sa; ia = ia >= h ? ia - h : ia;
+            ib += sb; ib = ib >= h ? ib - h : ib;
+        }
+        __syncthreads();
+    }
+    double *dst = ms + f.ms_off;
+    unsigned long long lo = ~0ull, hi = 0ull;
+#pragma unroll
+    for (int i = 0; i < 2; i++) {
+#pragma unroll
+        for (int j = 0; j < 2; j++) {
+            const int u = u0 + ty + 16 * i, v = v0 + tx + 16 * j;
+            if (u >= h || v >= wh) continue;
+            const double m = 20.0 * log(hypot(acc[i][j].x, acc[i][j].y) + 1.0);
+            dst[(int64_t)u * wh + v] = m;
+            const unsigned long long bits = (unsigned long long)__double_as_longlong(m);
+            lo = bits < lo ? bits : lo;
+            hi = bits > hi ? bits : hi;
+        }
+    }
+    atomicMin(&smin, lo);
+    atomicMax(&smax, hi);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        atomicMin(&minmax[2 * f.mm], smin);
+        atomicMax(&minmax[2 * f.mm + 1], smax);
+    }
+}
+
+// fft_rows_kernel for one pair of rows of one frame
+__global__ void __launch_bounds__(512) fft_rows_ragged_kernel(const SpecFrame *__restrict__ frames, int nf, const uint32_t *__restrict__ base,
+                                                              const SpecSize *__restrict__ sizes, const double2 *__restrict__ tw_arena,
+                                                              double2 *__restrict__ g)
+{
+    extern __shared__ double2 fbuf[];
+    const int fi = cta_frame(base, nf, blockIdx.x);
+    const SpecFrame f = frames[fi];
+    const int h = f.h, w = f.w, wh = f.wh;
+    const SpecSize &sz = sizes[f.sw];
+    const int y0 = 2 * (int)(blockIdx.x - base[fi]), y1 = y0 + 1;
+    const uint8_t *src = f.gray;
+    const uint8_t *r0 = src + (int64_t)y0 * f.row_stride, *r1 = src + (int64_t)(y1 < h ? y1 : y0) * f.row_stride;
+    for (int xb = 0; xb < w; xb += 4 * blockDim.x) {
+        uint8_t a[4], b[4];
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const int x = xb + j * blockDim.x + threadIdx.x;
+            a[j] = x < w ? r0[x] : 0;
+            b[j] = x < w ? r1[x] : 0;
+        }
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const int x = xb + j * blockDim.x + threadIdx.x;
+            if (x < w) fbuf[x] = make_double2((double)a[j], y1 < h ? (double)b[j] : 0.0);
+        }
+    }
+    __syncthreads();
+    const double2 *res = stockham(fbuf, fbuf + w, 1, sz.plan, tw_arena + sz.tw);
+    double2 *ga = g + f.g_off + (int64_t)y0 * wh;
+    for (int k = threadIdx.x; k < wh; k += blockDim.x) {
+        const double2 zk = res[k], zn = res[k == 0 ? 0 : w - k];
+        ga[k] = make_double2(0.5 * (zk.x + zn.x), 0.5 * (zk.y - zn.y));
+        if (y1 < h) ga[wh + k] = make_double2(0.5 * (zk.y + zn.y), 0.5 * (zn.x - zk.x));
+    }
+}
+
+// fft_cols_kernel for cc adjacent columns of one frame
+__global__ void __launch_bounds__(512) fft_cols_ragged_kernel(const SpecFrame *__restrict__ frames, int nf, const uint32_t *__restrict__ base,
+                                                              const SpecSize *__restrict__ sizes, const double2 *__restrict__ tw_arena,
+                                                              const double2 *__restrict__ g, double *__restrict__ ms,
+                                                              unsigned long long *__restrict__ minmax)
+{
+    extern __shared__ double2 fbuf[];
+    __shared__ unsigned long long smin, smax;
+    __shared__ LogTab logtab;
+    if (threadIdx.x == 0) { smin = ~0ull; smax = 0ull; }
+    logtab_fill(logtab);
+    const int fi = cta_frame(base, nf, blockIdx.x);
+    const SpecFrame f = frames[fi];
+    const int h = f.h, wh = f.wh, cc = f.cc;
+    const SpecSize &sz = sizes[f.sh];
+    const int v0 = (int)(blockIdx.x - base[fi]) * cc;
+    const double2 *src = g + f.g_off;
+    const int csh = cc == 4 ? 2 : (cc == 2 ? 1 : 0);
+    for (int ib = 0; ib < h * cc; ib += 4 * blockDim.x) {
+        double2 t[4];
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const int i = ib + j * blockDim.x + threadIdx.x;
+            const int y = i >> csh, c = i & (cc - 1);
+            t[j] = (i < h * cc && v0 + c < wh) ? src[(int64_t)y * wh + v0 + c] : make_double2(0.0, 0.0);
+        }
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const int i = ib + j * blockDim.x + threadIdx.x;
+            const int y = i >> csh, c = i & (cc - 1);
+            if (i < h * cc) fbuf[c * h + y] = t[j];
+        }
+    }
+    __syncthreads();
+    const double2 *res = stockham(fbuf, fbuf + cc * h, cc, sz.plan, tw_arena + sz.tw);
+    double *dst = ms + f.ms_off;
+    unsigned long long lo = ~0ull, hi = 0ull;
+    for (int i = threadIdx.x; i < h * cc; i += blockDim.x) {
+        const int u = i >> csh, c = i & (cc - 1);
+        if (v0 + c >= wh) continue;
+        const double2 fv = res[c * h + u];
+        const double m = log_magnitude20(logtab, fma(fv.x, fv.x, fv.y * fv.y));
+        dst[(int64_t)u * wh + v0 + c] = m;
+        const unsigned long long bits = (unsigned long long)__double_as_longlong(m);
+        lo = bits < lo ? bits : lo;
+        hi = bits > hi ? bits : hi;
+    }
+    atomicMin(&smin, lo);
+    atomicMax(&smax, hi);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        atomicMin(&minmax[2 * f.mm], smin);
+        atomicMax(&minmax[2 * f.mm + 1], smax);
+    }
+}
+
+// spectrum_image_kernel for one (column block, row block) of one frame: f.bx x f.by CTAs per frame
+__global__ void __launch_bounds__(256) spectrum_image_ragged_kernel(const SpecFrame *__restrict__ frames, int nf, const uint32_t *__restrict__ base,
+                                                                    const double *__restrict__ ms,
+                                                                    const unsigned long long *__restrict__ minmax)
+{
+    const int fi = cta_frame(base, nf, blockIdx.x);
+    const SpecFrame f = frames[fi];
+    const int local = (int)(blockIdx.x - base[fi]), by_ = local / f.bx, bx_ = local - by_ * f.bx;
+    const int h = f.h, w = f.w, wh = f.wh;
+    const double mn = __longlong_as_double((long long)minmax[2 * f.mm]), mx = __longlong_as_double((long long)minmax[2 * f.mm + 1]);
+    const double scale = (mx - mn) > 2.220446049250313e-16 ? 255.0 / (mx - mn) : 0.0;
+    const double shift = 0.0 - mn * scale;
+    const double *src = ms + f.ms_off;
+    uint8_t *dst = f.out;
+    for (int i = by_; i < h; i += f.by) {
+        int u0 = i - h / 2;
+        u0 = u0 < 0 ? u0 + h : u0;
+        const int um = u0 == 0 ? 0 : h - u0;
+        for (int j = bx_ * blockDim.x + threadIdx.x; j < w; j += f.bx * blockDim.x) {
+            int v = j - w / 2;
+            v = v < 0 ? v + w : v;
+            const int u = v >= wh ? um : u0;
+            v = v >= wh ? w - v : v;
+            double r = rint(__dadd_rn(__dmul_rn(src[(int64_t)u * wh + v], scale), shift));
             r = r < 0.0 ? 0.0 : (r > 255.0 ? 255.0 : r);
             dst[(int64_t)i * w + j] = (uint8_t)r;
         }

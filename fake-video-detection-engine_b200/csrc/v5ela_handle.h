@@ -131,6 +131,8 @@ struct v5ela_handle {
     v5host::DeviceBuf<double2> tw_w, tw_h;
     int tw_w_n = 0, tw_h_n = 0;
     bool fft_attr_set = false;
+    v5host::DeviceBuf<double2> tw_rag;     // ragged spectrum calls: the twiddle tables of the call's distinct sides
+    bool fft_rag_attr_set = false;
     v5host::DeviceBuf<double2> d_g;
     v5host::DeviceBuf<double> d_ms;
     v5host::DeviceBuf<unsigned long long> d_minmax;

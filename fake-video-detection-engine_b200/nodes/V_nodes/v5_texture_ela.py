@@ -10,8 +10,8 @@ Behaviour contract kept from the reference (line numbers: /root/reference/nodes/
 What runs on the B200 instead of Pillow/OpenCV/NumPy:
   * decoding the crop file, both as RGB (:64) and as its luma plane (:83), through ``v5ela_jpeg_decode_host`` — pixel-identical;
   * the error-level analysis (:66-78) through ``v5ela_analyze_host`` — bit-exact;
-  * the FFT log-magnitude image (:84-88) through ``v5ela_spectrum_host`` (within one grey level of NumPy; identical on
-    every golden crop);
+  * the FFT log-magnitude image (:84-88) of every crop through one ``v5ela_spectrum_ragged_host`` call (within one grey level of
+    NumPy; identical on every golden crop);
   * JPEG-encoding the three files the reference leaves in ``ela_analysis/`` — the scratch file ``temp_ela_{i}.jpg`` (:66-67,
     quality 90), ``ela_{i}.jpg`` (:80-81, quality 75) and ``fft_{i}.jpg`` (:90-91, quality 95, one component) — through
     ``v5ela_jpeg_encode_host``; the files equal the reference's byte for byte.
@@ -94,8 +94,9 @@ def _write_jpeg(path, image, quality, device, gpu_codec):
 
 def _gpu_artefacts(crops, ela_dir, state):
     """ELA + spectrum artefacts of the selected crops. ``crops``: list of (rank, crop_path). All crops — whatever their sizes — go
-    through ONE ragged analysis call (one upload, one launch sequence, one download: ``v5ela_analyze_ragged_host``); a crop that
-    cannot be read is reported and left out, like any per-face failure of the reference (:140-144).
+    through ONE ragged analysis call (one upload, one launch sequence, one download: ``v5ela_analyze_ragged_host``) and ONE ragged
+    spectrum call (``v5ela_spectrum_ragged_host``); a crop that cannot be read is reported and left out, like any per-face failure
+    of the reference (:140-144).
     Returns {rank: (feature dict, ela path, fft path)}."""
     from v5ela import host as v5host
     from v5ela.records import features
@@ -117,6 +118,8 @@ def _gpu_artefacts(crops, ela_dir, state):
     if not loaded:
         return out
     records, _, enhanced = v5host.analyze_ragged_host([rgb for _, rgb, _ in loaded], quality=quality, want_enhanced=True, device=device)
+    gpu_fft = state.get("v5_gpu_fft", True)
+    spectra = v5host.spectrum_ragged_host([gray for _, _, gray in loaded], device=device) if gpu_fft else None
     for j, (rank, rgb, gray) in enumerate(loaded):
         try:
             if state.get("v5_keep_temp_jpeg", True):
@@ -125,8 +128,8 @@ def _gpu_artefacts(crops, ela_dir, state):
             feats["rank"] = rank
             ela_path = os.path.join(ela_dir, f"ela_{rank}.jpg")
             _write_jpeg(ela_path, enhanced[j], 75, device, gpu_codec)      # PIL's default quality (reference :81)
-            if state.get("v5_gpu_fft", True):
-                spectrum = v5host.spectrum_host(gray, device=device)
+            if gpu_fft:
+                spectrum = spectra[j]
             else:
                 log_mag = 20 * np.log(np.abs(np.fft.fftshift(np.fft.fft2(gray))) + 1)
                 spectrum = cv2.normalize(log_mag, None, 0, 255, cv2.NORM_MINMAX, dtype=cv2.CV_8U)

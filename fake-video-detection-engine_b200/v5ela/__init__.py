@@ -4,6 +4,7 @@ Public surface:
   analyze_batch(frames_u8[N,H,W,3] on cuda) -> {"records", ["residual"], ["enhanced"]}   (v5ela.batch)
   analyze_ragged([frames_u8[H_i,W_i,3] ...]) -> the same for frames of different sizes, one launch (v5ela.batch)
   reduce_records(records, group)                                                           (v5ela.batch)
+  spectrum_batch(gray_u8[N,H,W]) / spectrum_ragged([gray_u8[H_i,W_i] ...])  (FFT log-magnitude images) (v5ela.batch)
   as_records / features / combine                                                          (v5ela.records)
   gen_frame / gen_batch / gen_batch_torch  (synthetic keyframes, SURVEY Appendix B)        (v5ela.synth)
   shard_range / analyze_sharded            (multi-GPU, one process per GPU, NCCL gather)   (v5ela.shard)
@@ -17,7 +18,7 @@ from .synth import gen_batch, gen_batch_torch, gen_frame  # noqa: F401
 
 
 def __getattr__(name):  # lazy: importing the package must not require the CUDA library (CPU-only tooling, tests)
-    if name in ("analyze_batch", "analyze_ragged", "reduce_records", "get_handle", "spectrum_batch", "analyze_jpeg_files"):
+    if name in ("analyze_batch", "analyze_ragged", "reduce_records", "get_handle", "spectrum_batch", "spectrum_ragged", "analyze_jpeg_files"):
         from . import batch
 
         return getattr(batch, name)

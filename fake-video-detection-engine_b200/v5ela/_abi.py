@@ -17,6 +17,7 @@ EXPORTS = (
     "v5ela_profile_read", "v5ela_spectrum", "v5ela_spectrum_host", "v5ela_jpeg_bound", "v5ela_jpeg_encode",
     "v5ela_jpeg_encode_host", "v5ela_jpeg_info", "v5ela_jpeg_info_batch", "v5ela_jpeg_decode", "v5ela_jpeg_decode_host",
     "v5ela_last_instantiation", "v5ela_set_block_stage", "v5ela_get_block_stage", "v5ela_analyze_ragged", "v5ela_analyze_ragged_host",
+    "v5ela_spectrum_ragged", "v5ela_spectrum_ragged_host",
 )
 BLOCK_STAGES = {"smem": 0, "mma": 1}
 INSTANTIATIONS = {0: "general", 1: "fast", 2: "texhist", -1: None}
@@ -26,6 +27,12 @@ class FrameDesc(ctypes.Structure):
     """v5ela_frame_desc (include/v5ela.h): one frame of a ragged batch."""
     _fields_ = [("rgb", ctypes.c_void_p), ("height", ctypes.c_int32), ("width", ctypes.c_int32), ("row_stride_bytes", ctypes.c_int64),
                 ("residual", ctypes.c_void_p), ("enhanced", ctypes.c_void_p)]
+
+
+class GrayDesc(ctypes.Structure):
+    """v5ela_gray_desc (include/v5ela.h): one image of a ragged spectrum batch."""
+    _fields_ = [("gray", ctypes.c_void_p), ("height", ctypes.c_int32), ("width", ctypes.c_int32), ("row_stride_bytes", ctypes.c_int64),
+                ("out", ctypes.c_void_p)]
 
 
 class V5ElaError(RuntimeError):
@@ -72,6 +79,8 @@ def load() -> ctypes.CDLL:
     lib.v5ela_analyze_host.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp]
     lib.v5ela_spectrum.argtypes = [vp, vp, i32, i32, i32, i64, i64, vp, vp]
     lib.v5ela_spectrum_host.argtypes = [vp, vp, i32, i32, i32, vp]
+    lib.v5ela_spectrum_ragged.argtypes = [vp, ctypes.POINTER(GrayDesc), i32, vp]
+    lib.v5ela_spectrum_ragged_host.argtypes = [vp, ctypes.POINTER(GrayDesc), i32]
     lib.v5ela_jpeg_bound.restype = i64
     lib.v5ela_jpeg_bound.argtypes = [i32, i32, i32]
     lib.v5ela_jpeg_encode.argtypes = [vp, vp, i32, i32, i32, i32, i64, i64, i32, vp, i64, vp, vp]
@@ -167,6 +176,14 @@ class Handle:
 
     def spectrum_host(self, gray_host: int, n: int, h: int, w: int, out_host: int):
         self._check(self._lib.v5ela_spectrum_host(self._h, gray_host, n, h, w, out_host))
+
+    def spectrum_ragged(self, descs, n: int, stream: int | None):
+        """descs: ctypes array of GrayDesc holding DEVICE pointers; one launch sequence for images of different sizes."""
+        self._check(self._lib.v5ela_spectrum_ragged(self._h, descs, n, stream or None))
+
+    def spectrum_ragged_host(self, descs, n: int):
+        """descs: ctypes array of GrayDesc holding HOST pointers; synchronous."""
+        self._check(self._lib.v5ela_spectrum_ragged_host(self._h, descs, n))
 
     def jpeg_encode(self, d_img: int, n: int, h: int, w: int, channels: int, frame_stride: int, row_stride: int, quality: int,
                     d_out: int, out_stride: int, d_sizes: int, stream: int | None):

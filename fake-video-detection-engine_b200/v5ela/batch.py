@@ -159,6 +159,50 @@ def spectrum_batch(gray, handle=None):
     return out
 
 
+def spectrum_ragged(grays, handle=None):
+    """FFT log-magnitude spectrum images of images of DIFFERENT sizes in one launch sequence (v5ela_spectrum_ragged): each output
+    is byte-identical to ``spectrum_batch`` of that image alone.
+
+    grays : sequence of torch.uint8 CUDA tensors (H_i, W_i), pixels dense (stride 1), any row stride, all on one device — e.g.
+    crop views into a decoded keyframe's luma plane. Returns a list of (H_i, W_i) uint8 tensors, views into one output arena.
+    Asynchronous on torch's current stream.
+    """
+    import torch
+
+    n = len(grays)
+    if n == 0:
+        return []
+    dev = grays[0].device
+    views = []
+    for g in grays:
+        if not isinstance(g, torch.Tensor) or g.dtype != torch.uint8 or not g.is_cuda or g.dim() != 2:
+            raise ValueError("grays must be torch.uint8 CUDA tensors of shape (H, W)")
+        if g.device != dev:
+            raise ValueError("all images must live on one device")
+        if g.shape[0] == 0 or g.shape[1] == 0:
+            raise ValueError("empty image in a ragged batch")
+        if g.stride(1) != 1:
+            g = g.contiguous()
+        views.append(g)
+    hd = handle or get_handle(dev.index if dev.index is not None else torch.cuda.current_device())
+    sizes = [g.shape[0] * g.shape[1] for g in views]
+    offs = [0]
+    for s_ in sizes:
+        offs.append(offs[-1] + (s_ + 255) // 256 * 256)
+    arena = torch.empty(offs[-1], dtype=torch.uint8, device=dev)
+    outs = [arena[offs[i]:offs[i] + sizes[i]].view(views[i].shape[0], views[i].shape[1]) for i in range(n)]
+    descs = (_abi.GrayDesc * n)()
+    for i, g in enumerate(views):
+        descs[i].gray = g.data_ptr()
+        descs[i].height, descs[i].width = int(g.shape[0]), int(g.shape[1])
+        descs[i].row_stride_bytes = int(g.stride(0))
+        descs[i].out = outs[i].data_ptr()
+    # Contiguous copies (if any) were allocated on this stream: torch's caching allocator hands their memory only to work
+    # ordered after this launch, so they need no reference beyond the call.
+    hd.spectrum_ragged(descs, n, torch.cuda.current_stream(dev).cuda_stream)
+    return outs
+
+
 def analyze_jpeg_files(files, quality: int = 90, device=0, want_residual: bool = False, want_enhanced: bool = False, handle=None):
     """Keyframes / crops as the reference holds them — JPEG files (bytes), all of one size — decoded on the GPU (pixel-identical
     to Image.open(..).convert('RGB'), v5_texture_ela.py:64) and analysed without the pixels ever crossing PCIe: only the

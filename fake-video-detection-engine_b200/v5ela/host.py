@@ -75,3 +75,26 @@ def spectrum_host(gray: np.ndarray, device: int = 0) -> np.ndarray:
     if n and h and w:
         get_handle(device).spectrum_host(g.ctypes.data, n, h, w, out.ctypes.data)
     return out[0] if single else out
+
+
+def spectrum_ragged_host(grays, device: int = 0):
+    """Spectrum images of (H_i, W_i) uint8 host arrays of different sizes through ``v5ela_spectrum_ragged_host``: one launch sequence
+    for the whole batch (the node's <= 3 face crops, v5_texture_ela.py:83-91). Returns a list of (H_i, W_i) uint8 arrays."""
+    from ._abi import GrayDesc
+
+    arrs = [np.asarray(g, dtype=np.uint8) for g in grays]
+    for a in arrs:
+        if a.ndim != 2 or a.shape[0] == 0 or a.shape[1] == 0:
+            raise ValueError("grays must be non-empty (H, W) arrays")
+    arrs = [a if a.strides[1] == 1 and a.strides[0] > 0 else np.ascontiguousarray(a) for a in arrs]
+    outs = [np.empty(a.shape, np.uint8) for a in arrs]
+    n = len(arrs)
+    if n:
+        descs = (GrayDesc * n)()
+        for i, a in enumerate(arrs):
+            descs[i].gray = a.ctypes.data
+            descs[i].height, descs[i].width = a.shape
+            descs[i].row_stride_bytes = a.strides[0]
+            descs[i].out = outs[i].ctypes.data
+        get_handle(device).spectrum_ragged_host(descs, n)
+    return outs

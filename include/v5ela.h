@@ -181,6 +181,31 @@ V5ELA_API int v5ela_spectrum_host(v5ela_handle *h, const uint8_t *gray_host, int
                         uint8_t *out_host);
 
 /*
+ * The same spectrum for a RAGGED batch — images of different sizes in ONE launch sequence: the node's face crops (v5…:83-91),
+ * or any number of crops of mixed sizes. Output i is byte-identical to what v5ela_spectrum writes for image i alone: every
+ * image takes the path the uniform call would take (the shared-memory FFT when both sides have only 2, 3 and 5 as prime
+ * factors, otherwise the exact-size DFT; V5ELA_FFT=0 forces the DFT for all), with the same float64 arithmetic.
+ *   frames_host : HOST array of n descriptors whose pointers are DEVICE pointers; `out` is height * width bytes, tightly packed.
+ * A null array, n < 0, or a descriptor with a null pointer, a non-positive size, a side over 65536 or a row stride smaller
+ * than the width is refused with V5ELA_ERR_INVALID before anything is launched; v5ela_last_error names the frame.
+ * The call plans everything on the host (twiddle tables of the distinct sides, chunks under the same workspace cap as
+ * v5ela_spectrum, the CTAs of every launch), uploads the plan through the handle's staging buffer (waiting first, on the host,
+ * for the previous ragged call's table upload, as v5ela_analyze_ragged does) and is otherwise asynchronous on `cuda_stream`.
+ * Launches: one twiddle kernel per call; per chunk two FFT kernels if an image there takes the FFT, two DFT kernels if one
+ * takes the DFT, and the image kernel. The twiddle tables v5ela_spectrum caches are left as they are.
+ */
+typedef struct v5ela_gray_desc {
+    const uint8_t *gray;        /* uint8 HW, one channel */
+    int32_t height, width;
+    int64_t row_stride_bytes;   /* >= width */
+    uint8_t *out;               /* height * width uint8, tightly packed */
+} v5ela_gray_desc;
+V5ELA_API int v5ela_spectrum_ragged(v5ela_handle *h, const v5ela_gray_desc *frames_host, int n, void *cuda_stream);
+/* The same with HOST pointers in the descriptors: one upload per image into one packed device arena, one launch sequence, one
+ * download per image; synchronises before returning. */
+V5ELA_API int v5ela_spectrum_ragged_host(v5ela_handle *h, const v5ela_gray_desc *frames_host, int n);
+
+/*
  * ---- Codec rows (SURVEY.md §8f-2, §8f-3): the JPEG files on either side of the ELA arithmetic, on the GPU ----------------
  *
  * Encoder: what the reference writes with PIL / OpenCV — `original.save(tmp,'JPEG',quality=90)` (v5_texture_ela.py:66-67),
