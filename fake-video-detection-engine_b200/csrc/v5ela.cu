@@ -160,12 +160,29 @@ static int launch_fused(v5ela_handle *h, const v5plan::KParams &p, int inst, lon
                                                        prof ? static_cast<cudaEvent_t>(h->prof_events[h->prof_used]) : nullptr,
                                                        prof ? static_cast<cudaEvent_t>(h->prof_events[h->prof_used + 1]) : nullptr);
     if (rc != 0) return fail(h, V5ELA_ERR_CUDA, "fused kernel launch: %s", cudaGetErrorString((cudaError_t)rc));
-    h->last_inst = inst == v5plan::INST_RAGGED ? V5ELA_INST_GENERAL : inst;
+    if (inst != v5plan::INST_SWEEP) h->last_inst = inst == v5plan::INST_RAGGED ? V5ELA_INST_GENERAL : inst;
     if (prof) h->prof_used += 2;
     v5::ela_finalize_kernel<<<p.n, 96, 0, st>>>(p.records, p.n);
     V5_CUDA(h, cudaGetLastError());
     h->launches += 2;
     return V5ELA_OK;
+}
+
+// The handle's table staging buffer (h_table) and its device copy (d_table), both at least `need` bytes, ready to be refilled: waits,
+// on the host, until the previous call's upload out of h_table has completed.
+static int staging_table(v5ela_handle *h, size_t need)
+{
+    int rc;
+    if (h->h_table.capacity() < need || h->d_table.capacity() < need) {   // the staging buffer and its device copy grow together
+        if (h->ev_table) cudaEventSynchronize(h->ev_table);
+        h->h_table.reset();
+        h->d_table.reset();
+        const size_t cap = need < 4096 ? 4096 : need * 2;
+        if ((rc = h->h_table.ensure(h, need, cap)) || (rc = h->d_table.ensure(h, cap))) return rc;
+    }
+    V5_CUDA(h, h->ev_table.create());
+    V5_CUDA(h, cudaEventSynchronize(h->ev_table));
+    return 0;
 }
 
 extern "C" {
@@ -298,15 +315,7 @@ int v5ela_analyze_ragged(v5ela_handle *h, const v5ela_frame_desc *frames_host, i
     int rc;
     if ((rc = h->d_ticket.ensure(h, sizeof(unsigned int)))) return rc;
     const size_t desc_bytes = (sizeof(v5plan::FrameDesc) * (size_t)n + 15) / 16 * 16, need = desc_bytes + sizeof(v5::EnhDesc) * (size_t)n;
-    if (h->h_table.capacity() < need || h->d_table.capacity() < need) {   // the staging buffer and its device copy grow together
-        if (h->ev_table) cudaEventSynchronize(h->ev_table);
-        h->h_table.reset();
-        h->d_table.reset();
-        const size_t cap = need < 4096 ? 4096 : need * 2;
-        if ((rc = h->h_table.ensure(h, need, cap)) || (rc = h->d_table.ensure(h, cap))) return rc;
-    }
-    V5_CUDA(h, h->ev_table.create());
-    V5_CUDA(h, cudaEventSynchronize(h->ev_table));              // the previous call's upload has left the staging buffer
+    if ((rc = staging_table(h, need))) return rc;
     long long total = 0;
     rc = v5plan::plan_ragged(reinterpret_cast<v5plan::FrameDesc *>(static_cast<uint8_t *>(h->h_table)), frames_host, n, h->seg_rows,
                              2 * h->sm_count * h->ctas_per_sm, &total);
@@ -388,6 +397,91 @@ try {
         if (f.residual) V5_CUDA(h, cudaMemcpyAsync(f.residual, h->d_in + off_res[i], bytes, cudaMemcpyDeviceToHost, st));
         if (f.enhanced) V5_CUDA(h, cudaMemcpyAsync(f.enhanced, h->d_in + off_enh[i], bytes, cudaMemcpyDeviceToHost, st));
     }
+    V5_CUDA(h, cudaStreamSynchronize(st));
+    return V5ELA_OK;
+} V5_CATCH(h)
+
+// The sweep's refusal, in v5ela_last_error: the frame or the quality index it names.
+static int sweep_refused(v5ela_handle *h, const char *fn, const v5plan::SweepPlan &P)
+{
+    if (P.bad_frame >= 0) snprintf(h->err, sizeof(h->err), "%s: frame %d: %s", fn, P.bad_frame, P.error);
+    else if (P.bad_quality >= 0) snprintf(h->err, sizeof(h->err), "%s: quality %d: %s", fn, P.bad_quality, P.error);
+    else snprintf(h->err, sizeof(h->err), "%s: %s", fn, P.error);
+    return P.status;
+}
+
+int v5ela_analyze_sweep(v5ela_handle *h, const v5ela_frame_desc *frames_host, int n, const int *qualities_host, int nq, void *d_records,
+                        uint32_t *d_ghost, void *cuda_stream)
+try {
+    if (!h) return V5ELA_ERR_INVALID;
+    if (n == 0) return V5ELA_OK;
+    if (!d_records) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_sweep: null record array%s");
+    v5plan::SweepPlan P;
+    v5plan::plan_sweep(P, frames_host, n, qualities_host, nq, d_ghost, h->seg_rows, 2 * h->sm_count * h->ctas_per_sm);
+    if (P.status) return sweep_refused(h, "v5ela_analyze_sweep", P);
+    DeviceGuard guard(h->device);
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    ScratchOrder order(h, st);                                  // ticket counter and tables are handle-owned
+    int rc;
+    if ((rc = h->d_ticket.ensure(h, sizeof(unsigned int)))) return rc;
+    if ((rc = staging_table(h, P.table_bytes))) return rc;
+    uint8_t *tab = h->h_table;
+    memcpy(tab, P.frames.data(), sizeof(v5plan::FrameDesc) * P.frames.size());
+    memcpy(tab + P.off_entries, P.entries.data(), sizeof(v5plan::SweepEntry) * P.entries.size());
+    memcpy(tab + P.off_quant, P.quant.data(), sizeof(v5plan::QuantTab) * P.quant.size());
+    const size_t records = P.frames.size();
+    V5_CUDA(h, cudaMemcpyAsync(h->d_table, h->h_table, P.table_bytes, cudaMemcpyHostToDevice, st));
+    V5_CUDA(h, cudaEventRecord(h->ev_table, st));
+    V5_CUDA(h, cudaMemsetAsync(h->d_ticket, 0, sizeof(unsigned int), st));
+    V5_CUDA(h, cudaMemsetAsync(d_records, 0, sizeof(v5ela_record) * records, st));
+    v5plan::KParams p;
+    memset(&p, 0, sizeof(p));
+    p.records = static_cast<v5ela_record *>(d_records);
+    p.n = (int)records;
+    p.ticket = h->d_ticket;
+    p.lane_consts = h->d_lane_consts;
+    p.frames = reinterpret_cast<const v5plan::FrameDesc *>(static_cast<uint8_t *>(h->d_table));   // the sweep's tables behind it
+    return launch_fused(h, p, v5plan::INST_SWEEP, P.total, st);
+} V5_CATCH(h)
+
+int v5ela_analyze_sweep_host(v5ela_handle *h, const v5ela_frame_desc *frames_host, int n, const int *qualities_host, int nq,
+                             void *records_host, uint32_t *ghost_host)
+try {
+    if (!h) return V5ELA_ERR_INVALID;
+    if (n == 0) return V5ELA_OK;
+    if (!records_host) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_sweep_host: null record array%s");
+    {   // refuse before anything is copied (the device call plans the same entries again, over the uploaded pixels)
+        v5plan::SweepPlan P;
+        v5plan::plan_sweep(P, frames_host, n, qualities_host, nq, nullptr, h->seg_rows, 2 * h->sm_count * h->ctas_per_sm);
+        if (P.status) return sweep_refused(h, "v5ela_analyze_sweep_host", P);
+    }
+    DeviceGuard guard(h->device);
+    int rc;
+    cudaStream_t st;
+    if ((rc = internal_stream(h, &st))) return rc;
+    ScratchOrder order(h, st);
+    // device arena: per frame its pixels (rows packed), 256-byte aligned; each frame goes up once for all qualities
+    std::vector<v5ela_frame_desc> dev((size_t)n);
+    std::vector<size_t> off((size_t)n);
+    size_t total = 0, maps = 0;
+    for (int i = 0; i < n; i++) {
+        const v5ela_frame_desc &f = frames_host[i];
+        off[(size_t)i] = total;
+        total += ((size_t)f.height * f.width * 3 + 255) / 256 * 256;
+        maps += (size_t)((f.height + 15) / 16) * ((f.width + 15) / 16);
+    }
+    const size_t records = (size_t)n * nq;
+    if ((rc = h->d_in.ensure(h, total)) || (rc = h->d_rec.ensure(h, sizeof(v5ela_record) * records))) return rc;
+    if (ghost_host && (rc = h->d_ghost.ensure(h, sizeof(uint32_t) * maps * nq))) return rc;
+    for (int i = 0; i < n; i++) {
+        const v5ela_frame_desc &f = frames_host[i];
+        V5_CUDA(h, cudaMemcpy2DAsync(h->d_in + off[(size_t)i], (size_t)3 * f.width, f.rgb, (size_t)f.row_stride_bytes, (size_t)3 * f.width,
+                                     (size_t)f.height, cudaMemcpyHostToDevice, st));
+        dev[(size_t)i] = v5ela_frame_desc{h->d_in + off[(size_t)i], f.height, f.width, (int64_t)3 * f.width, nullptr, nullptr};
+    }
+    if ((rc = v5ela_analyze_sweep(h, dev.data(), n, qualities_host, nq, h->d_rec, ghost_host ? (uint32_t *)h->d_ghost : nullptr, st))) return rc;
+    V5_CUDA(h, cudaMemcpyAsync(records_host, h->d_rec, sizeof(v5ela_record) * records, cudaMemcpyDeviceToHost, st));
+    if (ghost_host) V5_CUDA(h, cudaMemcpyAsync(ghost_host, h->d_ghost, sizeof(uint32_t) * maps * nq, cudaMemcpyDeviceToHost, st));
     V5_CUDA(h, cudaStreamSynchronize(st));
     return V5ELA_OK;
 } V5_CATCH(h)
@@ -642,15 +736,7 @@ try {
         (rc = h->d_ms.ensure(h, sizeof(double) * P.ms_max)) || (rc = h->d_minmax.ensure(h, sizeof(unsigned long long) * 2 * (size_t)P.mm_max)))
         return rc;
     const size_t need = P.table_bytes;
-    if (h->h_table.capacity() < need || h->d_table.capacity() < need) {   // the staging buffer and its device copy grow together
-        if (h->ev_table) cudaEventSynchronize(h->ev_table);
-        h->h_table.reset();
-        h->d_table.reset();
-        const size_t cap = need < 4096 ? 4096 : need * 2;
-        if ((rc = h->h_table.ensure(h, need, cap)) || (rc = h->d_table.ensure(h, cap))) return rc;
-    }
-    V5_CUDA(h, h->ev_table.create());
-    V5_CUDA(h, cudaEventSynchronize(h->ev_table));              // the previous call's upload has left the staging buffer
+    if ((rc = staging_table(h, need))) return rc;
     uint8_t *tab = h->h_table;
     memcpy(tab + P.off_sizes, P.sizes.data(), sizeof(v5fft::SpecSize) * P.sizes.size());
     memcpy(tab + P.off_frames, P.frames.data(), sizeof(v5fft::SpecFrame) * P.frames.size());

@@ -78,6 +78,20 @@ struct FrameDesc {
     uint32_t flags;             // bit 0: vec_ok, bit 1: resid_vec_ok
 };
 
+// One entry of a sweep (v5ela_analyze_sweep) beside its FrameDesc: the entry's quantisation tables and its JPEG-ghost map. Read by
+// the sweep kernel only (process_work_item's SWEEP).
+struct SweepEntry {
+    uint32_t *ghost;            // optional: ceil(h/16) x ceil(w/16) per-MCU sums of the squared residual
+    int32_t slot;               // tables sweep_quant(..)[2 * slot] (luma), [2 * slot + 1] (chroma)
+    int32_t pad;
+};
+
+// A sweep's device table (plan_sweep): its n entries' FrameDesc, then their SweepEntry, then two QuantTab per slot. The sweep kernel
+// finds the two tables behind KParams::frames, so that KParams, and with it every other kernel's parameter layout, stays as it is.
+V5_HOSTDEV const SweepEntry *sweep_entries(const FrameDesc *frames, int n) { return reinterpret_cast<const SweepEntry *>(frames + n); }
+V5_HOSTDEV const QuantTab *sweep_quant(const FrameDesc *frames, int n) { return reinterpret_cast<const QuantTab *>(sweep_entries(frames, n) + n); }
+static_assert(sizeof(FrameDesc) % 8 == 0 && sizeof(SweepEntry) % 8 == 0, "sweep table alignment");
+
 struct KParams {
     const uint8_t *rgb;
     int64_t frame_stride;
@@ -129,6 +143,7 @@ struct alignas(8) U2 { uint32_t x, y; };
 V5_DEV uint32_t umulhi32(uint32_t a, uint32_t b) { return __umulhi(a, b); }
 V5_DEV int clamp255(int v) { return __vimin_s32_relu(v, 255); }
 V5_DEV void smem_inc(uint32_t *p) { atomicAdd(p, 1u); }
+V5_DEV void smem_add(uint32_t *p, uint32_t v) { atomicAdd(p, v); }
 V5_DEV uint32_t absdiff4(uint32_t a, uint32_t b) { return __vabsdiffu4(a, b); }
 // PTX prmt (default mode): result byte i = byte sel[4i+2:4i] of {b,a}; selector bit 3 replicates that byte's sign bit.
 V5_DEV uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel)
@@ -141,6 +156,7 @@ V5_DEV uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel)
 inline uint32_t umulhi32(uint32_t a, uint32_t b) { return (uint32_t)(((uint64_t)a * b) >> 32); }
 inline int clamp255(int v) { return v < 0 ? 0 : (v > 255 ? 255 : v); }
 inline void smem_inc(uint32_t *p) { *p += 1u; }
+inline void smem_add(uint32_t *p, uint32_t v) { *p += v; }
 inline uint32_t absdiff4(uint32_t a, uint32_t b)
 {
     uint32_t r = 0;
@@ -204,6 +220,13 @@ V5_DEV int dp4a_us(uint32_t a, uint32_t b, int c)
     asm("dp4a.u32.s32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
     return d;
 }
+// dp4a_uu(a, b, c) = c + sum_i u8(a.byte[i]) * u8(b.byte[i])
+V5_DEV uint32_t dp4a_uu(uint32_t a, uint32_t b, uint32_t c)
+{
+    uint32_t d;
+    asm("dp4a.u32.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
+    return d;
+}
 V5_DEV int dp2a_lo_su(uint32_t a, uint32_t b, int c)
 {
     int d;
@@ -238,6 +261,11 @@ V5_DEV void hist_add(uint32_t *hist_c, uint32_t word, int k)
 inline int dp4a_us(uint32_t a, uint32_t b, int c)
 {
     for (int i = 0; i < 4; i++) c += (int)((a >> (8 * i)) & 0xff) * (int)(int8_t)((b >> (8 * i)) & 0xff);
+    return c;
+}
+inline uint32_t dp4a_uu(uint32_t a, uint32_t b, uint32_t c)
+{
+    for (int i = 0; i < 4; i++) c += ((a >> (8 * i)) & 0xff) * ((b >> (8 * i)) & 0xff);
     return c;
 }
 inline int dp2a_su_(uint32_t a, uint32_t b, int c, int hi, bool sgn)
@@ -392,7 +420,10 @@ struct alignas(16) Smem {
     uint8_t cenc[2][8][C_PITCH];        // downsampled Cb/Cr of the current band (input of the block stage)
     uint8_t cdec[2][16][C_PITCH];       // decoded Cb/Cr; band r chroma line j at [8*(r&1) + j]
     uint32_t hist[3][256];
-    uint32_t tex_hist[256];             // histogram of min(|Laplacian|, 255); only the TEXHIST instantiation touches it
+    union {
+        uint32_t tex_hist[256];         // histogram of min(|Laplacian|, 255); only the TEXHIST instantiation touches it
+        uint32_t ghost[2][TW_MAX];      // sweep kernel: the JPEG-ghost cells of the strip's MCUs, MCU row R in ghost[R & 1]
+    };
     unsigned long long tex_sumabs, tex_sumsq;
     unsigned long long full_bar[2];     // mbarriers: "band has landed in rgb[b]"
     unsigned long long done_bar;        // mbarrier (count NT): "every thread has finished the residual stage of the band before"
@@ -401,6 +432,7 @@ struct alignas(16) Smem {
     uint32_t next_work;                 // ticket drawn by thread 0 for the CTA's next work item
     uint32_t pad_[2];
 };
+static_assert(2 * TW_MAX <= 256, "the sweep kernel's ghost cells live in tex_hist's shared memory");
 
 // Per work item geometry (uniform across the CTA).
 struct Geo {
@@ -1003,8 +1035,10 @@ V5_DEV void upsample8_fast(const uint8_t *lc, const uint8_t *ln, bool left_edge,
 // TEXHIST: the optional tex_hist[256] output of the record table (SURVEY.md §8a) is wanted — one more shared-memory
 // increment per pixel; an instantiation of its own so that calls without it pay nothing.
 // Second half of a unit: given the upsampled chroma (minus 128) of its 8 pixels, reconstruct, residual, histogram, Laplacian.
-template <bool FAST, bool TEXHIST>
-V5_DEV void residual_row(Smem &S, const KParams &p, const Geo &g, ThreadAcc &acc, int r, int l, int ox, const int *cb, const int *cr)
+// SWEEP (the sweep kernel) with `ghost` set: the unit's sum of squared residuals goes into its MCU's ghost cell as well.
+template <bool FAST, bool TEXHIST, bool SWEEP = false>
+V5_DEV void residual_row(Smem &S, const KParams &p, const Geo &g, ThreadAcc &acc, int r, int l, int ox, const int *cb, const int *cr,
+                         bool ghost = false)
 {
     const int y = 16 * r + l;                                   // global pixel row
     const int gx0 = 16 * g.m0 + 8 * ox;                         // global pixel column of this unit
@@ -1089,6 +1123,12 @@ V5_DEV void residual_row(Smem &S, const KParams &p, const Geo &g, ThreadAcc &acc
     }
 #pragma unroll
     for (int b = 0; b < 24; b++) hist_add(S.hist[b % 3], dw[b >> 2], b & 3);
+    if (SWEEP && ghost) {                                       // outside pixels are zero by now
+        uint32_t sq = 0;
+#pragma unroll
+        for (int i = 0; i < 6; i++) sq = dp4a_uu(dw[i], dw[i], sq);
+        smem_add(&S.ghost[(y >> 4) & 1][ox >> 1], sq);
+    }
 
     // ---- texture: Laplacian of the original luma, BORDER_REFLECT_101 (§8a)
     int lu = l - 1, ld = l + 1;
@@ -1151,8 +1191,8 @@ V5_DEV void residual_row(Smem &S, const KParams &p, const Geo &g, ThreadAcc &acc
 }
 
 // 8 pixels of one output row: ox = 8-pixel column index inside the strip, l = band-relative line in [-1, 14].
-template <bool FAST, bool TEXHIST>
-V5_DEV void residual_unit(Smem &S, const KParams &p, const Geo &g, ThreadAcc &acc, int r, int l, int ox)
+template <bool FAST, bool TEXHIST, bool SWEEP = false>
+V5_DEV void residual_unit(Smem &S, const KParams &p, const Geo &g, ThreadAcc &acc, int r, int l, int ox, bool ghost = false)
 {
     const int y = 16 * r + l;                                   // global pixel row
     const int gx0 = 16 * g.m0 + 8 * ox;                         // global pixel column of this unit
@@ -1175,7 +1215,7 @@ V5_DEV void residual_unit(Smem &S, const KParams &p, const Geo &g, ThreadAcc &ac
         upsample8(&S.cdec[1][lcur][ccol], &S.cdec[1][lnb][ccol], gcx0, wc1, fancy, cr);
     }
 
-    residual_row<FAST, TEXHIST>(S, p, g, acc, r, l, ox, cb, cr);
+    residual_row<FAST, TEXHIST, SWEEP>(S, p, g, acc, r, l, ox, cb, cr, ghost);
 }
 
 // Two rows per unit (width-multiple-of-16 instantiation, -DV5_PAIR_ROWS=1). Band iteration r finishes rows 16r-1 .. 16r+14:
@@ -1247,8 +1287,8 @@ V5_DEV void stage_residual_pairs(int tid, Smem &S, const KParams &p, const Geo &
 }
 
 // Iteration r finishes pixel rows 16r-1 .. 16r+14 (clipped to the segment and the image).
-template <bool FAST, bool TEXHIST>
-V5_DEV void stage_residual(int tid, Smem &S, const KParams &p, const Geo &g, ThreadAcc &acc, int r)
+template <bool FAST, bool TEXHIST, bool SWEEP = false>
+V5_DEV void stage_residual(int tid, Smem &S, const KParams &p, const Geo &g, ThreadAcc &acc, int r, bool ghost = false)
 {
     const int n8 = 2 * (g.m1 - g.m0);                           // 8-pixel units per line (<= 60)
     const uint32_t inv = 65536u / (uint32_t)n8 + 1u;            // exact u / n8 for u < 16 * 60
@@ -1257,7 +1297,7 @@ V5_DEV void stage_residual(int tid, Smem &S, const KParams &p, const Geo &g, Thr
         const int wl = (int)(((uint32_t)u * inv) >> 16), ox = u - wl * n8;
         const int l = wl - 1, y = 16 * r + l;
         if (y < ylo || y >= yhi || (!FAST && 16 * g.m0 + 8 * ox >= g.w)) continue;
-        residual_unit<FAST, TEXHIST>(S, p, g, acc, r, l, ox);
+        residual_unit<FAST, TEXHIST, SWEEP>(S, p, g, acc, r, l, ox, ghost);
     }
 }
 

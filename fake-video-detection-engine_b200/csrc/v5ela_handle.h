@@ -120,8 +120,10 @@ struct v5ela_handle {
     size_t prof_used = 0;
     int host_chunk_frames = 0;             // 0 = auto
     v5host::DeviceBuf<uint8_t> d_in, d_res, d_enh, d_rec;
+    v5host::DeviceBuf<uint32_t> d_ghost;   // v5ela_analyze_sweep_host: the ghost maps
     v5host::DeviceBuf<unsigned int> d_ticket;
-    // ragged batches: the kernel's frame table (+ the enhancement kernel's table behind it), pinned host staging and device copy
+    // ragged batches and sweeps: the kernel's frame table (+ the enhancement kernel's, or the sweep's, tables behind it), pinned host
+    // staging and device copy
     v5host::PinnedBuf h_table;
     v5host::DeviceBuf<uint8_t> d_table;
     v5host::Event ev_table;                // the last upload out of h_table has completed

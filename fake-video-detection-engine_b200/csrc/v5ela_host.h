@@ -3,6 +3,7 @@
 #pragma once
 #include <cstdint>
 #include <cstring>
+#include <vector>
 
 #include "v5ela.h"
 #include "v5ela_device.cuh"
@@ -139,6 +140,14 @@ inline long long total_work_items(const KParams &p)
     return (long long)p.work_split + (long long)(p.n - p.split_frame) * p.n_strips * p.n_segs_b;
 }
 
+// A descriptor of a ragged batch has pixels, a size within 65536 x 65536 and 2^31 - 1 pixels (32-bit histogram counters), and a row
+// stride of at least 3 * width.
+inline bool frame_desc_ok(const v5ela_frame_desc &f)
+{
+    return f.rgb && f.height > 0 && f.width > 0 && f.height <= 65536 && f.width <= 65536 && (int64_t)f.height * f.width <= 0x7fffffffLL &&
+           f.row_stride_bytes >= (int64_t)3 * f.width;
+}
+
 // Ragged batch (v5ela_analyze_ragged): fills tab[0..n) — per frame its geometry, pointers, strips x segments and first work item —
 // and *total, the work items of the launch. fill_params' rule without its tail split: segments_wanted over the strips of the whole
 // batch (4 segments per frame when no CTA count is known), and narrower strips for every frame when the batch as a whole is short of
@@ -149,9 +158,7 @@ inline int plan_ragged(FrameDesc *tab, const v5ela_frame_desc *frames, int n, in
     int64_t columns = 0;
     for (int i = 0; i < n; i++) {
         const v5ela_frame_desc &f = frames[i];
-        if (!f.rgb || f.height <= 0 || f.width <= 0 || f.height > 65536 || f.width > 65536 || (int64_t)f.height * f.width > 0x7fffffffLL ||
-            f.row_stride_bytes < (int64_t)3 * f.width)
-            return -1;
+        if (!frame_desc_ok(f)) return -1;
         FrameDesc &d = tab[i];
         uint8_t *resid = f.residual ? f.residual : f.enhanced;                // an enhanced map alone: the residual is formed in place
         d.rgb = f.rgb;
@@ -186,6 +193,76 @@ inline int plan_ragged(FrameDesc *tab, const v5ela_frame_desc *frames, int n, in
     return 0;
 }
 
+// A sweep (v5ela_analyze_sweep): n frames at nq qualities, expanded quality-major into n * nq entries — entry q * n + i is frame i at
+// qualities[q] and writes record q * n + i — and cut by plan_ragged's rule over the whole expanded list. Beside the frame table, one
+// SweepEntry per entry: its table slot (one per distinct quality, in order of first appearance) and its ghost map, map (q, i) at
+// ghost + q * M + sum_{j<i} m_j with m_j = ceil(h_j/16) * ceil(w_j/16), M = sum_j m_j.
+struct SweepPlan {
+    int status = V5ELA_OK;                      // V5ELA_OK, or why the call is refused ...
+    const char *error = "";
+    int bad_frame = -1, bad_quality = -1;       // ... and the frame or the quality index it is refused for
+    std::vector<FrameDesc> frames;              // n * nq entries
+    std::vector<SweepEntry> entries;
+    std::vector<QuantTab> quant;                // luma, chroma of each slot
+    std::vector<int> slot_quality;
+    long long total = 0;                        // work items of the launch
+    size_t off_entries = 0, off_quant = 0, table_bytes = 0;   // device table: frames | entries | quant (sweep_entries, sweep_quant)
+};
+
+inline void plan_sweep(SweepPlan &P, const v5ela_frame_desc *frames, int n, const int *qualities, int nq, uint32_t *ghost, int seg_rows,
+                       int target_items)
+{
+    auto refuse = [&P](const char *why, int frame, int quality) {
+        P.status = V5ELA_ERR_INVALID;
+        P.error = why;
+        P.bad_frame = frame;
+        P.bad_quality = quality;
+    };
+    if (!frames || !qualities || n < 0) return refuse("null descriptor or quality array, or n < 0", -1, -1);
+    if (nq < 1 || nq > 100) return refuse("nq must be in 1..100", -1, -1);
+    for (int q = 0; q < nq; q++)
+        if (qualities[q] < 1 || qualities[q] > 100) return refuse("quality outside 1..100", -1, q);
+    for (int i = 0; i < n; i++) {
+        if (!frame_desc_ok(frames[i])) return refuse("bad pointer, size or stride", i, -1);
+        if (frames[i].residual || frames[i].enhanced) return refuse("residual and enhanced maps must be NULL in a sweep", i, -1);
+    }
+    const int64_t m = (int64_t)n * nq;
+    if (m > 0x7fffffffLL) return refuse("more than 2^31 - 1 work items", -1, -1);
+    std::vector<v5ela_frame_desc> expanded((size_t)m);
+    for (int q = 0; q < nq; q++)
+        for (int i = 0; i < n; i++) expanded[(size_t)q * n + i] = frames[i];
+    P.frames.resize((size_t)m);
+    if (m > 0 && plan_ragged(P.frames.data(), expanded.data(), (int)m, seg_rows, target_items, &P.total) != 0)
+        return refuse("more than 2^31 - 1 work items", -1, -1);
+    std::vector<int64_t> map_off((size_t)n);
+    int64_t M = 0;
+    for (int i = 0; i < n; i++) {
+        map_off[(size_t)i] = M;
+        M += (int64_t)P.frames[(size_t)i].mh * P.frames[(size_t)i].mw;
+    }
+    int slot_of[101];
+    for (int &s : slot_of) s = -1;
+    P.entries.resize((size_t)m);
+    for (int q = 0; q < nq; q++) {
+        int &slot = slot_of[qualities[q]];
+        if (slot < 0) {
+            slot = (int)P.slot_quality.size();
+            P.slot_quality.push_back(qualities[q]);
+        }
+        for (int i = 0; i < n; i++) {
+            SweepEntry &e = P.entries[(size_t)q * n + i];
+            e.ghost = ghost ? ghost + (int64_t)q * M + map_off[(size_t)i] : nullptr;
+            e.slot = slot;
+            e.pad = 0;
+        }
+    }
+    P.quant.resize(2 * P.slot_quality.size());
+    for (size_t s = 0; s < P.slot_quality.size(); s++) fill_quant(&P.quant[2 * s], P.slot_quality[s]);
+    P.off_entries = sizeof(FrameDesc) * P.frames.size();
+    P.off_quant = P.off_entries + sizeof(SweepEntry) * P.entries.size();
+    P.table_bytes = P.off_quant + sizeof(QuantTab) * P.quant.size();
+}
+
 // Which instantiation of the fused kernel a call takes (v5ela_device.cuh, FAST): widths that are a multiple of the MCU
 // width (1280, 1920, 3840, ...), 16-byte aligned, without a residual map — the statistics-only keyframe batches the
 // benchmark drives.
@@ -201,6 +278,9 @@ inline bool fast_path_ok(const KParams &p)
 // The general instantiation over a frame table (KParams::frames). Internal to the plan: v5ela_last_instantiation reports a ragged
 // launch as V5ELA_INST_GENERAL.
 constexpr int INST_RAGGED = V5ELA_INST_TEXHIST + 1;
+// The sweep kernel (v5ela_analyze_sweep's frame table, with the sweep's tables behind it). Internal to the plan as well, and not
+// reported by v5ela_last_instantiation.
+constexpr int INST_SWEEP = INST_RAGGED + 1;
 
 // The instantiation a launch takes: RAGGED for a frame table, TEXHIST if a texture histogram is wanted, else FAST where
 // fast_path_ok, else GENERAL.

@@ -38,13 +38,38 @@ __global__ void __launch_bounds__(NT, MIN_CTAS) ela_fused_kernel(const __grid_co
     }
 }
 
-// once per device: opt in to the dynamic shared memory the kernel needs
+// A sweep (v5ela_analyze_sweep): the ragged instantiation over its n x nq entries, each with its own quantisation tables and
+// optional JPEG-ghost map. A kernel of its own, so that ela_fused_kernel's instantiations are left exactly as they are.
+__global__ void __launch_bounds__(NT, MIN_CTAS) ela_sweep_kernel(const __grid_constant__ KParams p, int total_work)
+{
+    extern __shared__ __align__(16) uint8_t smem_raw[];
+    Smem &S = *reinterpret_cast<Smem *>(smem_raw);
+    ThreadAcc acc_store[1];
+    acc_store[0].phase = 0;
+    if (threadIdx.x == 0) {
+        mbar_init(reinterpret_cast<uint64_t *>(&S.full_bar[0]), 1);
+        mbar_init(reinterpret_cast<uint64_t *>(&S.full_bar[1]), 1);
+        mbar_init(reinterpret_cast<uint64_t *>(&S.done_bar), NT);
+        mbar_init_fence();
+    }
+    __syncthreads();
+    for (;;) {
+        if (threadIdx.x == 0) S.next_work = atomicAdd(p.ticket, 1u);
+        __syncthreads();
+        const int work = (int)S.next_work;
+        if (work >= total_work) break;
+        process_work_item<false, false, true, true>(S, p, work, acc_store);
+    }
+}
+
+// once per device: opt in to the dynamic shared memory the kernels need
 cudaError_t prepare()
 {
     cudaError_t e = cudaFuncSetAttribute(ela_fused_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ela_fused_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ela_fused_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ela_fused_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ela_sweep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
     return e;
 }
 
@@ -55,7 +80,8 @@ int launch(const KParams &p, int inst, long long total, int max_ctas, cudaStream
 {
     const int grid = total < max_ctas ? (int)total : max_ctas;
     if (ev_start) cudaEventRecord(ev_start, st);
-    if (inst == v5plan::INST_RAGGED) ela_fused_kernel<false, false, true><<<grid, NT, sizeof(Smem), st>>>(p, (int)total);
+    if (inst == v5plan::INST_SWEEP) ela_sweep_kernel<<<grid, NT, sizeof(Smem), st>>>(p, (int)total);
+    else if (inst == v5plan::INST_RAGGED) ela_fused_kernel<false, false, true><<<grid, NT, sizeof(Smem), st>>>(p, (int)total);
     else if (inst == V5ELA_INST_TEXHIST) ela_fused_kernel<false, true><<<grid, NT, sizeof(Smem), st>>>(p, (int)total);
     else if (inst == V5ELA_INST_FAST) ela_fused_kernel<true, false><<<grid, NT, sizeof(Smem), st>>>(p, (int)total);
     else ela_fused_kernel<false, false><<<grid, NT, sizeof(Smem), st>>>(p, (int)total);

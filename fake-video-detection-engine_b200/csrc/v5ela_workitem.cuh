@@ -134,21 +134,39 @@ inline void flush_global(int tid, Smem &S, v5ela_record *rec, uint32_t *tex_hist
 }
 #endif
 
+// The ghost cells of MCU row R of the work item's strip -> the entry's map (plain stores: each MCU belongs to one work item), and
+// zeroed for MCU row R + 2.
+V5_DEV void flush_ghost_row(int tid, Smem &S, const Geo &g, uint32_t *ghost, int R)
+{
+    for (int c = tid; c < g.m1 - g.m0; c += NT) {
+        ghost[(int64_t)R * g.mw + g.m0 + c] = S.ghost[R & 1][c];
+        S.ghost[R & 1][c] = 0;
+    }
+}
+
 // RAGGED: every frame has its own size and pointers (KParams::frames); only with the general instantiation.
-template <bool FAST, bool TEXHIST, bool RAGGED = false>
+// SWEEP (with RAGGED; the sweep kernel): every entry also has its own quantisation tables and, optionally, a JPEG-ghost map
+// (sweep_entries). The residual stage of iteration r completes MCU row r - 1, the loop's end the segment's last one.
+template <bool FAST, bool TEXHIST, bool RAGGED = false, bool SWEEP = false>
 V5_DEV void process_work_item(Smem &S, const KParams &p, int work, ThreadAcc *acc_store)
 {
     static_assert(!RAGGED || (!FAST && !TEXHIST), "ragged batches take the general instantiation");
+    static_assert(!SWEEP || RAGGED, "a sweep is a ragged batch");
     Geo g;
     int frame;
     make_geo<RAGGED>(p, work, g, frame);
+    const SweepEntry *const entry = SWEEP ? sweep_entries(p.frames, p.n) + frame : nullptr;
+    const QuantTab *const sweep_q = SWEEP ? sweep_quant(p.frames, p.n) + 2 * entry->slot : nullptr;
+    uint32_t *const ghost = SWEEP ? entry->ghost : nullptr;
 
     V5_FOR_THREADS({
         for (int i = tid; i < 3 * 256; i += NT) (&S.hist[0][0])[i] = 0;
         if (TEXHIST)
             for (int i = tid; i < 256; i += NT) S.tex_hist[i] = 0;
+        if (SWEEP)
+            for (int i = tid; i < 2 * TW_MAX; i += NT) (&S.ghost[0][0])[i] = 0;
         for (int i = tid; i < 2 * 64; i += NT) {
-            const QuantTab &q = p.q[i >> 6];
+            const QuantTab &q = SWEEP ? sweep_q[i >> 6] : p.q[i >> 6];
             const int k = i & 63;
 #if V5_MMA_BLOCKS
             S.qtab[i >> 6][mma::qswz_pos(k)] = mma::qswz_entry(q.recip[k], q.bias[k], q.t[k], q.unbias[k]);
@@ -286,12 +304,15 @@ V5_DEV void process_work_item(Smem &S, const KParams &p, int work, ThreadAcc *ac
                 })
                 pending = true;
             } else {
-                V5_FOR_THREADS(if (PAIRS) stage_residual_pairs<TEXHIST>(tid, S, p, g, acc, r); else stage_residual<FAST, TEXHIST>(tid, S, p, g, acc, r))
+                V5_FOR_THREADS(if (PAIRS) stage_residual_pairs<TEXHIST>(tid, S, p, g, acc, r); else stage_residual<FAST, TEXHIST, SWEEP>(tid, S, p, g, acc, r, ghost != nullptr))
+            }
+            if (SWEEP && ghost && r - 1 >= g.r0 && r < g.r1) {
+                V5_FOR_THREADS(flush_ghost_row(tid, S, g, ghost, r - 1))
             }
         }
     }
 
-    V5_FOR_THREADS(flush_partials(tid, S, acc))
+    V5_FOR_THREADS(flush_partials(tid, S, acc); if (SWEEP && ghost) flush_ghost_row(tid, S, g, ghost, g.r1 - 1))
     V5_FOR_THREADS(flush_global(tid, S, p.records + frame, TEXHIST ? p.tex_hist + (int64_t)frame * 256 : nullptr))
 }
 

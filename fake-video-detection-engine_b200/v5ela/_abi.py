@@ -17,7 +17,7 @@ EXPORTS = (
     "v5ela_profile_read", "v5ela_spectrum", "v5ela_spectrum_host", "v5ela_jpeg_bound", "v5ela_jpeg_encode",
     "v5ela_jpeg_encode_host", "v5ela_jpeg_info", "v5ela_jpeg_info_batch", "v5ela_jpeg_decode", "v5ela_jpeg_decode_host",
     "v5ela_last_instantiation", "v5ela_set_block_stage", "v5ela_get_block_stage", "v5ela_analyze_ragged", "v5ela_analyze_ragged_host",
-    "v5ela_spectrum_ragged", "v5ela_spectrum_ragged_host",
+    "v5ela_spectrum_ragged", "v5ela_spectrum_ragged_host", "v5ela_analyze_sweep", "v5ela_analyze_sweep_host",
 )
 BLOCK_STAGES = {"smem": 0, "mma": 1}
 INSTANTIATIONS = {0: "general", 1: "fast", 2: "texhist", -1: None}
@@ -74,6 +74,8 @@ def load() -> ctypes.CDLL:
     lib.v5ela_analyze_ex.argtypes = [vp, vp, i32, i32, i32, i64, i64, vp, vp, vp, vp]
     lib.v5ela_analyze_ragged.argtypes = [vp, ctypes.POINTER(FrameDesc), i32, vp, vp]
     lib.v5ela_analyze_ragged_host.argtypes = [vp, ctypes.POINTER(FrameDesc), i32, vp]
+    lib.v5ela_analyze_sweep.argtypes = [vp, ctypes.POINTER(FrameDesc), i32, ctypes.POINTER(i32), i32, vp, vp, vp]
+    lib.v5ela_analyze_sweep_host.argtypes = [vp, ctypes.POINTER(FrameDesc), i32, ctypes.POINTER(i32), i32, vp, vp]
     lib.v5ela_enhance.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp]
     lib.v5ela_reduce_records.argtypes = [vp, vp, i32, i32, vp, vp]
     lib.v5ela_analyze_host.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp]
@@ -157,6 +159,17 @@ class Handle:
     def analyze_ragged_host(self, descs, n: int, records_host: int):
         """descs: ctypes array of FrameDesc holding HOST pointers; synchronous."""
         self._check(self._lib.v5ela_analyze_ragged_host(self._h, descs, n, records_host))
+
+    def analyze_sweep(self, descs, n: int, qualities, d_records: int, d_ghost: int | None, stream: int | None):
+        """descs: ctypes array of FrameDesc holding DEVICE pointers, analysed at every quality of `qualities` in one launch sequence
+        (records quality-major); the handle's quality is left as it is."""
+        qs = (ctypes.c_int * len(qualities))(*[int(q) for q in qualities])
+        self._check(self._lib.v5ela_analyze_sweep(self._h, descs, n, qs, len(qualities), d_records, d_ghost or None, stream or None))
+
+    def analyze_sweep_host(self, descs, n: int, qualities, records_host: int, ghost_host: int | None):
+        """descs: ctypes array of FrameDesc holding HOST pointers; synchronous."""
+        qs = (ctypes.c_int * len(qualities))(*[int(q) for q in qualities])
+        self._check(self._lib.v5ela_analyze_sweep_host(self._h, descs, n, qs, len(qualities), records_host, ghost_host or None))
 
     def enhance(self, d_residual: int, d_records: int, n: int, h: int, w: int, d_enhanced: int, stream: int | None):
         self._check(self._lib.v5ela_enhance(self._h, d_residual, d_records, n, h, w, d_enhanced, stream or None))

@@ -128,6 +128,70 @@ def analyze_ragged(frames, quality: int = 90, want_residual: bool = False, want_
     return out
 
 
+def analyze_sweep(frames, qualities, want_ghost: bool = False, handle=None):
+    """Every frame at every JPEG quality of ``qualities`` in one launch sequence (v5ela_analyze_sweep), with, when asked, the JPEG-ghost
+    maps (Farid 2009): per MCU the sum over its pixels and channels of the squared residual. A region saved at quality q0 before has its
+    smallest residual at q0; a pasted region with another compression history has it elsewhere.
+
+    frames    : torch.uint8 CUDA tensor (N, H, W, 3), or a sequence of (H_i, W_i, 3) tensors on one device; pixels dense (stride 3 / 1),
+                any row / frame stride, as ``analyze_ragged`` takes them.
+    qualities : 1..100 JPEG qualities, 1 to 100 of them (duplicates allowed); the handle's own quality is left as it is.
+    Returns ``records`` uint8 (nq, N, 3144), record [q, i] byte-identical to ``analyze_ragged`` of frame i at qualities[q]; with
+    ``want_ghost`` also ``ghost``: for a tensor, int32 (nq, N, ceil(H/16), ceil(W/16)); for a list, nq lists of per-frame
+    (ceil(H_i/16), ceil(W_i/16)) int32 views into one arena. Asynchronous on torch's current stream.
+    """
+    import torch
+
+    qualities = [int(q) for q in qualities]
+    nq = len(qualities)
+    uniform = isinstance(frames, torch.Tensor)
+    if uniform:
+        if frames.dtype != torch.uint8 or frames.dim() != 4 or frames.shape[-1] != 3 or not frames.is_cuda:
+            raise ValueError("frames must be a torch.uint8 CUDA tensor of shape (N, H, W, 3)")
+        views = [frames[i] for i in range(frames.shape[0])]
+        dev = frames.device
+    else:
+        views = list(frames)
+        dev = views[0].device if views else torch.device("cuda", torch.cuda.current_device())
+    n = len(views)
+    for k, f in enumerate(views):
+        if not isinstance(f, torch.Tensor) or f.dtype != torch.uint8 or not f.is_cuda or f.dim() != 3 or f.shape[-1] != 3:
+            raise ValueError("frames must be torch.uint8 CUDA tensors of shape (H, W, 3)")
+        if f.device != dev:
+            raise ValueError("all frames must live on one device")
+        if f.shape[0] == 0 or f.shape[1] == 0:
+            raise ValueError("empty frame in a sweep")
+        if f.stride(2) != 1 or f.stride(1) != 3:
+            views[k] = f.contiguous()
+    hd = handle or get_handle(dev.index if dev.index is not None else torch.cuda.current_device())
+    records = torch.empty((nq, n, RECORD_BYTES), dtype=torch.uint8, device=dev)
+    out = {"records": records}
+    ghost = None
+    if want_ghost:
+        cells = [((f.shape[0] + 15) // 16, (f.shape[1] + 15) // 16) for f in views]
+        if uniform:
+            mh, mw = cells[0] if n else ((frames.shape[1] + 15) // 16, (frames.shape[2] + 15) // 16)
+            ghost = torch.empty((nq, n, mh, mw), dtype=torch.int32, device=dev)
+            out["ghost"] = ghost
+        else:
+            offs = [0]
+            for mh, mw in cells:
+                offs.append(offs[-1] + mh * mw)
+            ghost = torch.empty(nq * offs[-1], dtype=torch.int32, device=dev)
+            out["ghost"] = [[ghost[q * offs[-1] + offs[i]:q * offs[-1] + offs[i + 1]].view(*cells[i]) for i in range(n)] for q in range(nq)]
+    if n == 0:
+        return out
+    descs = (_abi.FrameDesc * n)()
+    for i, f in enumerate(views):
+        descs[i].rgb = f.data_ptr()
+        descs[i].height, descs[i].width = int(f.shape[0]), int(f.shape[1])
+        descs[i].row_stride_bytes = int(f.stride(0))
+    hd.analyze_sweep(descs, n, qualities, records.data_ptr(), ghost.data_ptr() if ghost is not None else None,
+                     torch.cuda.current_stream(dev).cuda_stream)
+    out["_keepalive"] = views                                   # contiguous copies (if any) must outlive the asynchronous launch
+    return out
+
+
 def reduce_records(records, group: int, handle=None):
     """Per-video aggregation on the device: (N, 3144) -> (N // group, 3144)."""
     import torch

@@ -62,6 +62,43 @@ def analyze_ragged_host(frames, quality: int = 90, want_residual: bool = False, 
     return recs, residual, enhanced
 
 
+def analyze_sweep_host(frames, qualities, want_ghost: bool = False, device: int = 0):
+    """Every frame at every JPEG quality of ``qualities`` through ``v5ela_analyze_sweep_host``: each frame uploaded once, one launch
+    sequence, one download. frames: (N, H, W, 3) uint8 array or a sequence of (H_i, W_i, 3) uint8 arrays. Returns (records (nq, N)
+    structured, ghost | None): ghost as ``v5ela.analyze_sweep`` gives it — (nq, N, ceil(H/16), ceil(W/16)) uint32 for an array, nq
+    lists of per-frame maps (views into one array) for a sequence."""
+    from ._abi import FrameDesc
+
+    qualities = [int(q) for q in qualities]
+    nq = len(qualities)
+    uniform = isinstance(frames, np.ndarray) and frames.ndim == 4
+    arrs = [np.asarray(f, dtype=np.uint8) for f in frames]
+    for a in arrs:
+        if a.ndim != 3 or a.shape[-1] != 3 or a.shape[0] == 0 or a.shape[1] == 0:
+            raise ValueError("frames must be non-empty (H, W, 3) arrays")
+    arrs = [a if a.strides[2] == 1 and a.strides[1] == 3 and a.strides[0] > 0 else np.ascontiguousarray(a) for a in arrs]
+    n = len(arrs)
+    recs = np.zeros((nq, n), dtype=RECORD_DTYPE)
+    cells = [((a.shape[0] + 15) // 16, (a.shape[1] + 15) // 16) for a in arrs]
+    offs = [0]
+    for mh, mw in cells:
+        offs.append(offs[-1] + mh * mw)
+    flat = np.zeros(nq * offs[-1], np.uint32) if want_ghost else None
+    if n:
+        descs = (FrameDesc * n)()
+        for i, a in enumerate(arrs):
+            descs[i].rgb = a.ctypes.data
+            descs[i].height, descs[i].width = a.shape[0], a.shape[1]
+            descs[i].row_stride_bytes = a.strides[0]
+        get_handle(device).analyze_sweep_host(descs, n, qualities, recs.ctypes.data, flat.ctypes.data if flat is not None else None)
+    if not want_ghost:
+        return recs, None
+    if uniform:
+        mh, mw = (frames.shape[1] + 15) // 16, (frames.shape[2] + 15) // 16
+        return recs, flat.reshape(nq, n, mh, mw)
+    return recs, [[flat[q * offs[-1] + offs[i]:q * offs[-1] + offs[i + 1]].reshape(cells[i]) for i in range(n)] for q in range(nq)]
+
+
 def spectrum_host(gray: np.ndarray, device: int = 0) -> np.ndarray:
     """FFT log-magnitude spectrum image(s) (v5_texture_ela.py:84-88) of (H, W) or (N, H, W) uint8 host arrays."""
     g = np.ascontiguousarray(gray, dtype=np.uint8)

@@ -38,6 +38,14 @@ def combine(records: np.ndarray) -> np.ndarray:
     return out
 
 
+def ghost_curve(records, pixels) -> np.ndarray:
+    """The JPEG-ghost curve of sweep records (v5ela.analyze_sweep): the mean squared residual sum_c ela_sumsq / (3 * pixels) as
+    float64, one value per record. ``records`` is a structured array of any shape, e.g. (nq, N); ``pixels`` is H*W, or an array that
+    broadcasts against it, e.g. the (N,) pixel counts of the frames. Its minimum over the qualities estimates a frame's earlier
+    JPEG quality."""
+    return records["ela_sumsq"].sum(axis=-1, dtype=np.uint64).astype(np.float64) / (3.0 * np.asarray(pixels, dtype=np.float64))
+
+
 def features(rec, n_pixels: int) -> dict:
     """Float64 features of one record over `n_pixels` pixels (H*W of the frame, or the sum over a video's frames).
 

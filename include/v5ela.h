@@ -139,6 +139,33 @@ V5ELA_API int v5ela_analyze_ragged(v5ela_handle *h, const v5ela_frame_desc *fram
 V5ELA_API int v5ela_analyze_ragged_host(v5ela_handle *h, const v5ela_frame_desc *frames_host, int n, void *records_host);
 
 /*
+ * A quality SWEEP — n frames of any sizes, each analysed at nq JPEG qualities, in ONE launch sequence — and, optionally, the
+ * JPEG-ghost map of every (quality, frame) (Farid, "Exposing Digital Forgeries from JPEG Ghosts", 2009): a region that was saved at
+ * quality q0 before is almost a fixed point of a re-save at q0, so where the residual is smallest over q says what its earlier
+ * quality was; a pasted region with another compression history shows its minimum at another q.
+ *   frames_host   : HOST array of n descriptors whose pointers are DEVICE pointers (as v5ela_analyze_ragged takes them); residual
+ *                   and enhanced must be NULL.
+ *   qualities_host: HOST array of nq qualities, each in 1..100, 1 <= nq <= 100; duplicates are allowed. The handle's own quality
+ *                   (v5ela_set_quality) is neither used nor changed.
+ *   d_records     : n * nq records, overwritten: record [q * n + i] is byte-identical to v5ela_analyze_ragged of frame i alone at
+ *                   quality qualities_host[q] (and to v5ela_analyze of it).
+ *   d_ghost       : optional (may be NULL), uint32: per (quality, frame) one ceil(h/16) x ceil(w/16) map, map (q, i) at element
+ *                   q * M + sum_{j<i} m_j, m_j = ceil(h_j/16) * ceil(w_j/16), M = sum_j m_j; entry (by, bx) = sum over the image
+ *                   pixels of MCU (by, bx) of sum_c residual_c^2 (residual as in v5ela_analyze).
+ * A null array, n < 0, nq outside 1..100, a quality outside 1..100, a descriptor v5ela_analyze_ragged would refuse, a non-NULL
+ * residual or enhanced pointer, or more than 2^31 - 1 work items is refused with V5ELA_ERR_INVALID before anything is launched or
+ * copied; v5ela_last_error names the frame or the quality index. n == 0 returns V5ELA_OK.
+ * Ordering as for v5ela_analyze_ragged (the tables go up through the same staging buffer). Launches: the sweep kernel and the
+ * finalize kernel, whatever n and nq. v5ela_last_instantiation is left as it is.
+ */
+V5ELA_API int v5ela_analyze_sweep(v5ela_handle *h, const v5ela_frame_desc *frames_host, int n, const int *qualities_host, int nq,
+                                  void *d_records, uint32_t *d_ghost, void *cuda_stream);
+/* The same with HOST pointers in the descriptors and HOST records / maps: each frame uploaded once, one launch sequence, one download;
+ * synchronises before returning. */
+V5ELA_API int v5ela_analyze_sweep_host(v5ela_handle *h, const v5ela_frame_desc *frames_host, int n, const int *qualities_host, int nq,
+                                       void *records_host, uint32_t *ghost_host);
+
+/*
  * Brightness enhancement of the residual map: `ImageEnhance.Brightness(diff).enhance(255.0 / max_diff)`
  * (v5_texture_ela.py:74-78) == u8(trunc(f32(x) * f32(scale))) clipped, with max_diff read per frame from the records
  * produced by v5ela_analyze on the same stream (0 -> 1 fix applied). d_enhanced may alias d_residual.
