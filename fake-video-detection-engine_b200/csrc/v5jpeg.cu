@@ -1,7 +1,7 @@
 // v5jpeg.cu — codec rows of libv5ela.so (SURVEY.md §8f-2 decode, §8f-3 encode): C-ABI entry points v5ela_jpeg_*.
 // Kernels: v5jpeg_enc.cuh, v5jpeg_dec.cuh. Host-side header writing / parsing: v5jpeg_common.h. The decoder's launch plan (files
 // parsed once, chunks, staging layout, upload runs, Huffman path; negative output offsets refused): v5jpeg_plan.h, which both
-// decode entry points run through run_plan.
+// decode entry points and both DCT-statistics entry points (v5jpeg_dct.cuh) run through run_plan.
 #include <cuda_runtime.h>
 
 #include <cstdlib>
@@ -16,6 +16,7 @@
 #include "v5jpeg_common.h"
 #include "v5jpeg_enc.cuh"
 #include "v5jpeg_dec.cuh"
+#include "v5jpeg_dct.cuh"
 #include "v5jpeg_plan.h"
 
 using namespace v5host;
@@ -45,6 +46,13 @@ struct v5jpeg_state {
     DeviceBuf<v5j::SubInfo> d_sub_info;
     DeviceBuf<uint8_t> d_dec_rgb, d_dec_gray;
     DeviceBuf<int32_t> d_dec_status;
+    // DCT statistics: per-chunk period tables (dct_lut_kernel -> dct_map_kernel); the host entry point's outputs
+    bool dct_ready = false;
+    DeviceBuf<double> d_dq_lut;
+    DeviceBuf<int32_t> d_dq_period;
+    DeviceBuf<uint32_t> d_dq_hist;
+    DeviceBuf<uint16_t> d_dq_qtab;
+    DeviceBuf<float> d_dq_map;
 };
 
 void v5host::JpegStateDelete::operator()(v5jpeg_state *s) const { delete s; }
@@ -278,6 +286,17 @@ v5j::DecodeCall decode_call(const v5ela_handle *h, const uint8_t *const *files_h
     return c;
 }
 
+// A coefficient-only call: the decode call's files and knobs, no pixel outputs, the DCT statistics instead.
+v5j::DecodeCall dct_call(const v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n, bool want_map,
+                         const int64_t *map_offsets)
+{
+    v5j::DecodeCall c = decode_call(h, files_host, lens, n, nullptr, nullptr, false, false);
+    c.coef_only = true;
+    c.want_map = want_map;
+    c.map_offsets = want_map ? map_offsets : nullptr;
+    return c;
+}
+
 int refused(v5ela_handle *h, const char *entry, const v5j::DecodePlan &P)
 {
     char which[64] = "";
@@ -287,9 +306,17 @@ int refused(v5ela_handle *h, const char *entry, const v5j::DecodePlan &P)
     return fail(h, P.status, "%s", msg);
 }
 
-// Runs plan P of call c on stream st: per chunk, the workspaces, the staging buffer, the upload and the launches.
+// The outputs of a coefficient-only call (v5ela_jpeg_dct_stats): DEVICE pointers, qtab and map optional.
+struct DctOut {
+    uint32_t *hist = nullptr;
+    uint16_t *qtab = nullptr;
+    float *map = nullptr;
+};
+
+// Runs plan P of call c on stream st: per chunk, the workspaces, the staging buffer, the upload and the launches. A
+// coefficient-only call (c.coef_only) stops the decode after dc_kernel and writes the statistics to *dq instead of pixels.
 int run_plan(v5ela_handle *h, v5jpeg_state *s, const v5j::DecodeCall &c, const v5j::DecodePlan &P, uint8_t *d_rgb, uint8_t *d_gray,
-             int32_t *d_status, cudaStream_t st)
+             int32_t *d_status, cudaStream_t st, const DctOut *dq = nullptr)
 {
     int rc;
     if (!s->upload_stream) {
@@ -302,6 +329,10 @@ int run_plan(v5ela_handle *h, v5jpeg_state *s, const v5j::DecodeCall &c, const v
         V5_CUDA(h, cudaFuncSetAttribute(v5j::huffman_sync_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(v5j::HuffSmem)));
         V5_CUDA(h, cudaFuncSetAttribute(v5j::huffman_write_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(v5j::HuffSmem)));
     }
+    if (c.coef_only && !s->dct_ready) {
+        V5_CUDA(h, cudaFuncSetAttribute(v5j::dct_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(uint32_t) * v5j::DQ_HIST)));
+        s->dct_ready = true;
+    }
     for (const v5j::DecChunk &C : P.chunks) {
         const int cn = (int)C.images.size();
         const int b = s->toggle;
@@ -313,7 +344,9 @@ int run_plan(v5ela_handle *h, v5jpeg_state *s, const v5j::DecodeCall &c, const v
         if ((rc = s->d_stage[b].ensure(h, C.stage_bytes))) return rc;
         if ((rc = s->d_streams.ensure(h, C.stream_bytes))) return rc;
         if ((rc = s->d_dcoef.ensure(h, C.coef_blocks * 128))) return rc;
-        if ((rc = s->d_planes.ensure(h, C.plane_bytes))) return rc;
+        if (!c.coef_only && (rc = s->d_planes.ensure(h, C.plane_bytes))) return rc;
+        if (c.want_map && (rc = s->d_dq_lut.ensure(h, sizeof(double) * v5j::DQ_FREQS * v5j::DQ_LUT * (size_t)cn))) return rc;
+        if (c.want_map && (rc = s->d_dq_period.ensure(h, sizeof(int32_t) * v5j::DQ_FREQS * (size_t)cn))) return rc;
         if ((rc = s->d_bits.ensure(h, sizeof(uint32_t) * (size_t)cn))) return rc;
         if ((rc = s->d_status.ensure(h, sizeof(int32_t) * (size_t)cn))) return rc;
         if ((rc = s->d_dc.ensure(h, sizeof(int16_t) * C.coef_blocks))) return rc;
@@ -330,6 +363,7 @@ int run_plan(v5ela_handle *h, v5jpeg_state *s, const v5j::DecodeCall &c, const v
         memcpy(stage_host + C.off_img, C.images.data(), sizeof(v5j::DecImage) * (size_t)cn);
         memcpy(stage_host + C.off_tab, P.tabsets.data(), sizeof(v5j::DecTabSet) * P.tabsets.size());
         for (size_t k = 0; k < P.qsets.size(); k++) memcpy(stage_host + C.off_q + 256 * k, P.qsets[k].data(), 256);
+        if (c.want_map) memcpy(stage_host + C.off_map, C.map_off.data(), sizeof(int64_t) * (size_t)cn);
         V5_CUDA(h, cudaStreamWaitEvent(up, s->consumed[b], 0));
         V5_CUDA(h, cudaMemcpyAsync(d_stage, stage_host, C.host_stage_bytes, cudaMemcpyHostToDevice, up));
         for (const v5j::UploadRun &r : C.runs)
@@ -371,12 +405,28 @@ int run_plan(v5ela_handle *h, v5jpeg_state *s, const v5j::DecodeCall &c, const v
         }
         v5j::dc_kernel<<<cn, 1024, 0, st>>>(d_images, s->d_dc);
         V5_CUDA(h, cudaGetLastError());
-        v5j::idct_kernel<<<dim3((unsigned)((C.max_blocks + 63) / 64), (unsigned)cn), 256, 0, st>>>(
-            d_images, d_q, s->d_dcoef, s->d_dc, s->d_planes);
-        V5_CUDA(h, cudaGetLastError());
-        v5j::colour_kernel<<<dim3((unsigned)((C.max_groups + 255) / 256), (unsigned)cn), 256, 0, st>>>(
-            d_images, s->d_planes, d_rgb, d_gray);
-        V5_CUDA(h, cudaGetLastError());
+        if (c.coef_only) {
+            uint32_t *hist = dq->hist + (size_t)C.file_index[0] * v5j::DQ_HIST;
+            V5_CUDA(h, cudaMemsetAsync(hist, 0, sizeof(uint32_t) * v5j::DQ_HIST * (size_t)cn, st));
+            v5j::dct_hist_kernel<<<dim3((unsigned)((C.max_blocks + v5j::DQ_CHUNK - 1) / v5j::DQ_CHUNK), (unsigned)cn), v5j::DQ_HIST_NT,
+                                   sizeof(uint32_t) * v5j::DQ_HIST, st>>>(d_images, d_q, s->d_dcoef, s->d_dc, hist,
+                                                                          dq->qtab ? dq->qtab + (size_t)C.file_index[0] * 3 * 64 : nullptr);
+            V5_CUDA(h, cudaGetLastError());
+            if (c.want_map) {
+                v5j::dct_lut_kernel<<<cn, v5j::DQ_FREQS * 32, 0, st>>>(hist, s->d_dq_lut, s->d_dq_period);
+                V5_CUDA(h, cudaGetLastError());
+                v5j::dct_map_kernel<<<dim3((unsigned)((C.max_luma_blocks + 255) / 256), (unsigned)cn), 256, 0, st>>>(
+                    d_images, reinterpret_cast<const int64_t *>(d_stage + C.off_map), s->d_dcoef, s->d_dq_lut, s->d_dq_period, dq->map);
+                V5_CUDA(h, cudaGetLastError());
+            }
+        } else {
+            v5j::idct_kernel<<<dim3((unsigned)((C.max_blocks + 63) / 64), (unsigned)cn), 256, 0, st>>>(
+                d_images, d_q, s->d_dcoef, s->d_dc, s->d_planes);
+            V5_CUDA(h, cudaGetLastError());
+            v5j::colour_kernel<<<dim3((unsigned)((C.max_groups + 255) / 256), (unsigned)cn), 256, 0, st>>>(
+                d_images, s->d_planes, d_rgb, d_gray);
+            V5_CUDA(h, cudaGetLastError());
+        }
         if (d_status)                                                      // chunks keep file order: one contiguous range
             V5_CUDA(h, cudaMemcpyAsync(d_status + C.file_index[0], d_st, sizeof(int32_t) * (size_t)cn, cudaMemcpyDeviceToDevice, st));
         V5_CUDA(h, cudaEventRecord(s->consumed[b], st));
@@ -457,5 +507,94 @@ try {
         }
     return V5ELA_OK;
 } V5_CATCH(h)
+
+// ------------------------------------------------------------------------------------------------- DCT statistics
+int v5ela_jpeg_dct_stats(v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n, uint32_t *d_hist,
+                         uint16_t *d_qtab, float *d_map, const int64_t *map_offsets, int32_t *d_status, void *cuda_stream)
+try {
+    if (!h) return V5ELA_ERR_INVALID;
+    if (n == 0) return V5ELA_OK;
+    if (!files_host || !lens || n < 0 || !d_hist) return fail(h, V5ELA_ERR_INVALID, "v5ela_jpeg_dct_stats: bad pointer or count%s");
+    DeviceGuard guard(h->device);
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    ScratchOrder order(h, st);                                  // the codec workspace is handle-owned
+    v5jpeg_state *s;
+    int rc;
+    if ((rc = jpeg_state(h, &s))) return rc;
+    const v5j::DecodeCall c = dct_call(h, files_host, lens, n, d_map != nullptr, map_offsets);
+    v5j::DecodePlan P;
+    v5j::plan_decode(c, P);
+    if (P.status) return refused(h, "v5ela_jpeg_dct_stats", P);
+    DctOut dq;
+    dq.hist = d_hist;
+    dq.qtab = d_qtab;
+    dq.map = d_map;
+    return run_plan(h, s, c, P, nullptr, nullptr, d_status, st, &dq);
+} V5_CATCH(h)
+
+int v5ela_jpeg_dct_stats_host(v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n, uint32_t *hist_host,
+                              uint16_t *qtab_host, float *map_host, const int64_t *map_offsets)
+try {
+    if (!h) return V5ELA_ERR_INVALID;
+    if (n == 0) return V5ELA_OK;
+    if (!files_host || !lens || n < 0 || !hist_host) return fail(h, V5ELA_ERR_INVALID, "v5ela_jpeg_dct_stats_host: bad pointer or count%s");
+    DeviceGuard guard(h->device);
+    v5jpeg_state *s;
+    int rc;
+    if ((rc = jpeg_state(h, &s))) return rc;
+    cudaStream_t st;
+    if ((rc = internal_stream(h, &st))) return rc;
+    const v5j::DecodeCall c = dct_call(h, files_host, lens, n, map_host != nullptr, map_offsets);
+    v5j::DecodePlan P;
+    v5j::plan_decode(c, P);
+    if (P.status) return refused(h, "v5ela_jpeg_dct_stats_host", P);
+    int64_t map_end = 0;                                        // map extent on the device, from the plan's offsets
+    for (const v5j::DecChunk &C : P.chunks)
+        for (size_t k = 0; k < C.map_off.size(); k++) {
+            const int64_t e = C.map_off[k] + (int64_t)((C.images[k].h + 7) / 8) * ((C.images[k].w + 7) / 8);
+            if (e > map_end) map_end = e;
+        }
+    const size_t hist_bytes = sizeof(uint32_t) * v5j::DQ_HIST * (size_t)n, qtab_bytes = sizeof(uint16_t) * 3 * 64 * (size_t)n;
+    if ((rc = s->d_dq_hist.ensure(h, hist_bytes))) return rc;
+    if (qtab_host && (rc = s->d_dq_qtab.ensure(h, qtab_bytes))) return rc;
+    if (map_host && (rc = s->d_dq_map.ensure(h, sizeof(float) * (size_t)map_end))) return rc;
+    if ((rc = s->d_dec_status.ensure(h, sizeof(int32_t) * (size_t)n))) return rc;
+    ScratchOrder order(h, st);                                  // the codec workspace is handle-owned
+    DctOut dq;
+    dq.hist = s->d_dq_hist;
+    dq.qtab = qtab_host ? static_cast<uint16_t *>(s->d_dq_qtab) : nullptr;
+    dq.map = map_host ? static_cast<float *>(s->d_dq_map) : nullptr;
+    if ((rc = run_plan(h, s, c, P, nullptr, nullptr, s->d_dec_status, st, &dq))) return rc;
+    std::vector<int32_t> status((size_t)n, 0);
+    V5_CUDA(h, cudaMemcpyAsync(status.data(), s->d_dec_status, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    V5_CUDA(h, cudaMemcpyAsync(hist_host, s->d_dq_hist, hist_bytes, cudaMemcpyDeviceToHost, st));
+    if (qtab_host) V5_CUDA(h, cudaMemcpyAsync(qtab_host, s->d_dq_qtab, qtab_bytes, cudaMemcpyDeviceToHost, st));
+    if (map_host)                                               // only each file's own map comes back
+        for (const v5j::DecChunk &C : P.chunks)
+            for (size_t k = 0; k < C.map_off.size(); k++) {
+                const size_t cnt = (size_t)((C.images[k].h + 7) / 8) * ((C.images[k].w + 7) / 8);
+                V5_CUDA(h, cudaMemcpyAsync(map_host + C.map_off[k], s->d_dq_map + C.map_off[k], sizeof(float) * cnt,
+                                           cudaMemcpyDeviceToHost, st));
+            }
+    V5_CUDA(h, cudaStreamSynchronize(st));
+    for (int i = 0; i < n; i++)
+        if (status[(size_t)i] != 0) {
+            char which[64];
+            snprintf(which, sizeof(which), " (file %d)", i);
+            return fail(h, V5ELA_ERR_INVALID, "v5ela_jpeg_dct_stats_host: entropy-coded data ends early or is corrupt%s", which);
+        }
+    return V5ELA_OK;
+} V5_CATCH(h)
+
+int v5ela_jpeg_ijg_quality(const uint16_t luma[64], const uint16_t *chroma)
+{
+    if (!luma) return V5ELA_ERR_INVALID;
+    for (int q = 1; q <= 100; q++) {
+        uint16_t ql[64], qc[64];
+        v5plan::quant_tables(q, ql, qc);                        // what v5ela_set_quality derives for the handle
+        if (!memcmp(ql, luma, sizeof(ql)) && (!chroma || !memcmp(qc, chroma, sizeof(qc)))) return q;
+    }
+    return 0;
+}
 
 }  // extern "C"

@@ -47,6 +47,11 @@ struct DecodeCall {
     int huff_parts = 0;        // parts per file of the three-launch path, 1..16; anything else: chosen per chunk
     int threads = 1;           // helper threads (parallel_for)
     size_t chunk_bytes = 0;    // workspace per chunk: streams, coefficients and planes stay under it
+    // Coefficients only (v5ela_jpeg_dct_stats): the decode stops after dc_kernel and the DCT statistics kernels run instead
+    // of the inverse DCT and colour conversion; no sample planes. want_map adds the double-compression map, file i's at
+    // element offset map_offsets[i] (null = packed in file order).
+    bool coef_only = false, want_map = false;
+    const int64_t *map_offsets = nullptr;
 };
 
 // One host-to-device copy of pinned file bytes: `bytes` from `src` to `dev_off` inside the chunk's staging buffer.
@@ -60,8 +65,10 @@ struct UploadRun {
 struct DecChunk {
     std::vector<DecImage> images;              // as uploaded: scan_off is relative to the staging buffer
     std::vector<int> file_index;               // the file of each image: consecutive files, in file order
-    // staging layout: descriptors (off_img) | table sets | quantisation tables | scan segments
-    size_t off_img = 0, off_tab = 0, off_q = 0, off_scan = 0;
+    std::vector<int64_t> map_off;              // coefficient-only calls with a map: where each image's map starts (elements)
+    // staging layout: descriptors (off_img) | table sets | quantisation tables | map offsets (coefficient-only calls with a
+    // map, one int64 per image) | scan segments
+    size_t off_img = 0, off_tab = 0, off_q = 0, off_map = 0, off_scan = 0;
     size_t stage_bytes = 0;                    // the device staging buffer
     size_t host_stage_bytes = 0;               // what goes through the pinned host staging buffer (all of it for pageable files)
     std::vector<UploadRun> runs;               // pinned files: copied from the caller's memory, one run per group of close files
@@ -71,6 +78,7 @@ struct DecChunk {
     uint32_t max_windows = 1;
     int max_intervals = 0;
     int max_blocks = 0;
+    int max_luma_blocks = 0;                   // real luma blocks of the largest image (coefficient-only calls)
     int64_t max_groups = 0;                    // 8-pixel groups of the largest image
     // Huffman decoding: one CTA per file in one launch, or a file's windows shared out among `parts` CTAs in three launches
     bool one_launch = true;
@@ -115,7 +123,8 @@ inline void plan_decode(const DecodeCall &c, DecodePlan &P)
         if (prc == JPEG_UNSUPPORTED)
             return refuse(P, V5ELA_ERR_UNSUPPORTED, "not an 8-bit baseline one-component / 4:2:0 / 4:2:2 / 4:4:4 JPEG", i);
         if (prc != JPEG_OK) return refuse(P, V5ELA_ERR_INVALID, "corrupt JPEG headers", i);
-        if ((c.rgb_offsets && c.rgb_offsets[i] < 0) || (c.gray_offsets && c.gray_offsets[i] < 0))
+        if ((c.rgb_offsets && c.rgb_offsets[i] < 0) || (c.gray_offsets && c.gray_offsets[i] < 0) ||
+            (c.want_map && c.map_offsets && c.map_offsets[i] < 0))
             return refuse(P, V5ELA_ERR_INVALID, "negative output offset", i);
         const FileInfo &F = P.info[(size_t)i];
         HuffSpecSet ts;                        // (HuffSpec has no padding bytes and parse_file zeroes what it does not fill)
@@ -139,7 +148,7 @@ inline void plan_decode(const DecodeCall &c, DecodePlan &P)
 
     // ---- chunks of files whose workspace stays under c.chunk_bytes (a 1080p file needs ~11 MB: coefficients, planes, streams)
     P.chunks.resize(1);
-    int64_t rgb_run = 0, gray_run = 0;
+    int64_t rgb_run = 0, gray_run = 0, map_run = 0;
     for (int i = 0; i < n; i++) {
         const FileInfo &F = P.info[(size_t)i];
         DecImage im;
@@ -147,7 +156,7 @@ inline void plan_decode(const DecodeCall &c, DecodePlan &P)
         dec_geometry(im, F.h, F.w, F.ncomp, F.hs, F.vs);
         im.tabset = tab_of[(size_t)i];
         im.qt = q_of[(size_t)i];
-        const size_t planes = (size_t)im.yw * im.yh + 2 * (size_t)im.cw * im.ch;
+        const size_t planes = c.coef_only ? 0 : (size_t)im.yw * im.yh + 2 * (size_t)im.cw * im.ch;
         const size_t need = F.scan_len * 2 + (size_t)im.blocks * 128 + planes + 256;
         DecChunk *C = &P.chunks.back();
         if (!C->images.empty() && (C->scan_bytes * 2 + C->coef_blocks * 128 + C->plane_bytes + need > c.chunk_bytes || C->images.size() >= 65535)) {
@@ -194,6 +203,10 @@ inline void plan_decode(const DecodeCall &c, DecodePlan &P)
         im.gray_off = c.want_gray ? (c.gray_offsets ? c.gray_offsets[i] : gray_run) : -1;
         rgb_run += (int64_t)F.h * F.w * 3;
         gray_run += (int64_t)F.h * F.w;
+        const int luma_blocks = ((F.h + 7) / 8) * ((F.w + 7) / 8);
+        if (c.want_map) C->map_off.push_back(c.map_offsets ? c.map_offsets[i] : map_run);
+        map_run += luma_blocks;
+        if (luma_blocks > C->max_luma_blocks) C->max_luma_blocks = luma_blocks;
         C->scan_bytes = start + F.scan_len;
         C->stream_bytes += align_up(F.scan_len + 32, 16);
         C->coef_blocks += (size_t)im.blocks;
@@ -209,7 +222,8 @@ inline void plan_decode(const DecodeCall &c, DecodePlan &P)
         C.off_img = 0;
         C.off_tab = align_up(sizeof(DecImage) * (size_t)cn, 16);
         C.off_q = C.off_tab + align_up(sizeof(DecTabSet) * P.tabsets.size(), 16);
-        C.off_scan = C.off_q + align_up(256 * P.qsets.size(), 16);
+        C.off_map = C.off_q + align_up(256 * P.qsets.size(), 16);
+        C.off_scan = C.off_map + (c.want_map ? align_up(sizeof(int64_t) * (size_t)cn, 16) : 0);
         C.stage_bytes = C.off_scan + align_up(C.scan_bytes, 16);
         // Files in pinned (page-locked) host memory are copied to the device straight from where they are — the caller keeps
         // them alive until the stream has been synchronised; pageable files go through the handle's pinned staging buffer.
@@ -226,7 +240,8 @@ inline void plan_decode(const DecodeCall &c, DecodePlan &P)
         C.parts = parts;
         // nothing to gain from splitting when there is no room for two parts per file, or no file has more than one window
         C.one_launch = c.huff_path ? c.huff_path == 1 : (c.sm_count / cn < 2 || C.max_windows < 2);
-        C.launches = (C.one_launch ? 5 : 7) + (C.max_intervals > 0 ? 1 : 0);
+        // unstuff, Huffman (1 or 3), dc, then idct + colour, or the statistics: histogram (+ tables and map)
+        C.launches = (C.one_launch ? 3 : 5) + (C.max_intervals > 0 ? 1 : 0) + (c.coef_only ? (c.want_map ? 3 : 1) : 2);
     }
 }
 

@@ -18,6 +18,7 @@ EXPORTS = (
     "v5ela_jpeg_encode_host", "v5ela_jpeg_info", "v5ela_jpeg_info_batch", "v5ela_jpeg_decode", "v5ela_jpeg_decode_host",
     "v5ela_last_instantiation", "v5ela_set_block_stage", "v5ela_get_block_stage", "v5ela_analyze_ragged", "v5ela_analyze_ragged_host",
     "v5ela_spectrum_ragged", "v5ela_spectrum_ragged_host", "v5ela_analyze_sweep", "v5ela_analyze_sweep_host",
+    "v5ela_jpeg_dct_stats", "v5ela_jpeg_dct_stats_host", "v5ela_jpeg_ijg_quality",
 )
 BLOCK_STAGES = {"smem": 0, "mma": 1}
 INSTANTIATIONS = {0: "general", 1: "fast", 2: "texhist", -1: None}
@@ -91,6 +92,9 @@ def load() -> ctypes.CDLL:
     lib.v5ela_jpeg_info_batch.argtypes = [vp, vp, i32, vp, ctypes.POINTER(i32)]
     lib.v5ela_jpeg_decode.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp, vp, vp]
     lib.v5ela_jpeg_decode_host.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp]
+    lib.v5ela_jpeg_dct_stats.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp, vp, vp]
+    lib.v5ela_jpeg_dct_stats_host.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp]
+    lib.v5ela_jpeg_ijg_quality.argtypes = [vp, vp]
     lib.v5ela_profile_enable.argtypes = [vp, i32]
     lib.v5ela_profile_read.argtypes = [vp, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(i64), i32]
     lib.v5ela_last_instantiation.argtypes = [vp]
@@ -216,6 +220,15 @@ class Handle:
     def jpeg_decode_host(self, files, lens, n: int, rgb_host: int | None, rgb_offsets, gray_host: int | None, gray_offsets):
         self._check(self._lib.v5ela_jpeg_decode_host(self._h, files, lens, n, rgb_host or None, rgb_offsets, gray_host or None,
                                                      gray_offsets))
+
+    def jpeg_dct_stats(self, files, lens, n: int, d_hist: int, d_qtab: int | None, d_map: int | None, map_offsets,
+                       d_status: int | None, stream: int | None):
+        self._check(self._lib.v5ela_jpeg_dct_stats(self._h, files, lens, n, d_hist, d_qtab or None, d_map or None, map_offsets,
+                                                   d_status or None, stream or None))
+
+    def jpeg_dct_stats_host(self, files, lens, n: int, hist_host: int, qtab_host: int | None, map_host: int | None, map_offsets):
+        self._check(self._lib.v5ela_jpeg_dct_stats_host(self._h, files, lens, n, hist_host, qtab_host or None, map_host or None,
+                                                        map_offsets))
 
     def profile_enable(self, enable: bool = True):
         self._check(self._lib.v5ela_profile_enable(self._h, 1 if enable else 0))

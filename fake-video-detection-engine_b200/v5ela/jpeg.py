@@ -4,6 +4,9 @@
                                 (reference v5_texture_ela.py:64, :83) — pixel-identical
   encode_host / encode_batch  : Image.save(.., 'JPEG', quality=q) and cv2.imwrite('.jpg', gray)
                                 (reference v5_texture_ela.py:66-67, :80-81, :90-91) — byte-identical
+  dct_stats / dct_stats_host  : per-frequency histograms of the files' quantised DCT coefficients, their quantisation tables
+                                and a per-block map of aligned double compression (DESIGN.md §4.8)
+  ijg_quality                 : the IJG quality whose tables a file's DQT equals
 No CPU implementation exists behind these; files outside the decoder's supported set raise V5ElaError(status -5).
 """
 from __future__ import annotations
@@ -154,3 +157,94 @@ def decode_batch(files, device=0, want_rgb: bool = True, want_gray: bool = False
                                            torch.cuda.current_stream(dev).cuda_stream)
     del keep
     return out
+
+
+DQ_HIST_SHAPE = (3, 64, 129)
+
+
+def _map_layout(files, table):
+    """(per-file map shapes (ceil(H/8), ceil(W/8)), packed element offsets (N + 1))"""
+    shapes = [((int(h) + 7) // 8, (int(w) + 7) // 8) for h, w, _ in info_batch(files, table)]
+    offs = np.concatenate([[0], np.cumsum([a * b for a, b in shapes])]).astype(np.int64)
+    return shapes, offs
+
+
+def dct_stats(files, want_qtab: bool = True, want_map: bool = False, device=0, handle=None):
+    """files: list of bytes (or uint8 arrays; any mix of sizes and layouts) -> dict of CUDA tensors, asynchronous on the current
+    stream:
+      'hist'   int32 (N, 3, 64, 129): [i][c][k][v + 64] counts the real blocks of component c of file i whose quantised coefficient
+               at natural-order position k is v, clamped to -64..64 (the counts are uint32 in the library; int32 is a view)
+      'qtab'   uint16 (N, 3, 64): each component's quantisation table, natural order (want_qtab)
+      'map'    list of N float32 (ceil(H/8), ceil(W/8)) views into one arena: per luma block, the posterior that the block was not
+               aligned-double-compressed (want_map)
+      'status' int32 (N): 0, or -1 for a file whose entropy-coded data ends early
+    Header parsing happens on the calling thread; files that are views into pinned memory are read asynchronously."""
+    import torch
+
+    n = len(files)
+    dev = torch.device("cuda", device) if not isinstance(device, torch.device) else device
+    out = {"hist": torch.zeros((n,) + DQ_HIST_SHAPE, dtype=torch.int32, device=dev),
+           "status": torch.zeros(n, dtype=torch.int32, device=dev)}
+    if want_qtab:
+        out["qtab"] = torch.zeros((n, 3, 64), dtype=torch.uint16, device=dev)
+    if n == 0:
+        if want_map:
+            out["map"] = []
+        return out
+    table = _file_table(files)
+    arena = None
+    if want_map:
+        shapes, offs = _map_layout(files, table)
+        arena = torch.empty(int(offs[-1]), dtype=torch.float32, device=dev)
+        out["map"] = [arena[int(offs[i]):int(offs[i + 1])].view(shapes[i]) for i in range(n)]
+    keep, ptrs, lens = table
+    (handle or _abi.get_handle(dev.index or 0)).jpeg_dct_stats(
+        ptrs, lens, n, out["hist"].data_ptr(), out["qtab"].data_ptr() if want_qtab else None,
+        arena.data_ptr() if want_map else None, None, out["status"].data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+    del keep
+    return out
+
+
+def dct_stats_host(files, want_qtab: bool = True, want_map: bool = False, device=0, handle=None):
+    """The same as NumPy arrays ('hist' uint32, 'qtab' uint16, 'map' list of float32 views into one array); synchronous, and a file
+    whose entropy-coded data ends early raises V5ElaError(-1)."""
+    n = len(files)
+    out = {"hist": np.zeros((n,) + DQ_HIST_SHAPE, np.uint32)}
+    if want_qtab:
+        out["qtab"] = np.zeros((n, 3, 64), np.uint16)
+    if n == 0:
+        if want_map:
+            out["map"] = []
+        return out
+    table = _file_table(files)
+    arena = None
+    if want_map:
+        shapes, offs = _map_layout(files, table)
+        arena = np.empty(int(offs[-1]), np.float32)
+        out["map"] = [arena[offs[i]:offs[i + 1]].reshape(shapes[i]) for i in range(n)]
+    keep, ptrs, lens = table
+    (handle or _abi.get_handle(device)).jpeg_dct_stats_host(ptrs, lens, n, out["hist"].ctypes.data,
+                                                            out["qtab"].ctypes.data if want_qtab else None,
+                                                            arena.ctypes.data if want_map else None, None)
+    del keep
+    return out
+
+
+def ijg_quality(qtab):
+    """qtab: one file's quantisation tables, natural order — (3, 64) as dct_stats returns them (components a one-component file
+    lacks are zero), (2, 64) luma + chroma, or (64,) luma alone; a tensor or an array. -> the IJG quality 1..100 whose
+    jpeg_set_quality tables (what libjpeg, and so PIL and OpenCV, write for `quality`) equal them, or None. Host only."""
+    if hasattr(qtab, "detach"):
+        qtab = qtab.detach().cpu().numpy()
+    q = np.ascontiguousarray(np.asarray(qtab).reshape(-1, 64), dtype=np.uint16)
+    if q.shape[0] not in (1, 2, 3):
+        raise ValueError("qtab must hold one, two or three tables of 64 entries")
+    chroma = None
+    if q.shape[0] >= 2 and q[1:].any():
+        if q.shape[0] == 3 and not np.array_equal(q[1], q[2]):
+            return None                                                   # the IJG tables give Cb and Cr the same table
+        chroma = q[1]
+    r = _abi.load().v5ela_jpeg_ijg_quality(q[0].ctypes.data, chroma.ctypes.data if chroma is not None else None)
+    if r < 0:
+        raise _abi.V5ElaError(r, "v5ela_jpeg_ijg_quality: bad table")
+    return int(r) or None

@@ -287,6 +287,40 @@ V5ELA_API int v5ela_jpeg_decode_host(v5ela_handle *h, const uint8_t *const *file
                            uint8_t *rgb_host, const int64_t *rgb_offsets, uint8_t *gray_host, const int64_t *gray_offsets);
 
 /*
+ * DCT statistics of JPEG files (DESIGN.md §4.8): what the decoder reads from the files before any pixel exists — the quantised
+ * coefficients and quantisation tables — as per-frequency histograms, and a per-block map of aligned double JPEG compression
+ * (Popescu & Farid 2004; Lin, He, Tang & Tang 2009). The files, the supported set, the refusals (V5ELA_ERR_UNSUPPORTED naming
+ * the file), the staging of pinned and pageable files and the Huffman decoding are v5ela_jpeg_decode's; the decode stops once
+ * the coefficients are known (no inverse DCT, no colour conversion).
+ *   d_hist  : DEVICE uint32 [n][3][64][129]. Entry [i][c][k][v + 64] counts the blocks of component c (0 Y, 1 Cb, 2 Cr) of file i
+ *             whose quantised coefficient at NATURAL-order position k equals v, values clamped to -64 .. 64 (the end bins
+ *             saturate). k = 0 is the DC value with the prediction undone. Only real blocks count: bx < ceil(ceil(W h_c / h_max) / 8),
+ *             by < ceil(ceil(H v_c / v_max) / 8); the padding blocks of the MCU grid do not. A one-component file leaves c = 1, 2 zero.
+ *   d_qtab  : optional DEVICE uint16 [n][3][64]: each component's quantisation table, natural order, as the file's DQT gives it
+ *             (zero for the components a one-component file lacks).
+ *   d_map   : optional DEVICE float32 maps, one per file with one entry per real luma 8x8 block (ceil(H/8) rows of ceil(W/8)):
+ *             the posterior that the block was NOT aligned-double-compressed. File i's map starts at element map_offsets[i], or
+ *             the maps are packed in file order when map_offsets is NULL; a negative offset is refused with V5ELA_ERR_INVALID
+ *             before anything is launched. The estimator, per file, for the 15 luma AC frequencies k at zigzag positions 1..15:
+ *               h = the luma histogram of k, g(v) = h(v) + h(-v) for v = 1..63, N = sum g; N < 64: p_k = 1. Otherwise, with
+ *               r(v) = g(v) - (g(v-1) + g(v+1)) / 2 (v = 2..62) and S(p) = |sum r(v) e^{-2 pi i v / p}| / max(sum |r|, 1) for
+ *               p = 2..12, p* = argmax S (the smaller p on ties) and p_k = p* if S(p*) >= 0.5 and sum |r| >= 0.05 N, else 1.
+ *               P_u(v) = h(v) / (sum of h over the p_k bins from p_k floor(v / p_k) on, clipped to -63..63), 1 / p_k where that
+ *               sum is 0; the clamped values +-64 use the entries of +-63. P_t = 1 / p_k.
+ *               map = 1 / (1 + exp(sum over the k with p_k > 1 of log P_u(v_k) - log P_t)), 0.5 when no k has p_k > 1.
+ *   d_status: optional DEVICE int32 [n], as v5ela_jpeg_decode's.
+ * Asynchronous on `cuda_stream`; the workspace is the decoder's, inside the handle.
+ */
+V5ELA_API int v5ela_jpeg_dct_stats(v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n, uint32_t *d_hist,
+                                   uint16_t *d_qtab, float *d_map, const int64_t *map_offsets, int32_t *d_status, void *cuda_stream);
+/* Same with HOST outputs (map offsets likewise); synchronises, and reports truncated / corrupt entropy data as V5ELA_ERR_INVALID. */
+V5ELA_API int v5ela_jpeg_dct_stats_host(v5ela_handle *h, const uint8_t *const *files_host, const int64_t *lens, int n,
+                                        uint32_t *hist_host, uint16_t *qtab_host, float *map_host, const int64_t *map_offsets);
+/* The IJG quality 1..100 whose tables (libjpeg's jpeg_set_quality, baseline-forced: what v5ela_set_quality derives) equal
+ * luma[64] and, unless chroma is NULL, chroma[64] (natural order, as in d_qtab); 0 when no quality does. No device needed. */
+V5ELA_API int v5ela_jpeg_ijg_quality(const uint16_t luma[64], const uint16_t *chroma);
+
+/*
  * Measurement hook: while enabled, every v5ela_analyze records a CUDA event pair around the fused kernel on the launch
  * stream. v5ela_profile_read waits for the recorded events, returns the summed kernel time and launch count since the
  * last reset, and optionally resets. Used by bench.py for the roofline line; off by default.
