@@ -343,12 +343,14 @@ int v5ela_analyze_ragged(v5ela_handle *h, const v5ela_frame_desc *frames_host, i
     p.frames = reinterpret_cast<const v5plan::FrameDesc *>(static_cast<uint8_t *>(h->d_table));
     v5plan::fill_quant(p.q, h->quality);
     if ((rc = launch_fused(h, p, v5plan::choose_instantiation(p), total, st))) return rc;
-    if (any_enh) {
-        if (n > 65535) return fail(h, V5ELA_ERR_INVALID, "v5ela_analyze_ragged: more than 65535 frames with enhanced maps%s");
-        v5::ela_enhance_ragged_kernel<<<dim3(32, (unsigned)n), 256, 0, st>>>(
-            reinterpret_cast<const v5::EnhDesc *>(h->d_table + desc_bytes), static_cast<const v5ela_record *>(d_records));
-        V5_CUDA(h, cudaGetLastError());
-        h->launches += 1;
+    if (any_enh) {                                              // one launch per 65535 frames (grid y)
+        const v5::EnhDesc *tab = reinterpret_cast<const v5::EnhDesc *>(h->d_table + desc_bytes);
+        for (int f0 = 0; f0 < n; f0 += 65535) {
+            const int fn = n - f0 < 65535 ? n - f0 : 65535;
+            v5::ela_enhance_ragged_kernel<<<dim3(32, (unsigned)fn), 256, 0, st>>>(tab + f0, static_cast<const v5ela_record *>(d_records) + f0);
+            V5_CUDA(h, cudaGetLastError());
+            h->launches += 1;
+        }
     }
     return V5ELA_OK;
 }
@@ -498,11 +500,13 @@ int v5ela_enhance(v5ela_handle *h, const uint8_t *d_residual, const void *d_reco
     long long bx = (bytes / 16 + 255) / 256;
     if (bx < 1) bx = 1;
     if (bx > 4LL * h->sm_count) bx = 4LL * h->sm_count;
-    if (n > 65535) return fail(h, V5ELA_ERR_INVALID, "v5ela_enhance: more than 65535 frames per call%s");
-    v5::ela_enhance_kernel<<<dim3((unsigned)bx, (unsigned)n), 256, 0, static_cast<cudaStream_t>(cuda_stream)>>>(
-        d_residual, static_cast<const v5ela_record *>(d_records), d_enhanced, bytes);
-    V5_CUDA(h, cudaGetLastError());
-    h->launches += 1;
+    for (int f0 = 0; f0 < n; f0 += 65535) {                    // one launch per 65535 frames (grid y)
+        const int fn = n - f0 < 65535 ? n - f0 : 65535;
+        v5::ela_enhance_kernel<<<dim3((unsigned)bx, (unsigned)fn), 256, 0, static_cast<cudaStream_t>(cuda_stream)>>>(
+            d_residual + (int64_t)f0 * bytes, static_cast<const v5ela_record *>(d_records) + f0, d_enhanced + (int64_t)f0 * bytes, bytes);
+        V5_CUDA(h, cudaGetLastError());
+        h->launches += 1;
+    }
     return V5ELA_OK;
 }
 

@@ -26,7 +26,8 @@ struct v5jpeg_state {
     DeviceBuf<v5j::EncTables> d_enc_tabs;
     DeviceBuf<uint8_t> d_header;
     DeviceBuf<int16_t> d_coef;
-    DeviceBuf<uint32_t> d_bitoff, d_total, d_raw;
+    DeviceBuf<uint64_t> d_bitoff, d_total;
+    DeviceBuf<uint32_t> d_raw;
     // host-buffer entry points
     DeviceBuf<uint8_t> d_img, d_out;
     DeviceBuf<int32_t> d_sizes;
@@ -115,14 +116,14 @@ try {
     // images per pass: keep the workspace (coefficients 128 B/block, offsets, unstuffed stream) under ~8 GiB (one pass for a
     // few hundred 1080p frames: the per-image-CTA kernels cost the same for 8 images as for 148)
     const int64_t raw_words = (out_stride_bytes + 3) / 4;
-    const size_t per_image = (size_t)g.blocks * (128 + 4) + (size_t)raw_words * 4 + 16;
+    const size_t per_image = (size_t)g.blocks * (128 + 8) + (size_t)raw_words * 4 + 16;
     int chunk = (int)(((size_t)8 << 30) / per_image);
     if (chunk < 1) chunk = 1;
     if (chunk > n) chunk = n;
     if (chunk > 65535) chunk = 65535;
     if ((rc = s->d_coef.ensure(h, (size_t)chunk * g.blocks * 128))) return rc;
-    if ((rc = s->d_bitoff.ensure(h, (size_t)chunk * g.blocks * 4))) return rc;
-    if ((rc = s->d_total.ensure(h, (size_t)chunk * 4))) return rc;
+    if ((rc = s->d_bitoff.ensure(h, (size_t)chunk * g.blocks * 8))) return rc;
+    if ((rc = s->d_total.ensure(h, (size_t)chunk * 8))) return rc;
     if ((rc = s->d_raw.ensure(h, (size_t)chunk * raw_words * 4))) return rc;
 
     v5j::CoefParams cp;

@@ -243,6 +243,10 @@ inline bool make_dec_table(const HuffSpec &h, DecTable &t) { return make_dec_tab
 
 enum { JPEG_OK = 0, JPEG_CORRUPT = -1, JPEG_UNSUPPORTED = -2 };
 
+// The decoder's Huffman state holds bit positions in the unstuffed entropy-coded segment as 32-bit numbers, and rounds them up
+// to whole subsequences: a segment of kMaxScanBytes (2^29 - 2^20 bytes, 511 MiB) or more is refused as unsupported.
+constexpr size_t kMaxScanBytes = ((size_t)1 << 29) - ((size_t)1 << 20);
+
 struct FileInfo {
     int h = 0, w = 0, ncomp = 0;
     int hs = 1, vs = 1;       // luma sampling factors = luma blocks per MCU across / down (chroma is always 1 x 1)

@@ -434,8 +434,9 @@ __global__ void __launch_bounds__(ENC_NT) coef_kernel(const __grid_constant__ Co
 
 struct EntropyParams {
     const int16_t *coef;               // [n][blocks][64]
-    uint32_t *bitoff;                  // [n][blocks]: lengths after count_kernel, exclusive offsets after scan_kernel
-    uint32_t *total_bits;              // [n]
+    uint64_t *bitoff;                  // [n][blocks]: lengths after count_kernel, exclusive offsets after scan_kernel (64-bit:
+                                       // a file of up to 1 GiB holds 2^33 bits)
+    uint64_t *total_bits;              // [n]
     uint32_t *raw;                     // [n][raw_words] zero-initialised
     int64_t raw_words;
     int blocks, bpm, n;
@@ -461,9 +462,9 @@ __global__ void __launch_bounds__(128) entropy_kernel(const EntropyParams p, con
         encode_block(c, pred, s_dc[t], s_ac[t], cnt);
         p.bitoff[(int64_t)img * p.blocks + g] = cnt.total;
     } else {
-        const uint32_t off = p.bitoff[(int64_t)img * p.blocks + g];
-        const uint32_t end = g + 1 < p.blocks ? p.bitoff[(int64_t)img * p.blocks + g + 1] : p.total_bits[img];
-        if (end < off || (uint64_t)end > (uint64_t)p.raw_words * 32) return;       // does not fit: reported by stuff_kernel
+        const uint64_t off = p.bitoff[(int64_t)img * p.blocks + g];
+        const uint64_t end = g + 1 < p.blocks ? p.bitoff[(int64_t)img * p.blocks + g + 1] : p.total_bits[img];
+        if (end < off || end > (uint64_t)p.raw_words * 32) return;                 // does not fit: reported by stuff_kernel
         BitSink sink;
         sink.init(p.raw + (int64_t)img * p.raw_words, off);
         encode_block(c, pred, s_dc[t], s_ac[t], sink);
@@ -505,11 +506,11 @@ __global__ void __launch_bounds__(1024) scan_kernel(const EntropyParams p)
 {
     __shared__ uint32_t warp_sums[33];
     const int img = (int)blockIdx.x;
-    uint32_t *a = p.bitoff + (int64_t)img * p.blocks;
-    uint32_t running = 0;
+    uint64_t *a = p.bitoff + (int64_t)img * p.blocks;
+    uint64_t running = 0;                                                 // a block codes to < 2^12 bits: 1024 of them fit 32 bits
     for (int base = 0; base < p.blocks; base += 1024) {
         const int i = base + (int)threadIdx.x;
-        const uint32_t v = i < p.blocks ? a[i] : 0u;
+        const uint32_t v = i < p.blocks ? (uint32_t)a[i] : 0u;
         uint32_t sum;
         const uint32_t ex = cta_exclusive_scan(v, warp_sums, &sum);
         if (i < p.blocks) a[i] = running + ex;
@@ -521,7 +522,7 @@ __global__ void __launch_bounds__(1024) scan_kernel(const EntropyParams p)
 struct StuffParams {
     const uint32_t *raw;
     int64_t raw_words;
-    const uint32_t *total_bits;
+    const uint64_t *total_bits;
     const uint8_t *header;
     int header_len;
     uint8_t *out;                      // [n][out_stride]
@@ -535,9 +536,9 @@ __global__ void __launch_bounds__(1024) stuff_kernel(const StuffParams p)
     const int img = (int)blockIdx.x;
     const uint32_t *raw = p.raw + (int64_t)img * p.raw_words;
     uint8_t *out = p.out + (int64_t)img * p.out_stride;
-    const uint32_t bits = p.total_bits[img];
-    const uint32_t nbytes = (bits + 7) >> 3;
-    const bool fits_raw = (uint64_t)nbytes <= (uint64_t)p.raw_words * 4;
+    const uint64_t bits = p.total_bits[img];
+    const bool fits_raw = (bits + 7) >> 3 <= (uint64_t)p.raw_words * 4;
+    const uint32_t nbytes = fits_raw ? (uint32_t)((bits + 7) >> 3) : 0u;   // raw_words * 4 <= 2^30 + 3 (v5ela_jpeg_encode)
     for (int i = threadIdx.x; i < p.header_len && i < p.out_stride; i += blockDim.x) out[i] = p.header[i];
     uint32_t running = (uint32_t)p.header_len;
     const uint32_t nwords = (nbytes + 3) >> 2;
@@ -545,7 +546,7 @@ __global__ void __launch_bounds__(1024) stuff_kernel(const StuffParams p)
         const uint32_t wi = base + threadIdx.x;
         uint32_t word = 0, nb = 0, nff = 0;
         if (wi < nwords) {
-            word = fits_raw ? raw[wi] : 0u;
+            word = raw[wi];
             nb = nbytes - 4 * wi < 4 ? nbytes - 4 * wi : 4;
             if (wi == nwords - 1 && (bits & 7)) word |= (0xffu >> (bits & 7)) << (8 * (3 - ((nbytes - 1) & 3)));   // pad with ones
             for (uint32_t k = 0; k < nb; k++) nff += ((word >> (24 - 8 * k)) & 0xffu) == 0xffu;
@@ -568,7 +569,7 @@ __global__ void __launch_bounds__(1024) stuff_kernel(const StuffParams p)
             out[running] = 0xFF;
             out[running + 1] = 0xD9;
         }
-        p.sizes[img] = fits_raw ? (int32_t)(running + 2) : 0x7fffffff;
+        p.sizes[img] = fits_raw && running + 2 <= 0x7fffffffu ? (int32_t)(running + 2) : 0x7fffffff;
     }
 }
 #endif  // __CUDACC__

@@ -123,6 +123,8 @@ inline void plan_decode(const DecodeCall &c, DecodePlan &P)
         if (prc == JPEG_UNSUPPORTED)
             return refuse(P, V5ELA_ERR_UNSUPPORTED, "not an 8-bit baseline one-component / 4:2:0 / 4:2:2 / 4:4:4 JPEG", i);
         if (prc != JPEG_OK) return refuse(P, V5ELA_ERR_INVALID, "corrupt JPEG headers", i);
+        if (P.info[(size_t)i].scan_len >= kMaxScanBytes)
+            return refuse(P, V5ELA_ERR_UNSUPPORTED, "entropy-coded segment of 2^29 - 2^20 bytes or more", i);
         if ((c.rgb_offsets && c.rgb_offsets[i] < 0) || (c.gray_offsets && c.gray_offsets[i] < 0) ||
             (c.want_map && c.map_offsets && c.map_offsets[i] < 0))
             return refuse(P, V5ELA_ERR_INVALID, "negative output offset", i);

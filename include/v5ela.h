@@ -124,7 +124,7 @@ V5ELA_API int v5ela_analyze_ex(v5ela_handle *h, const uint8_t *d_rgb, int n, int
  * The descriptor table goes to the device through a small pinned staging buffer inside the handle (the only host work besides
  * filling it; before refilling it the call waits, on the host, for the PREVIOUS ragged call's table upload — a few microseconds
  * of copy, normally long finished). Otherwise asynchronous on `cuda_stream`; launches: memsets, the fused kernel, the finalize kernel and — only when a frame
- * asks for an enhanced map — one enhancement kernel for the whole batch.
+ * asks for an enhanced map — one enhancement kernel per 65535 frames of the batch.
  */
 typedef struct v5ela_frame_desc {
     const uint8_t *rgb;         /* uint8 HWC RGB */
@@ -168,7 +168,8 @@ V5ELA_API int v5ela_analyze_sweep_host(v5ela_handle *h, const v5ela_frame_desc *
 /*
  * Brightness enhancement of the residual map: `ImageEnhance.Brightness(diff).enhance(255.0 / max_diff)`
  * (v5_texture_ela.py:74-78) == u8(trunc(f32(x) * f32(scale))) clipped, with max_diff read per frame from the records
- * produced by v5ela_analyze on the same stream (0 -> 1 fix applied). d_enhanced may alias d_residual.
+ * produced by v5ela_analyze on the same stream (0 -> 1 fix applied). d_enhanced may alias d_residual. Any n: one launch per
+ * 65535 frames.
  */
 V5ELA_API int v5ela_enhance(v5ela_handle *h, const uint8_t *d_residual, const void *d_records, int n, int height, int width,
                   uint8_t *d_enhanced, void *cuda_stream);
@@ -239,8 +240,9 @@ V5ELA_API int v5ela_spectrum_ragged_host(v5ela_handle *h, const v5ela_gray_desc 
  * `enhanced_diff.save(ela_i.jpg)` (v5…:80-81, PIL default quality 75) and `cv2.imwrite(fft_i.jpg, spectrum)` (v5…:90-91, OpenCV
  * default quality 95, one component) — byte-identical to libjpeg's output: baseline sequential, Annex K tables scaled by
  * `quality`, 4:2:0 for three channels, the standard Huffman tables, JFIF 1.01 header.
- *   d_img      : n images, uint8, `channels` = 1 (HW) or 3 (HWC, RGB), all height x width.
- *   d_out      : n x out_stride_bytes; file i starts at d_out + i * out_stride_bytes.
+ *   d_img      : n images, uint8, `channels` = 1 (HW) or 3 (HWC, RGB), all height x width; sides up to 65535.
+ *   d_out      : n x out_stride_bytes (at most 1 GiB); file i starts at d_out + i * out_stride_bytes. Every file that fits comes
+ *                out right, however long its entropy-coded stream (up to 2^33 bits).
  *   d_sizes    : n file sizes. A size larger than out_stride_bytes means that file did not fit and its bytes are undefined;
  *                v5ela_jpeg_bound() is a capacity that always fits (it is ~13 bytes per pixel; real files are far smaller).
  * Asynchronous on `cuda_stream`; owns a workspace inside the handle.
@@ -258,9 +260,11 @@ V5ELA_API int v5ela_jpeg_encode_host(v5ela_handle *h, const uint8_t *img_host, i
  * `cv2.imread(crop_path, cv2.IMREAD_GRAYSCALE)` (v5…:83) — the crops V1 wrote with cv2.imwrite (v1_keyframes_facetrack.py:166).
  * Pixel-identical to libjpeg's defaults (ISLOW inverse DCT, fancy upsampling). Supported: 8-bit baseline Huffman files with
  * one component, or three components with the luma sampled 2x2 (4:2:0), 2x1 (4:2:2) or 1x1 (4:4:4) against 1x1 chroma; one
- * scan; any Huffman / quantisation tables; with or without restart intervals — everything PIL's and OpenCV's writers produce
- * by default (4:2:0, no restarts) plus what their sampling and restart options add. Anything else (progressive, other
- * sampling factors, CMYK, 12-bit, arithmetic coding) returns V5ELA_ERR_UNSUPPORTED and v5ela_last_error names the file.
+ * scan; any Huffman / quantisation tables; with or without restart intervals; an entropy-coded segment (stuffed bytes
+ * included) of less than 2^29 - 2^20 bytes (511 MiB; the decoder's Huffman state holds 32-bit bit positions) — everything
+ * PIL's and OpenCV's writers produce by default (4:2:0, no restarts) plus what their sampling and restart options add. Anything
+ * else (progressive, other sampling factors, CMYK, 12-bit, arithmetic coding, larger entropy-coded segments) returns
+ * V5ELA_ERR_UNSUPPORTED before anything is uploaded or launched, and v5ela_last_error names the file.
  *   files_host / lens : n complete JPEG files in HOST memory (they come from disk); sizes may differ from file to file.
  *             Files that all live in page-locked memory (cudaHostAlloc / cudaHostRegister / torch pin_memory) are copied
  *             to the device asynchronously from where they are — keep them alive until the stream has been synchronised;
