@@ -589,18 +589,6 @@ try {
     return V5ELA_OK;
 } V5_CATCH(h)
 
-// threads per CTA of the FFT kernels: 256; 512 measured no faster (profiles/r02/spectrum.txt). V5ELA_FFT_THREADS overrides
-// (tuning knob: 128 / 256 / 512)
-static unsigned fft_threads(int points)
-{
-    if (const char *env = getenv("V5ELA_FFT_THREADS")) {
-        const int v = atoi(env);
-        if (v == 128 || v == 256 || v == 512) return (unsigned)v;
-    }
-    (void)points;
-    return 256u;
-}
-
 // V5ELA_FFT=0 sends every frame down the exact-size DFT (tests compare the two paths); read on every call.
 static bool fft_enabled()
 {
@@ -616,6 +604,25 @@ static size_t spec_chunk_bytes()
         if (v >= 1 && v <= 4096) return (size_t)v << 20;
     }
     return (size_t)1 << 30;
+}
+
+// Lets the four FFT kernels (uniform and ragged) take up to FFT_SMEM_MAX of dynamic shared memory; once per handle.
+static int allow_fft_smem(v5ela_handle *h)
+{
+    if (h->fft_attr_set) return V5ELA_OK;
+    for (const void *k : {(const void *)v5fft::fft_rows_kernel, (const void *)v5fft::fft_cols_kernel, (const void *)v5fft::fft_rows_ragged_kernel,
+                          (const void *)v5fft::fft_cols_ragged_kernel})
+        V5_CUDA(h, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)v5fft::FFT_SMEM_MAX));
+    h->fft_attr_set = true;
+    return V5ELA_OK;
+}
+
+// The min/max pairs of n frames to {~0, 0}, ready for the column kernels' atomicMin / atomicMax.
+static int reset_minmax(v5ela_handle *h, int n, cudaStream_t st)
+{
+    V5_CUDA(h, cudaMemsetAsync(h->d_minmax, 0, sizeof(unsigned long long) * 2 * (size_t)n, st));
+    V5_CUDA(h, cudaMemset2DAsync(h->d_minmax, 16, 0xff, 8, (size_t)n, st));
+    return V5ELA_OK;
 }
 
 int v5ela_spectrum(v5ela_handle *h, const uint8_t *d_gray, int n, int height, int width, int64_t frame_stride_bytes,
@@ -662,21 +669,16 @@ int v5ela_spectrum(v5ela_handle *h, const uint8_t *d_gray, int n, int height, in
     const bool fast = v5fft::fft_path(fft_enabled(), height, width, plan_w, plan_h, shape) && n <= 65535;
     const int cc = shape.cc;
     const size_t rows_smem = shape.rows_smem, cols_smem = shape.cols_smem;
-    if (fast && !h->fft_attr_set) {
-        V5_CUDA(h, cudaFuncSetAttribute(v5fft::fft_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 << 10));
-        V5_CUDA(h, cudaFuncSetAttribute(v5fft::fft_cols_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 << 10));
-        h->fft_attr_set = true;
-    }
+    if (fast && (rc = allow_fft_smem(h))) return rc;
+    const v5fft::ImageGrid ig = v5fft::image_grid(height, width);
     for (int f0 = 0; f0 < n; f0 += chunk) {
         const int fn = f0 + chunk <= n ? chunk : n - f0;
-        // min/max slots: {~0, 0} per frame
-        V5_CUDA(h, cudaMemsetAsync(h->d_minmax, 0, sizeof(unsigned long long) * 2 * (size_t)fn, st));
-        V5_CUDA(h, cudaMemset2DAsync(h->d_minmax, 16, 0xff, 8, (size_t)fn, st));
+        if ((rc = reset_minmax(h, fn, st))) return rc;
         if (fast) {
-            v5fft::fft_rows_kernel<<<dim3((unsigned)((height + 1) / 2), (unsigned)fn), fft_threads(width), rows_smem, st>>>(
+            v5fft::fft_rows_kernel<<<dim3((unsigned)((height + 1) / 2), (unsigned)fn), 256, rows_smem, st>>>(
                 d_gray + (int64_t)f0 * frame_stride_bytes, frame_stride_bytes, row_stride_bytes, height, width, wh, plan_w, h->tw_w, h->d_g);
             V5_CUDA(h, cudaGetLastError());
-            v5fft::fft_cols_kernel<<<dim3((unsigned)((wh + cc - 1) / cc), (unsigned)fn), fft_threads(cc * height), cols_smem, st>>>(
+            v5fft::fft_cols_kernel<<<dim3((unsigned)((wh + cc - 1) / cc), (unsigned)fn), 256, cols_smem, st>>>(
                 h->d_g, height, wh, cc, plan_h, h->tw_h, h->d_ms, h->d_minmax);
             V5_CUDA(h, cudaGetLastError());
         } else {
@@ -688,12 +690,8 @@ int v5ela_spectrum(v5ela_handle *h, const uint8_t *d_gray, int n, int height, in
             v5fft::dft_cols_kernel<<<gr, 256, 0, st>>>(h->d_g, height, wh, h->tw_h, h->d_ms, h->d_minmax);
             V5_CUDA(h, cudaGetLastError());
         }
-        // every CTA walks ~16 rows: the per-thread set-up (the double-precision 255 / (max - min)) is paid once per 16 pixels
-        const unsigned bx = (unsigned)((width + 255) / 256);
-        unsigned by = (unsigned)((height + 15) / 16);
-        by = by < 1 ? 1 : (by > 65535 ? 65535 : by);
-        v5fft::spectrum_image_kernel<<<dim3(bx, by, (unsigned)fn), 256, 0, st>>>(h->d_ms, h->d_minmax, height, width, wh,
-                                                                                  d_out + (int64_t)f0 * height * width);
+        v5fft::spectrum_image_kernel<<<dim3((unsigned)ig.bx, (unsigned)ig.by, (unsigned)fn), 256, 0, st>>>(h->d_ms, h->d_minmax, height, width,
+                                                                                                            wh, d_out + (int64_t)f0 * height * width);
         V5_CUDA(h, cudaGetLastError());
         h->launches += 3;
     }
@@ -748,11 +746,7 @@ try {
     memcpy(tab + P.off_bases, P.bases.data(), sizeof(uint32_t) * P.bases.size());
     V5_CUDA(h, cudaMemcpyAsync(h->d_table, h->h_table, need, cudaMemcpyHostToDevice, st));
     V5_CUDA(h, cudaEventRecord(h->ev_table, st));
-    if (!h->fft_rag_attr_set) {
-        V5_CUDA(h, cudaFuncSetAttribute(v5fft::fft_rows_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)v5fft::FFT_SMEM_MAX));
-        V5_CUDA(h, cudaFuncSetAttribute(v5fft::fft_cols_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)v5fft::FFT_SMEM_MAX));
-        h->fft_rag_attr_set = true;
-    }
+    if ((rc = allow_fft_smem(h))) return rc;
     const uint8_t *dt = h->d_table;
     const auto *sizes = reinterpret_cast<const v5fft::SpecSize *>(dt + P.off_sizes);
     const auto *frames = reinterpret_cast<const v5fft::SpecFrame *>(dt + P.off_frames);
@@ -765,9 +759,7 @@ try {
         const v5fft::SpecFrame *cf = frames + C.f0;
         const uint32_t *base = bases + C.off_base;
         auto kind = [&](int k) { return base + (size_t)k * (C.n + 1); };
-        // min/max slots: {~0, 0} per frame
-        V5_CUDA(h, cudaMemsetAsync(h->d_minmax, 0, sizeof(unsigned long long) * 2 * (size_t)C.n, st));
-        V5_CUDA(h, cudaMemset2DAsync(h->d_minmax, 16, 0xff, 8, (size_t)C.n, st));
+        if ((rc = reset_minmax(h, C.n, st))) return rc;
         if (C.ctas[v5fft::L_FFT_ROWS]) {
             v5fft::fft_rows_ragged_kernel<<<C.ctas[v5fft::L_FFT_ROWS], 256, C.rows_smem, st>>>(cf, C.n, kind(v5fft::L_FFT_ROWS), sizes, h->tw_rag, h->d_g);
             V5_CUDA(h, cudaGetLastError());

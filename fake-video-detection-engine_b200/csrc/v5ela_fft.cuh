@@ -7,6 +7,10 @@
 // |F|, 20*ln(|F|+1) and the per-frame min/max; a last kernel normalises, shifts (fftshift) and mirrors the half
 // spectrum into the uint8 image. float64 throughout like NumPy; parity target is +-1 LSB of the uint8 image (the
 // reference's pocketfft sums in a different order), SURVEY.md §8f-1.
+//
+// Each stage is one __device__ body that takes a frame's geometry and pointers as arguments, called by a uniform kernel
+// (v5ela_spectrum) and a ragged one (v5ela_spectrum_ragged, planned in v5ela_spec_plan.h) that differ only in how a CTA finds its
+// frame: both run the same arithmetic, so every frame's image is byte-identical between the two calls.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -15,26 +19,38 @@
 
 namespace v5fft {
 
-// tw[m] = exp(-2*pi*i*m/n)
-__global__ void twiddle_kernel(double2 *tw, int n)
+// tw[m] = exp(-2*pi*i*m/n); nothing for m >= n
+__device__ __forceinline__ void twiddle_one(double2 *tw, int n, int m)
 {
-    const int m = blockIdx.x * blockDim.x + threadIdx.x;
     if (m >= n) return;
     double s, c;
     sincospi(2.0 * (double)m / (double)n, &s, &c);
     tw[m] = make_double2(c, -s);
 }
 
+// Folds every thread's (lo, hi) into the CTA's pair (smin, smax), which thread 0 set to {~0, 0} before a barrier, then the CTA's pair
+// into the frame's pair slot[0] (min), slot[1] (max). Must be called by every thread of the CTA.
+__device__ __forceinline__ void minmax_flush(unsigned long long &smin, unsigned long long &smax, unsigned long long lo,
+                                             unsigned long long hi, unsigned long long *slot)
+{
+    atomicMin(&smin, lo);
+    atomicMax(&smax, hi);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        atomicMin(&slot[0], smin);
+        atomicMax(&slot[1], smax);
+    }
+}
+
 constexpr int KC = 32;       // reduction chunk staged in shared memory
 
-// G[y][v] = sum_x gray[y][x] * twW[(x*v) mod W],  v in [0, W/2]
-__global__ void __launch_bounds__(256) dft_rows_kernel(const uint8_t *__restrict__ gray, int64_t frame_stride, int64_t row_stride,
-                                                       int h, int w, int wh, const double2 *__restrict__ tw, double2 *__restrict__ g)
+// G[y][v] = sum_x gray[y][x] * twW[(x*v) mod W],  v in [0, W/2], for the TILE x TILE outputs at (y0, v0) of one frame: src its
+// pixels, dst its G (h x wh). 256 threads.
+__device__ __forceinline__ void dft_rows_tile(const uint8_t *__restrict__ src, int64_t row_stride, int h, int w, int wh, int y0, int v0,
+                                              const double2 *__restrict__ tw, double2 *__restrict__ dst)
 {
     __shared__ double xs[TILE][KC + 1];
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const int y0 = blockIdx.y * TILE, v0 = blockIdx.x * TILE;
-    const uint8_t *src = gray + (int64_t)blockIdx.z * frame_stride;
     const int va = v0 + tx, vb = v0 + tx + 16;
     int ia = 0, ib = 0;                                         // (x * v) mod w for the two columns of this thread
     const int sa = va % w, sb = vb % w;
@@ -59,7 +75,6 @@ __global__ void __launch_bounds__(256) dft_rows_kernel(const uint8_t *__restrict
         }
         __syncthreads();
     }
-    double2 *dst = g + (int64_t)blockIdx.z * h * wh;
 #pragma unroll
     for (int i = 0; i < 2; i++) {
         const int y = y0 + ty + 16 * i;
@@ -69,15 +84,14 @@ __global__ void __launch_bounds__(256) dft_rows_kernel(const uint8_t *__restrict
     }
 }
 
-// ms[u][v] = 20*ln(|sum_y G[y][v] * twH[(u*y) mod H]| + 1); per-frame min/max as ordered uint64 (ms >= 0)
-__global__ void __launch_bounds__(256) dft_cols_kernel(const double2 *__restrict__ g, int h, int wh, const double2 *__restrict__ tw,
-                                                       double *__restrict__ ms, unsigned long long *__restrict__ minmax)
+// ms[u][v] = 20*ln(|sum_y G[y][v] * twH[(u*y) mod H]| + 1) for the TILE x TILE outputs at (u0, v0) of one frame: src its G, dst its
+// ms (both h x wh); the frame's min/max as ordered uint64 (ms >= 0) into minmax_slot. 256 threads.
+__device__ __forceinline__ void dft_cols_tile(const double2 *__restrict__ src, int h, int wh, int u0, int v0, const double2 *__restrict__ tw,
+                                              double *__restrict__ dst, unsigned long long *__restrict__ minmax_slot)
 {
     __shared__ double2 gs[KC][TILE + 1];
     __shared__ unsigned long long smin, smax;
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const int u0 = blockIdx.y * TILE, v0 = blockIdx.x * TILE;
-    const double2 *src = g + (int64_t)blockIdx.z * h * wh;
     if (threadIdx.x == 0) { smin = ~0ull; smax = 0ull; }
     const int ua = u0 + ty, ub = u0 + ty + 16;
     int ia = 0, ib = 0;
@@ -104,7 +118,6 @@ __global__ void __launch_bounds__(256) dft_cols_kernel(const double2 *__restrict
         }
         __syncthreads();
     }
-    double *dst = ms + (int64_t)blockIdx.z * h * wh;
     unsigned long long lo = ~0ull, hi = 0ull;
 #pragma unroll
     for (int i = 0; i < 2; i++) {
@@ -119,13 +132,7 @@ __global__ void __launch_bounds__(256) dft_cols_kernel(const double2 *__restrict
             hi = bits > hi ? bits : hi;
         }
     }
-    atomicMin(&smin, lo);
-    atomicMax(&smax, hi);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        atomicMin(&minmax[2 * blockIdx.z], smin);
-        atomicMax(&minmax[2 * blockIdx.z + 1], smax);
-    }
+    minmax_flush(smin, smax, lo, hi, minmax_slot);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -206,15 +213,13 @@ __device__ double2 *stockham(double2 *x, double2 *y, int nseq, const FftPlan &pl
     return x;
 }
 
-// Rows: two real rows ride in one complex transform (z = a + i b); the half spectra of both are separated with
-// A_k = (Z_k + conj(Z_{N-k}))/2, B_k = (Z_k - conj(Z_{N-k}))/(2i).
-__global__ void __launch_bounds__(512) fft_rows_kernel(const uint8_t *__restrict__ gray, int64_t frame_stride, int64_t row_stride,
-                                                       int h, int w, int wh, const __grid_constant__ FftPlan plan,
-                                                       const double2 *__restrict__ tw, double2 *__restrict__ g)
+// Rows y0 and y0 + 1 of one frame (src its pixels) into its G rows from dst_row on. The two real rows ride in one complex
+// transform (z = a + i b); the half spectra of both are separated with A_k = (Z_k + conj(Z_{N-k}))/2, B_k = (Z_k - conj(Z_{N-k}))/(2i).
+__device__ __forceinline__ void fft_rows_pair(const uint8_t *__restrict__ src, int64_t row_stride, int h, int w, int wh, int y0,
+                                              const FftPlan &plan, const double2 *__restrict__ tw, double2 *__restrict__ dst_row)
 {
     extern __shared__ double2 fbuf[];
-    const int y0 = 2 * blockIdx.x, y1 = y0 + 1;
-    const uint8_t *src = gray + (int64_t)blockIdx.y * frame_stride;
+    const int y1 = y0 + 1;
     // all of a thread's pixels are requested before the first one is converted (memory-level parallelism: the kernel is latency-bound)
     const uint8_t *r0 = src + (int64_t)y0 * row_stride, *r1 = src + (int64_t)(y1 < h ? y1 : y0) * row_stride;
     for (int xb = 0; xb < w; xb += 4 * blockDim.x) {
@@ -233,11 +238,10 @@ __global__ void __launch_bounds__(512) fft_rows_kernel(const uint8_t *__restrict
     }
     __syncthreads();
     const double2 *res = stockham(fbuf, fbuf + w, 1, plan, tw);
-    double2 *ga = g + ((int64_t)blockIdx.y * h + y0) * wh;
     for (int k = threadIdx.x; k < wh; k += blockDim.x) {
         const double2 zk = res[k], zn = res[k == 0 ? 0 : w - k];
-        ga[k] = make_double2(0.5 * (zk.x + zn.x), 0.5 * (zk.y - zn.y));
-        if (y1 < h) ga[wh + k] = make_double2(0.5 * (zk.y + zn.y), 0.5 * (zn.x - zk.x));
+        dst_row[k] = make_double2(0.5 * (zk.x + zn.x), 0.5 * (zk.y - zn.y));
+        if (y1 < h) dst_row[wh + k] = make_double2(0.5 * (zk.y + zn.y), 0.5 * (zn.x - zk.x));
     }
 }
 
@@ -276,18 +280,17 @@ __device__ __forceinline__ double log_magnitude20(const LogTab &t, double s)
     return 20.0 * fabs(fma((double)e, 0.69314718055994530942, t.neg_ln_inv_c[i]) + p * q);
 }
 
-// Columns: `cc` adjacent columns per CTA (cc * 16 contiguous bytes per row), transform, then |F|, 20 ln(|F|+1), min/max.
-__global__ void __launch_bounds__(512) fft_cols_kernel(const double2 *__restrict__ g, int h, int wh, int cc,
-                                                       const __grid_constant__ FftPlan plan, const double2 *__restrict__ tw,
-                                                       double *__restrict__ ms, unsigned long long *__restrict__ minmax)
+// Columns v0 .. v0 + cc - 1 of one frame (src its G, dst its ms, both h x wh; cc * 16 contiguous bytes per row): transform, then |F|,
+// 20 ln(|F|+1), and the frame's min/max into minmax_slot.
+__device__ __forceinline__ void fft_cols_group(const double2 *__restrict__ src, int h, int wh, int cc, int v0, const FftPlan &plan,
+                                               const double2 *__restrict__ tw, double *__restrict__ dst,
+                                               unsigned long long *__restrict__ minmax_slot)
 {
     extern __shared__ double2 fbuf[];
     __shared__ unsigned long long smin, smax;
     __shared__ LogTab logtab;
     if (threadIdx.x == 0) { smin = ~0ull; smax = 0ull; }
     logtab_fill(logtab);
-    const int v0 = blockIdx.x * cc;
-    const double2 *src = g + (int64_t)blockIdx.y * h * wh;
     const int csh = cc == 4 ? 2 : (cc == 2 ? 1 : 0);              // cc is 1, 2 or 4 (host): i / cc and i % cc are a shift and a mask
     for (int ib = 0; ib < h * cc; ib += 4 * blockDim.x) {          // four loads in flight per thread before the first store
         double2 t[4];
@@ -306,7 +309,6 @@ __global__ void __launch_bounds__(512) fft_cols_kernel(const double2 *__restrict
     }
     __syncthreads();
     const double2 *res = stockham(fbuf, fbuf + cc * h, cc, plan, tw);
-    double *dst = ms + (int64_t)blockIdx.y * h * wh;
     unsigned long long lo = ~0ull, hi = 0ull;
     for (int i = threadIdx.x; i < h * cc; i += blockDim.x) {
         const int u = i >> csh, c = i & (cc - 1);
@@ -319,297 +321,142 @@ __global__ void __launch_bounds__(512) fft_cols_kernel(const double2 *__restrict
         lo = bits < lo ? bits : lo;
         hi = bits > hi ? bits : hi;
     }
-    atomicMin(&smin, lo);
-    atomicMax(&smax, hi);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        atomicMin(&minmax[2 * blockIdx.y], smin);
-        atomicMax(&minmax[2 * blockIdx.y + 1], smax);
-    }
+    minmax_flush(smin, smax, lo, hi, minmax_slot);
 }
 
-// out[i][j] = u8(rint(ms_shifted[i][j] * scale + shift)), cv2.normalize(NORM_MINMAX, 0..255) + np.fft.fftshift.
-// grid (column blocks, rows, frames): no index divisions.
-__global__ void __launch_bounds__(256) spectrum_image_kernel(const double *__restrict__ ms, const unsigned long long *__restrict__ minmax,
-                                                             int h, int w, int wh, uint8_t *__restrict__ out)
+// out[i][j] = u8(rint(ms_shifted[i][j] * scale + shift)), cv2.normalize(NORM_MINMAX, 0..255) + np.fft.fftshift, for one frame (ms its
+// half spectrum, minmax_slot its min/max, out its image): this CTA is column block bx of nbx and row block by of nby, so no index
+// divisions.
+__device__ __forceinline__ void spectrum_image_part(const double *__restrict__ ms, const unsigned long long *__restrict__ minmax_slot, int h,
+                                                    int w, int wh, int bx, int by, int nbx, int nby, uint8_t *__restrict__ out)
 {
-    const int frame = blockIdx.z;
-    const double mn = __longlong_as_double((long long)minmax[2 * frame]), mx = __longlong_as_double((long long)minmax[2 * frame + 1]);
+    const double mn = __longlong_as_double((long long)minmax_slot[0]), mx = __longlong_as_double((long long)minmax_slot[1]);
     const double scale = (mx - mn) > 2.220446049250313e-16 ? 255.0 / (mx - mn) : 0.0;   // cv::normalize: DBL_EPSILON guard
     const double shift = 0.0 - mn * scale;
-    const double *src = ms + (int64_t)frame * h * wh;
-    uint8_t *dst = out + (int64_t)frame * h * w;
-    for (int i = blockIdx.y; i < h; i += gridDim.y) {
+    for (int i = by; i < h; i += nby) {
         int u0 = i - h / 2;                                      // fftshift: y[i] = x[(i - n//2) mod n]
         u0 = u0 < 0 ? u0 + h : u0;
         const int um = u0 == 0 ? 0 : h - u0;                     // Hermitian mirror row: |F[u][v]| = |F[-u][-v]|
-        for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < w; j += gridDim.x * blockDim.x) {
+        for (int j = bx * blockDim.x + threadIdx.x; j < w; j += nbx * blockDim.x) {
             int v = j - w / 2;
             v = v < 0 ? v + w : v;
             const int u = v >= wh ? um : u0;
             v = v >= wh ? w - v : v;
-            double r = rint(__dadd_rn(__dmul_rn(src[(int64_t)u * wh + v], scale), shift));   // cvRound: ties to even
+            double r = rint(__dadd_rn(__dmul_rn(ms[(int64_t)u * wh + v], scale), shift));   // cvRound: ties to even
             r = r < 0.0 ? 0.0 : (r > 255.0 ? 255.0 : r);
-            dst[(int64_t)i * w + j] = (uint8_t)r;
+            out[(int64_t)i * w + j] = (uint8_t)r;
         }
     }
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// Ragged calls (v5ela_spectrum_ragged): frames of different sizes in one launch sequence, planned on the host
-// (v5ela_spec_plan.h). Each kernel flattens its grid in x; a CTA finds its frame through the chunk's CTA prefix table
-// (cta_frame) and then runs the body of the uniform kernel above for that frame, with the frame's FftPlan read from the size
-// table instead of a __grid_constant__. The bodies are copies, not shared functions, so that the uniform kernels' code stays
-// exactly as it is; every arithmetic step is the same, so every frame's image is byte-identical to v5ela_spectrum's.
+// Uniform calls (v5ela_spectrum): n frames of one size at a fixed stride. The frame is the last grid dimension; the others are
+// the DFT's TILE x TILE tiles (x across wh, y down h), the FFT's row pairs or column groups, and the image kernel's image_grid.
+__global__ void twiddle_kernel(double2 *tw, int n)
+{
+    twiddle_one(tw, n, blockIdx.x * blockDim.x + threadIdx.x);
+}
 
+__global__ void __launch_bounds__(256) dft_rows_kernel(const uint8_t *__restrict__ gray, int64_t frame_stride, int64_t row_stride,
+                                                       int h, int w, int wh, const double2 *__restrict__ tw, double2 *__restrict__ g)
+{
+    dft_rows_tile(gray + (int64_t)blockIdx.z * frame_stride, row_stride, h, w, wh, blockIdx.y * TILE, blockIdx.x * TILE, tw,
+                  g + (int64_t)blockIdx.z * h * wh);
+}
+
+__global__ void __launch_bounds__(256) dft_cols_kernel(const double2 *__restrict__ g, int h, int wh, const double2 *__restrict__ tw,
+                                                       double *__restrict__ ms, unsigned long long *__restrict__ minmax)
+{
+    dft_cols_tile(g + (int64_t)blockIdx.z * h * wh, h, wh, blockIdx.y * TILE, blockIdx.x * TILE, tw, ms + (int64_t)blockIdx.z * h * wh,
+                  minmax + 2 * blockIdx.z);
+}
+
+__global__ void __launch_bounds__(512) fft_rows_kernel(const uint8_t *__restrict__ gray, int64_t frame_stride, int64_t row_stride,
+                                                       int h, int w, int wh, const __grid_constant__ FftPlan plan,
+                                                       const double2 *__restrict__ tw, double2 *__restrict__ g)
+{
+    const int y0 = 2 * blockIdx.x;
+    fft_rows_pair(gray + (int64_t)blockIdx.y * frame_stride, row_stride, h, w, wh, y0, plan, tw, g + ((int64_t)blockIdx.y * h + y0) * wh);
+}
+
+__global__ void __launch_bounds__(512) fft_cols_kernel(const double2 *__restrict__ g, int h, int wh, int cc,
+                                                       const __grid_constant__ FftPlan plan, const double2 *__restrict__ tw,
+                                                       double *__restrict__ ms, unsigned long long *__restrict__ minmax)
+{
+    fft_cols_group(g + (int64_t)blockIdx.y * h * wh, h, wh, cc, blockIdx.x * cc, plan, tw, ms + (int64_t)blockIdx.y * h * wh,
+                   minmax + 2 * blockIdx.y);
+}
+
+__global__ void __launch_bounds__(256) spectrum_image_kernel(const double *__restrict__ ms, const unsigned long long *__restrict__ minmax,
+                                                             int h, int w, int wh, uint8_t *__restrict__ out)
+{
+    const int frame = blockIdx.z;
+    spectrum_image_part(ms + (int64_t)frame * h * wh, minmax + 2 * frame, h, w, wh, blockIdx.x, blockIdx.y, gridDim.x, gridDim.y,
+                        out + (int64_t)frame * h * w);
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// Ragged calls (v5ela_spectrum_ragged): one flat grid per launch; CTA blockIdx.x belongs to frame cta_frame(base, nf, blockIdx.x)
+// of the chunk's frame table, with local index blockIdx.x - base[frame] (SpecFrame: gx, cc, bx and by give the local layout).
 // The twiddle tables of every distinct side of the call, back to back in one arena: blockDim.x entries per CTA.
 __global__ void __launch_bounds__(256) twiddle_ragged_kernel(const SpecSize *__restrict__ sizes, int ns, const uint32_t *__restrict__ base,
                                                              double2 *__restrict__ tw)
 {
     const int k = cta_frame(base, ns, blockIdx.x);
-    const int n = sizes[k].n;
-    const int m = (int)(blockIdx.x - base[k]) * blockDim.x + threadIdx.x;
-    if (m >= n) return;
-    double s, c;
-    sincospi(2.0 * (double)m / (double)n, &s, &c);
-    tw[sizes[k].tw + m] = make_double2(c, -s);
+    twiddle_one(tw + sizes[k].tw, sizes[k].n, (int)(blockIdx.x - base[k]) * blockDim.x + threadIdx.x);
 }
 
-// dft_rows_kernel for one TILE x TILE output tile of one frame
 __global__ void __launch_bounds__(256) dft_rows_ragged_kernel(const SpecFrame *__restrict__ frames, int nf, const uint32_t *__restrict__ base,
                                                               const SpecSize *__restrict__ sizes, const double2 *__restrict__ tw_arena,
                                                               double2 *__restrict__ g)
 {
-    __shared__ double xs[TILE][KC + 1];
     const int fi = cta_frame(base, nf, blockIdx.x);
     const SpecFrame f = frames[fi];
-    const int local = (int)(blockIdx.x - base[fi]), ty_ = local / f.gx;
-    const int h = f.h, w = f.w, wh = f.wh;
-    const int64_t row_stride = f.row_stride;
-    const double2 *__restrict__ tw = tw_arena + sizes[f.sw].tw;
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const int y0 = ty_ * TILE, v0 = (local - ty_ * f.gx) * TILE;
-    const uint8_t *src = f.gray;
-    const int va = v0 + tx, vb = v0 + tx + 16;
-    int ia = 0, ib = 0;
-    const int sa = va % w, sb = vb % w;
-    double2 acc[2][2] = {{{0, 0}, {0, 0}}, {{0, 0}, {0, 0}}};
-    for (int x0 = 0; x0 < w; x0 += KC) {
-        for (int i = threadIdx.x; i < TILE * KC; i += 256) {
-            const int r = i / KC, c = i - r * KC;
-            const int y = y0 + r, x = x0 + c;
-            xs[r][c] = (y < h && x < w) ? (double)src[(int64_t)y * row_stride + x] : 0.0;
-        }
-        __syncthreads();
-        const int kn = min(KC, w - x0);
-        for (int k = 0; k < kn; k++) {
-            const double2 ta = tw[ia], tb = tw[ib];
-            const double xa = xs[ty][k], xb = xs[ty + 16][k];
-            acc[0][0].x = fma(xa, ta.x, acc[0][0].x); acc[0][0].y = fma(xa, ta.y, acc[0][0].y);
-            acc[0][1].x = fma(xa, tb.x, acc[0][1].x); acc[0][1].y = fma(xa, tb.y, acc[0][1].y);
-            acc[1][0].x = fma(xb, ta.x, acc[1][0].x); acc[1][0].y = fma(xb, ta.y, acc[1][0].y);
-            acc[1][1].x = fma(xb, tb.x, acc[1][1].x); acc[1][1].y = fma(xb, tb.y, acc[1][1].y);
-            ia += sa; ia = ia >= w ? ia - w : ia;
-            ib += sb; ib = ib >= w ? ib - w : ib;
-        }
-        __syncthreads();
-    }
-    double2 *dst = g + f.g_off;
-#pragma unroll
-    for (int i = 0; i < 2; i++) {
-        const int y = y0 + ty + 16 * i;
-        if (y >= h) continue;
-        if (va < wh) dst[(int64_t)y * wh + va] = acc[i][0];
-        if (vb < wh) dst[(int64_t)y * wh + vb] = acc[i][1];
-    }
+    const int local = (int)(blockIdx.x - base[fi]), ty = local / f.gx;
+    dft_rows_tile(f.gray, f.row_stride, f.h, f.w, f.wh, ty * TILE, (local - ty * f.gx) * TILE, tw_arena + sizes[f.sw].tw, g + f.g_off);
 }
 
-// dft_cols_kernel for one TILE x TILE output tile of one frame
 __global__ void __launch_bounds__(256) dft_cols_ragged_kernel(const SpecFrame *__restrict__ frames, int nf, const uint32_t *__restrict__ base,
                                                               const SpecSize *__restrict__ sizes, const double2 *__restrict__ tw_arena,
                                                               const double2 *__restrict__ g, double *__restrict__ ms,
                                                               unsigned long long *__restrict__ minmax)
 {
-    __shared__ double2 gs[KC][TILE + 1];
-    __shared__ unsigned long long smin, smax;
     const int fi = cta_frame(base, nf, blockIdx.x);
     const SpecFrame f = frames[fi];
-    const int local = (int)(blockIdx.x - base[fi]), ty_ = local / f.gx;
-    const int h = f.h, wh = f.wh;
-    const double2 *__restrict__ tw = tw_arena + sizes[f.sh].tw;
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const int u0 = ty_ * TILE, v0 = (local - ty_ * f.gx) * TILE;
-    const double2 *src = g + f.g_off;
-    if (threadIdx.x == 0) { smin = ~0ull; smax = 0ull; }
-    const int ua = u0 + ty, ub = u0 + ty + 16;
-    int ia = 0, ib = 0;
-    const int sa = ua % h, sb = ub % h;
-    double2 acc[2][2] = {{{0, 0}, {0, 0}}, {{0, 0}, {0, 0}}};
-    for (int y0 = 0; y0 < h; y0 += KC) {
-        for (int i = threadIdx.x; i < KC * TILE; i += 256) {
-            const int r = i / TILE, c = i - r * TILE;
-            const int y = y0 + r, v = v0 + c;
-            gs[r][c] = (y < h && v < wh) ? src[(int64_t)y * wh + v] : make_double2(0.0, 0.0);
-        }
-        __syncthreads();
-        const int kn = min(KC, h - y0);
-        for (int k = 0; k < kn; k++) {
-            const double2 ta = tw[ia], tb = tw[ib];
-            const double2 ga = gs[k][tx], gb = gs[k][tx + 16];
-            acc[0][0].x = fma(ga.x, ta.x, fma(-ga.y, ta.y, acc[0][0].x)); acc[0][0].y = fma(ga.x, ta.y, fma(ga.y, ta.x, acc[0][0].y));
-            acc[0][1].x = fma(gb.x, ta.x, fma(-gb.y, ta.y, acc[0][1].x)); acc[0][1].y = fma(gb.x, ta.y, fma(gb.y, ta.x, acc[0][1].y));
-            acc[1][0].x = fma(ga.x, tb.x, fma(-ga.y, tb.y, acc[1][0].x)); acc[1][0].y = fma(ga.x, tb.y, fma(ga.y, tb.x, acc[1][0].y));
-            acc[1][1].x = fma(gb.x, tb.x, fma(-gb.y, tb.y, acc[1][1].x)); acc[1][1].y = fma(gb.x, tb.y, fma(gb.y, tb.x, acc[1][1].y));
-            ia += sa; ia = ia >= h ? ia - h : ia;
-            ib += sb; ib = ib >= h ? ib - h : ib;
-        }
-        __syncthreads();
-    }
-    double *dst = ms + f.ms_off;
-    unsigned long long lo = ~0ull, hi = 0ull;
-#pragma unroll
-    for (int i = 0; i < 2; i++) {
-#pragma unroll
-        for (int j = 0; j < 2; j++) {
-            const int u = u0 + ty + 16 * i, v = v0 + tx + 16 * j;
-            if (u >= h || v >= wh) continue;
-            const double m = 20.0 * log(hypot(acc[i][j].x, acc[i][j].y) + 1.0);
-            dst[(int64_t)u * wh + v] = m;
-            const unsigned long long bits = (unsigned long long)__double_as_longlong(m);
-            lo = bits < lo ? bits : lo;
-            hi = bits > hi ? bits : hi;
-        }
-    }
-    atomicMin(&smin, lo);
-    atomicMax(&smax, hi);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        atomicMin(&minmax[2 * f.mm], smin);
-        atomicMax(&minmax[2 * f.mm + 1], smax);
-    }
+    const int local = (int)(blockIdx.x - base[fi]), ty = local / f.gx;
+    dft_cols_tile(g + f.g_off, f.h, f.wh, ty * TILE, (local - ty * f.gx) * TILE, tw_arena + sizes[f.sh].tw, ms + f.ms_off,
+                  minmax + 2 * f.mm);
 }
 
-// fft_rows_kernel for one pair of rows of one frame
 __global__ void __launch_bounds__(512) fft_rows_ragged_kernel(const SpecFrame *__restrict__ frames, int nf, const uint32_t *__restrict__ base,
                                                               const SpecSize *__restrict__ sizes, const double2 *__restrict__ tw_arena,
                                                               double2 *__restrict__ g)
 {
-    extern __shared__ double2 fbuf[];
     const int fi = cta_frame(base, nf, blockIdx.x);
     const SpecFrame f = frames[fi];
-    const int h = f.h, w = f.w, wh = f.wh;
-    const SpecSize &sz = sizes[f.sw];
-    const int y0 = 2 * (int)(blockIdx.x - base[fi]), y1 = y0 + 1;
-    const uint8_t *src = f.gray;
-    const uint8_t *r0 = src + (int64_t)y0 * f.row_stride, *r1 = src + (int64_t)(y1 < h ? y1 : y0) * f.row_stride;
-    for (int xb = 0; xb < w; xb += 4 * blockDim.x) {
-        uint8_t a[4], b[4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const int x = xb + j * blockDim.x + threadIdx.x;
-            a[j] = x < w ? r0[x] : 0;
-            b[j] = x < w ? r1[x] : 0;
-        }
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const int x = xb + j * blockDim.x + threadIdx.x;
-            if (x < w) fbuf[x] = make_double2((double)a[j], y1 < h ? (double)b[j] : 0.0);
-        }
-    }
-    __syncthreads();
-    const double2 *res = stockham(fbuf, fbuf + w, 1, sz.plan, tw_arena + sz.tw);
-    double2 *ga = g + f.g_off + (int64_t)y0 * wh;
-    for (int k = threadIdx.x; k < wh; k += blockDim.x) {
-        const double2 zk = res[k], zn = res[k == 0 ? 0 : w - k];
-        ga[k] = make_double2(0.5 * (zk.x + zn.x), 0.5 * (zk.y - zn.y));
-        if (y1 < h) ga[wh + k] = make_double2(0.5 * (zk.y + zn.y), 0.5 * (zn.x - zk.x));
-    }
+    const int y0 = 2 * (int)(blockIdx.x - base[fi]);
+    fft_rows_pair(f.gray, f.row_stride, f.h, f.w, f.wh, y0, sizes[f.sw].plan, tw_arena + sizes[f.sw].tw, g + f.g_off + (int64_t)y0 * f.wh);
 }
 
-// fft_cols_kernel for cc adjacent columns of one frame
 __global__ void __launch_bounds__(512) fft_cols_ragged_kernel(const SpecFrame *__restrict__ frames, int nf, const uint32_t *__restrict__ base,
                                                               const SpecSize *__restrict__ sizes, const double2 *__restrict__ tw_arena,
                                                               const double2 *__restrict__ g, double *__restrict__ ms,
                                                               unsigned long long *__restrict__ minmax)
 {
-    extern __shared__ double2 fbuf[];
-    __shared__ unsigned long long smin, smax;
-    __shared__ LogTab logtab;
-    if (threadIdx.x == 0) { smin = ~0ull; smax = 0ull; }
-    logtab_fill(logtab);
     const int fi = cta_frame(base, nf, blockIdx.x);
     const SpecFrame f = frames[fi];
-    const int h = f.h, wh = f.wh, cc = f.cc;
-    const SpecSize &sz = sizes[f.sh];
-    const int v0 = (int)(blockIdx.x - base[fi]) * cc;
-    const double2 *src = g + f.g_off;
-    const int csh = cc == 4 ? 2 : (cc == 2 ? 1 : 0);
-    for (int ib = 0; ib < h * cc; ib += 4 * blockDim.x) {
-        double2 t[4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const int i = ib + j * blockDim.x + threadIdx.x;
-            const int y = i >> csh, c = i & (cc - 1);
-            t[j] = (i < h * cc && v0 + c < wh) ? src[(int64_t)y * wh + v0 + c] : make_double2(0.0, 0.0);
-        }
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const int i = ib + j * blockDim.x + threadIdx.x;
-            const int y = i >> csh, c = i & (cc - 1);
-            if (i < h * cc) fbuf[c * h + y] = t[j];
-        }
-    }
-    __syncthreads();
-    const double2 *res = stockham(fbuf, fbuf + cc * h, cc, sz.plan, tw_arena + sz.tw);
-    double *dst = ms + f.ms_off;
-    unsigned long long lo = ~0ull, hi = 0ull;
-    for (int i = threadIdx.x; i < h * cc; i += blockDim.x) {
-        const int u = i >> csh, c = i & (cc - 1);
-        if (v0 + c >= wh) continue;
-        const double2 fv = res[c * h + u];
-        const double m = log_magnitude20(logtab, fma(fv.x, fv.x, fv.y * fv.y));
-        dst[(int64_t)u * wh + v0 + c] = m;
-        const unsigned long long bits = (unsigned long long)__double_as_longlong(m);
-        lo = bits < lo ? bits : lo;
-        hi = bits > hi ? bits : hi;
-    }
-    atomicMin(&smin, lo);
-    atomicMax(&smax, hi);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        atomicMin(&minmax[2 * f.mm], smin);
-        atomicMax(&minmax[2 * f.mm + 1], smax);
-    }
+    fft_cols_group(g + f.g_off, f.h, f.wh, f.cc, (int)(blockIdx.x - base[fi]) * f.cc, sizes[f.sh].plan, tw_arena + sizes[f.sh].tw,
+                   ms + f.ms_off, minmax + 2 * f.mm);
 }
 
-// spectrum_image_kernel for one (column block, row block) of one frame: f.bx x f.by CTAs per frame
 __global__ void __launch_bounds__(256) spectrum_image_ragged_kernel(const SpecFrame *__restrict__ frames, int nf, const uint32_t *__restrict__ base,
                                                                     const double *__restrict__ ms,
                                                                     const unsigned long long *__restrict__ minmax)
 {
     const int fi = cta_frame(base, nf, blockIdx.x);
     const SpecFrame f = frames[fi];
-    const int local = (int)(blockIdx.x - base[fi]), by_ = local / f.bx, bx_ = local - by_ * f.bx;
-    const int h = f.h, w = f.w, wh = f.wh;
-    const double mn = __longlong_as_double((long long)minmax[2 * f.mm]), mx = __longlong_as_double((long long)minmax[2 * f.mm + 1]);
-    const double scale = (mx - mn) > 2.220446049250313e-16 ? 255.0 / (mx - mn) : 0.0;
-    const double shift = 0.0 - mn * scale;
-    const double *src = ms + f.ms_off;
-    uint8_t *dst = f.out;
-    for (int i = by_; i < h; i += f.by) {
-        int u0 = i - h / 2;
-        u0 = u0 < 0 ? u0 + h : u0;
-        const int um = u0 == 0 ? 0 : h - u0;
-        for (int j = bx_ * blockDim.x + threadIdx.x; j < w; j += f.bx * blockDim.x) {
-            int v = j - w / 2;
-            v = v < 0 ? v + w : v;
-            const int u = v >= wh ? um : u0;
-            v = v >= wh ? w - v : v;
-            double r = rint(__dadd_rn(__dmul_rn(src[(int64_t)u * wh + v], scale), shift));
-            r = r < 0.0 ? 0.0 : (r > 255.0 ? 255.0 : r);
-            dst[(int64_t)i * w + j] = (uint8_t)r;
-        }
-    }
+    const int local = (int)(blockIdx.x - base[fi]), by = local / f.bx;
+    spectrum_image_part(ms + f.ms_off, minmax + 2 * f.mm, f.h, f.w, f.wh, local - by * f.bx, by, f.bx, f.by, f.out);
 }
 
 }  // namespace v5fft

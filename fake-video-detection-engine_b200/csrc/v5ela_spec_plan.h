@@ -73,6 +73,14 @@ inline bool fft_path(bool fft_on, int height, int width, FftPlan &plan_w, FftPla
            s.cols_smem <= FFT_SMEM_MAX;
 }
 
+// The image kernel's CTAs for one height x width frame: column blocks of 256 pixels, and row blocks such that every CTA walks ~16
+// rows, so that the per-thread set-up (the double-precision 255 / (max - min)) is paid once per 16 pixels. Sides of at most 65536
+// keep by <= 4096, within a grid's y limit.
+struct ImageGrid {
+    int bx, by;
+};
+inline ImageGrid image_grid(int height, int width) { return {(width + 255) / 256, (height + 15) / 16}; }
+
 // ------------------------------------------------------------------------------------------------------------ ragged calls
 // One distinct side length of a call: its twiddle table (tw[m] = exp(-2 pi i m / n), m < n) in the call's twiddle arena, and
 // its FFT plan (valid when `fft` is set).
@@ -201,9 +209,9 @@ inline void plan_spectrum_ragged(const v5ela_gray_desc *frames, int n, bool fft_
         FftShape s;
         f.cc = fft_path(fft_on, f.h, f.w, pw, ph, s) ? s.cc : 0;
         f.gx = (f.wh + TILE - 1) / TILE;
-        f.bx = (f.w + 255) / 256;                              // every CTA walks ~16 rows (v5ela_spectrum)
-        f.by = (f.h + 15) / 16;
-        f.by = f.by > 65535 ? 65535 : f.by;
+        const ImageGrid ig = image_grid(f.h, f.w);
+        f.bx = ig.bx;
+        f.by = ig.by;
     }
     P.tw_base.resize(P.sizes.size() + 1);
     P.tw_base[0] = 0;
