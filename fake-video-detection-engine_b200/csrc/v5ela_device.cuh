@@ -725,19 +725,23 @@ V5_DEV void fdct8(int *v)
 }
 
 // Inverse 8-point pass. FINAL: row pass, descale 18, +128 (the clamp to 0..255 happens in the saturating pack that
-// follows); otherwise column pass, descale 11.
-template <int S, bool FINAL>
+// follows); otherwise column pass, descale 11. WRAP16 (the JPEG decoder, v5jpeg_dec.cuh): the four sums that libjpeg-turbo's
+// x86 SIMD code forms in 16-bit lanes — in0 + in4, in0 - in4, in3 + in7, in1 + in5 — wrap to int16 as they do there, and the
+// row pass leaves out the +128 (the caller adds it after saturating to int8, as that code does). Inputs are int16, so every
+// other sum and product is exact in 32 bits: the largest magnitude is 2.12e9, too close to 2^31 to fold 128 << 18 into it.
+template <int S, bool FINAL, bool WRAP16 = false>
 V5_DEV void idct8(int *v)
 {
     const int n = FINAL ? 18 : 11;
-    const int rnd = (1 << (n - 1)) + (FINAL ? (128 << 18) : 0);
+    const int rnd = (1 << (n - 1)) + (FINAL && !WRAP16 ? (128 << 18) : 0);
     const int i2 = v[2 * S], i6 = v[6 * S];
     const int t2 = i2 * V5_C0_541 + i6 * (V5_C0_541 - V5_C1_847);
     const int t3 = i6 * V5_C0_541 + i2 * (V5_C0_541 + V5_C0_765);
-    const int t0 = (v[0] + v[4 * S]) * 8192 + rnd, t1 = (v[0] - v[4 * S]) * 8192 + rnd;
+    const int e0 = v[0] + v[4 * S], e1 = v[0] - v[4 * S];
+    const int t0 = (WRAP16 ? (int)(int16_t)e0 : e0) * 8192 + rnd, t1 = (WRAP16 ? (int)(int16_t)e1 : e1) * 8192 + rnd;
     int u0 = v[7 * S], u1 = v[5 * S], u2 = v[3 * S], u3 = v[S];
     const int z1 = (u0 + u3) * -V5_C0_899, z2 = (u1 + u2) * -V5_C2_562;
-    const int z3 = u0 + u2, z4 = u1 + u3;
+    const int z3 = WRAP16 ? (int)(int16_t)(u0 + u2) : u0 + u2, z4 = WRAP16 ? (int)(int16_t)(u1 + u3) : u1 + u3;
     const int z5 = (z3 + z4) * V5_C1_175;
     const int z3b = z3 * -V5_C1_961 + z5, z4b = z4 * -V5_C0_390 + z5;
     u0 = u0 * V5_C0_298 + z1 + z3b;

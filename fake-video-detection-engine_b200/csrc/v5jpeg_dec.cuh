@@ -477,6 +477,44 @@ V5_HOSTDEV void dc_apply_mcu(int16_t *mcu_dc, int bpm, int &py, int &pcb, int &p
 }
 
 // ------------------------------------------------------------------------------------------- inverse DCT of a block
+// The arithmetic of libjpeg-turbo's x86 SIMD ISLOW code (SSE2 / AVX2), which is what Pillow and OpenCV decode with on x86-64:
+// 16-bit lanes throughout. Dequantisation keeps the low 16 bits of coefficient x table entry; in0 +- in4, in3 + in7 and
+// in1 + in5 wrap to int16 (idct8<.., WRAP16>); the column-pass outputs saturate to int16 and the row-pass outputs to int8
+// before the +128. A block whose AC rows 1..7 are all zero takes a shortcut in the column pass: every output is the
+// dequantised DC of its column << 2, wrapping in 16 bits. Files written from pixels never leave int16 anywhere here
+// (DESIGN.md 4.1), so for them this is T.81 A.6 in wide integers; libjpeg-turbo's C path gives other samples than this on
+// blocks that do (DESIGN.md 4.6).
+
+// two ints -> an int16 pair, each saturated (PTX cvt.pack.sat.s16.s32 puts its first source in the high half)
+#ifdef __CUDA_ARCH__
+V5_DEV uint32_t pack_sat_s16(int lo, int hi)
+{
+    uint32_t d;
+    asm("cvt.pack.sat.s16.s32 %0, %1, %2;" : "=r"(d) : "r"(hi), "r"(lo));
+    return d;
+}
+// cvt.pack.sat.s8.s32: d = (c.lo16 << 16) | (sat_s8(a) << 8) | sat_s8(b)
+V5_DEV uint32_t packsat2_s8(int a, int b, uint32_t c)
+{
+    uint32_t d;
+    asm("cvt.pack.sat.s8.s32.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
+    return d;
+}
+#else
+inline uint32_t pack_sat_s16(int lo, int hi)
+{
+    const auto sat = [](int v) { return (uint32_t)(uint16_t)(v < -32768 ? -32768 : (v > 32767 ? 32767 : v)); };
+    return sat(lo) | (sat(hi) << 16);
+}
+inline uint32_t packsat2_s8(int a, int b, uint32_t c)
+{
+    const auto sat = [](int v) { return (uint32_t)(uint8_t)(v < -128 ? -128 : (v > 127 ? 127 : v)); };
+    return ((c & 0xffffu) << 16) | (sat(a) << 8) | sat(b);
+}
+#endif
+// four row-pass outputs -> samples [v0, v1, v2, v3]: each saturated to -128..127, then + 128 (flipping the top bit of a byte)
+V5_DEV uint32_t pack4_samples(int v0, int v1, int v2, int v3) { return packsat2_s8(v1, v0, packsat2_s8(v3, v2, 0u)) ^ 0x80808080u; }
+
 // `nat`: the block's 64 coefficients in NATURAL order (8 rows of 8 int16, 16-byte rows), `qt` likewise. Thread j of 4 takes
 // columns 2j, 2j+1 — one 32-bit word per row — dequantises, runs the column pass and leaves int16 pairs in ws; then rows
 // 2j, 2j+1 (one 128-bit load each) -> 8 clamped samples each.
@@ -484,17 +522,30 @@ V5_DEV void idct_cols(const int16_t *nat, const uint16_t *qt, int j, int16_t *ws
 {
     const uint32_t *cw = reinterpret_cast<const uint32_t *>(nat), *qw = reinterpret_cast<const uint32_t *>(qt);
     uint32_t *ww = reinterpret_cast<uint32_t *>(ws);
+    const v5::U4 *rows = reinterpret_cast<const v5::U4 *>(nat);
+    uint32_t ac = 0;                                                       // any AC coefficient in rows 1..7, all 8 columns
+#pragma unroll
+    for (int k = 1; k < 8; k++) {
+        const v5::U4 r = rows[k];
+        ac |= r.x | r.y | r.z | r.w;
+    }
     int a[8], b[8];
 #pragma unroll
     for (int k = 0; k < 8; k++) {
         const uint32_t c = cw[4 * k + j], q = qw[4 * k + j];
-        a[k] = v5::s16_lo(c) * (int)(q & 0xffffu);
-        b[k] = v5::s16_hi(c) * (int)(q >> 16);
+        a[k] = (int)(int16_t)(v5::s16_lo(c) * (int)(q & 0xffffu));
+        b[k] = (int)(int16_t)(v5::s16_hi(c) * (int)(q >> 16));
     }
-    v5::idct8<1, false>(a);
-    v5::idct8<1, false>(b);
+    if (!ac) {
+        const uint32_t w = v5::prmt((uint32_t)a[0] << 2, (uint32_t)b[0] << 2, 0x5410u);
 #pragma unroll
-    for (int k = 0; k < 8; k++) ww[4 * k + j] = v5::pack_s16(a[k], b[k]);
+        for (int k = 0; k < 8; k++) ww[4 * k + j] = w;
+        return;
+    }
+    v5::idct8<1, false, true>(a);
+    v5::idct8<1, false, true>(b);
+#pragma unroll
+    for (int k = 0; k < 8; k++) ww[4 * k + j] = pack_sat_s16(a[k], b[k]);
 }
 
 V5_DEV void idct_rows(const int16_t *ws, int j, uint8_t *dst, int pitch)
@@ -504,9 +555,9 @@ V5_DEV void idct_rows(const int16_t *ws, int j, uint8_t *dst, int pitch)
         const int r = 2 * j + rr;
         const v5::U4 w = *reinterpret_cast<const v5::U4 *>(ws + 8 * r);
         int v[8] = {v5::s16_lo(w.x), v5::s16_hi(w.x), v5::s16_lo(w.y), v5::s16_hi(w.y), v5::s16_lo(w.z), v5::s16_hi(w.z), v5::s16_lo(w.w), v5::s16_hi(w.w)};
-        v5::idct8<1, true>(v);
+        v5::idct8<1, true, true>(v);
         // plane rows are 8-byte aligned (plane offsets are multiples of 16, pitches multiples of 8)
-        *reinterpret_cast<v5::U2 *>(dst + r * pitch) = v5::U2{v5::pack4sat(v[0], v[1], v[2], v[3]), v5::pack4sat(v[4], v[5], v[6], v[7])};
+        *reinterpret_cast<v5::U2 *>(dst + r * pitch) = v5::U2{pack4_samples(v[0], v[1], v[2], v[3]), pack4_samples(v[4], v[5], v[6], v[7])};
     }
 }
 

@@ -258,9 +258,13 @@ V5ELA_API int v5ela_jpeg_encode_host(v5ela_handle *h, const uint8_t *img_host, i
 /*
  * Decoder: what the reference reads with `Image.open(crop_path).convert('RGB')` (v5_texture_ela.py:64) and
  * `cv2.imread(crop_path, cv2.IMREAD_GRAYSCALE)` (v5…:83) — the crops V1 wrote with cv2.imwrite (v1_keyframes_facetrack.py:166).
- * Pixel-identical to libjpeg's defaults (ISLOW inverse DCT, fancy upsampling). Supported: 8-bit baseline Huffman files with
+ * Pixel-identical to libjpeg's defaults (ISLOW inverse DCT, fancy upsampling) as Pillow and OpenCV run them on x86-64, i.e.
+ * libjpeg-turbo's x86 SIMD inverse DCT: its 16-bit arithmetic (dequantisation modulo 2^16, some sums wrapping, saturation
+ * between the passes) is reproduced exactly. Files written from pixels never reach that range; blocks a file can still carry
+ * (AC values near +-1023, large or 16-bit quantisation entries) decode differently in libjpeg-turbo's plain C path, which
+ * this decoder does not follow. Supported: 8-bit baseline Huffman files with
  * one component, or three components with the luma sampled 2x2 (4:2:0), 2x1 (4:2:2) or 1x1 (4:4:4) against 1x1 chroma; one
- * scan; any Huffman / quantisation tables; with or without restart intervals; an entropy-coded segment (stuffed bytes
+ * scan; any Huffman / quantisation tables (16-bit ones under SOF1 too); with or without restart intervals; an entropy-coded segment (stuffed bytes
  * included) of less than 2^29 - 2^20 bytes (511 MiB; the decoder's Huffman state holds 32-bit bit positions) — everything
  * PIL's and OpenCV's writers produce by default (4:2:0, no restarts) plus what their sampling and restart options add. Anything
  * else (progressive, other sampling factors, CMYK, 12-bit, arithmetic coding, larger entropy-coded segments) returns

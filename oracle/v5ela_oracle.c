@@ -325,6 +325,5 @@ void v5o_enhance_lut(int max_diff, uint8_t lut[256])
     }
 }
 
-/* Exported 1-D passes and helpers for the codec restatement (oracle/v5jpeg_oracle.c), which is linked into the same .so. */
+/* Exported 1-D pass for the codec restatement (oracle/v5jpeg_oracle.c), which is linked into the same .so. */
 void v5o_fdct_1d(const int32_t d[8], int32_t o[8], int first) { fdct_1d(d, o, first); }
-void v5o_idct_1d(const int32_t in[8], int32_t out[8], int n) { idct_1d(in, out, n); }

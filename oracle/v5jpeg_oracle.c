@@ -25,7 +25,6 @@
 
 void v5o_quant_tables(int quality, uint16_t luma[64], uint16_t chroma[64]);
 void v5o_fdct_1d(const int32_t d[8], int32_t o[8], int first);
-void v5o_idct_1d(const int32_t in[8], int32_t out[8], int n);
 
 /* zigzag position -> natural (row-major) index, T.81 Figure A.6 */
 static const uint8_t k_zigzag[64] = {0,  1,  8,  16, 9,  2,  3,  10, 17, 24, 32, 25, 18, 11, 4,  5,  12, 19, 26, 33, 40, 48,
@@ -520,17 +519,52 @@ int v5jo_layout(const uint8_t *data, size_t len, int *hs, int *vs, int *restart_
     return 0;
 }
 
-/* Dequantise + IDCT of one block (coefficients natural order) into a plane (A.6). */
+/* int16 wrap and saturation */
+static inline int32_t w16(int32_t v) { return (int32_t)(int16_t)(uint16_t)(uint32_t)v; }
+static inline int32_t sat16(int32_t v) { return v < -32768 ? -32768 : (v > 32767 ? 32767 : v); }
+
+/* One 8-point ISLOW pass (T.81 A.6 with libjpeg's constants) as libjpeg-turbo's x86 SIMD code computes it on int16 inputs:
+ * in0 + in4, in0 - in4, in3 + in7 and in1 + in5 are 16-bit lane adds that wrap; every product is a 16 x 16 -> 32-bit
+ * multiply-add, so the rest is exact (no 32-bit sum of int16 inputs reaches 2^31). -> (sum + 2^(n-1)) >> n. */
+static void simd_idct_1d(const int32_t in[8], int32_t out[8], int n)
+{
+    const int32_t t0 = w16(in[0] + in[4]) * 8192, t1 = w16(in[0] - in[4]) * 8192;
+    const int32_t t2 = in[2] * 4433 + in[6] * (4433 - 15137), t3 = in[2] * (4433 + 6270) + in[6] * 4433;
+    const int32_t e10 = t0 + t3, e13 = t0 - t3, e11 = t1 + t2, e12 = t1 - t2;
+    const int32_t z3 = w16(in[7] + in[3]), z4 = w16(in[5] + in[1]);
+    const int32_t z3b = z3 * (9633 - 16069) + z4 * 9633, z4b = z3 * 9633 + z4 * (9633 - 3196);
+    const int32_t o0 = in[7] * (2446 - 7373) + in[1] * -7373 + z3b;
+    const int32_t o3 = in[7] * -7373 + in[1] * (12299 - 7373) + z4b;
+    const int32_t o1 = in[5] * (16819 - 20995) + in[3] * -20995 + z4b;
+    const int32_t o2 = in[5] * -20995 + in[3] * (25172 - 20995) + z3b;
+    const int32_t r = 1 << (n - 1);
+    out[0] = (e10 + o3 + r) >> n; out[7] = (e10 - o3 + r) >> n;
+    out[1] = (e11 + o2 + r) >> n; out[6] = (e11 - o2 + r) >> n;
+    out[2] = (e12 + o1 + r) >> n; out[5] = (e12 - o1 + r) >> n;
+    out[3] = (e13 + o0 + r) >> n; out[4] = (e13 - o0 + r) >> n;
+}
+
+/* Dequantise + IDCT of one block (coefficients natural order) into a plane: ISLOW (A.6) with the arithmetic of libjpeg-turbo's
+ * x86 SIMD code, the decode Pillow and OpenCV give on x86-64. Dequantisation keeps the low 16 bits of coefficient x entry, the
+ * column-pass outputs saturate to int16 (or, when AC rows 1..7 of the block are all zero, are the dequantised DC << 2 wrapped
+ * to 16 bits), the samples saturate to 0..255. On the coefficients of files written from pixels nothing leaves int16 and this
+ * is A.6 in wide integers. */
 static void block_inverse(const int16_t coef[64], const uint16_t tab[64], uint8_t *plane, int pitch)
 {
     int32_t ws[64], tmp[8], res[8];
+    int ac = 0;
+    for (int k = 8; k < 64; k++) ac |= coef[k];
     for (int c = 0; c < 8; c++) {
-        for (int r = 0; r < 8; r++) tmp[r] = (int32_t)coef[r * 8 + c] * (int32_t)tab[r * 8 + c];
-        v5o_idct_1d(tmp, res, 11);
-        for (int r = 0; r < 8; r++) ws[r * 8 + c] = res[r];
+        for (int r = 0; r < 8; r++) tmp[r] = w16((int32_t)coef[r * 8 + c] * (int32_t)tab[r * 8 + c]);
+        if (ac) {
+            simd_idct_1d(tmp, res, 11);
+            for (int r = 0; r < 8; r++) ws[r * 8 + c] = sat16(res[r]);
+        } else {
+            for (int r = 0; r < 8; r++) ws[r * 8 + c] = w16(tmp[0] * 4);
+        }
     }
     for (int r = 0; r < 8; r++) {
-        v5o_idct_1d(&ws[r * 8], res, 18);
+        simd_idct_1d(&ws[r * 8], res, 18);
         for (int c = 0; c < 8; c++) plane[r * pitch + c] = clamp_u8(res[c] + 128);
     }
 }

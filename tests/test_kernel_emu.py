@@ -8,7 +8,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from helpers import HERE, golden_frame, load_json, record_matches_golden, sha
+from helpers import adversarial_blocks_frame, HERE, golden_frame, load_json, record_matches_golden, sha
 from oracle import c_oracle
 from oracle.pil_oracle import RECORD_DTYPE
 from v5ela.synth import gen_frame
@@ -264,40 +264,6 @@ def test_emulated_two_regime_decomposition(emu):
             assert emu.lib.v5emu_last_split_frame() == 36 and emu.lib.v5emu_last_segments(0) == 1 and emu.lib.v5emu_last_segments(1) == 3
     finally:
         emu.lib.v5emu_set_target_items(0)
-
-
-def adversarial_blocks_frame(rng=None):
-    """A frame whose 8x8 blocks drive the intermediates of the round trip to their extremes: for every pair (u, v) the sign
-    pattern of the 2-D basis function (u, v) at full swing (0 / 255) and its negative — these maximise the forward row / column
-    outputs and, at coarse tables, the quantisation error that the inverse column pass amplifies — plus the rounded cosine itself,
-    single-pixel impulses, and all of it again per channel in saturated colours (chroma blocks see the same patterns)."""
-    import math
-
-    blocks = []
-    for u in range(8):
-        for v in range(8):
-            cu = [math.cos((2 * x + 1) * u * math.pi / 16) for x in range(8)]
-            cv = [math.cos((2 * y + 1) * v * math.pi / 16) for y in range(8)]
-            sign = np.array([[255 if cu[x] * cv[y] >= 0 else 0 for x in range(8)] for y in range(8)], np.uint8)
-            cosb = np.array([[int(round(127.5 + 127.5 * cu[x] * cv[y])) for x in range(8)] for y in range(8)], np.uint8)
-            blocks += [sign, 255 - sign, cosb, 255 - cosb]
-    for k in range(8):
-        imp = np.zeros((8, 8), np.uint8)
-        imp[k, 7 - k] = 255
-        blocks += [imp, 255 - imp]
-    n = len(blocks)                                       # 272 luma blocks -> 17 x 16 blocks
-    cols = 16
-    rows = (n + cols - 1) // cols
-    plane = np.zeros((8 * rows, 8 * cols), np.uint8)
-    for i, b in enumerate(blocks):
-        plane[8 * (i // cols):8 * (i // cols) + 8, 8 * (i % cols):8 * (i % cols) + 8] = b
-    gray = np.repeat(plane[..., None], 3, axis=2)
-    # chroma sees 2x2-averaged planes: upscale the patterns by two so that the chroma blocks get the same extremes
-    big = np.kron(plane, np.ones((2, 2), np.uint8))
-    col = np.zeros(big.shape + (3,), np.uint8)
-    col[..., 0] = big                                     # red swings: Cr (and Cb) at full range
-    col[..., 2] = 255 - big
-    return gray, col
 
 
 @pytest.mark.parametrize("q", [1, 2, 25, 50, 90, 100])
